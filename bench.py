@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W [--workload full|ofdm] [--streams S]
   python bench.py --impl reference ...      # the reference's own CPU implementation on the host cores
+  python bench.py ... --dump-outputs DIR    # also writes what the last timed step computed to DIR/<name>.npy
 
 Workload (BASELINE.json configs[3], the north-star target): the FULL chain -- OFDM demodulation (PRS sync, FFT, DQPSK,
 frequency de-interleave) -> FIC + 18 x EEP 3-A DAB+ sub-channels (time de-interleave, de-puncture, K=7 Viterbi, energy
@@ -369,6 +370,48 @@ def channel_legs(pkg, tx, np, torch, local_rank, stream, n_streams=256, reps=6):
     return out
 
 
+DUMP_STREAMS, DUMP_SOFT_STREAMS, DUMP_SEED = 512, 16, 2024   # about 44 MB of .npy for the default ensemble
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, np, ctxs, n_subs):
+    """Writes what a caller of the timed step receives after its last step, for a fixed seeded sample of the streams (the same
+    sample on every run with the same --streams): decoded FIC/MSC bytes as dabgpu_chan_get_fic / dabgpu_chan_get_msc return
+    them and the newest soft-bit frame as dabgpu_ofdm_fetch_latest returns it.  Integer outputs are stored as float32 (exact)."""
+    per_ctx = ctxs[0].max_streams
+    n_all = per_ctx * len(ctxs)
+    rng = np.random.default_rng(DUMP_SEED)
+    streams = np.sort(rng.choice(n_all, size=min(n_all, DUMP_STREAMS), replace=False))
+    soft_streams = np.sort(rng.choice(streams, size=min(streams.size, DUMP_SOFT_STREAMS), replace=False))
+    where = lambda s: (ctxs[int(s) // per_ctx], int(s) % per_ctx)
+    out = {"streams": streams, "soft_bit_streams": soft_streams}
+    latest = [where(s)[0].ofdm_fetch_latest(where(s)[1], 1) for s in soft_streams]
+    out["soft_bits"] = np.concatenate([f for f, _ in latest])
+    out["soft_bits_produced"] = np.concatenate([p for _, p in latest])
+    out["soft_bits"][out["soft_bits_produced"] == 0] = 0      # no frame this step: the staging rows hold stale bytes
+
+    if n_subs:
+        fic, fic_ok, msc, msc_valid, status = [], [], [], [], []
+        for s in streams:
+            g, i = where(s)
+            fibs, ok = g.get_fic(i)
+            fic.append(fibs)
+            fic_ok.append(ok)
+            subs = [g.get_msc(i, k) for k in range(n_subs)]
+            msc.append(np.concatenate([b for b, _ in subs], axis=1))      # [nb_cifs, bytes of every sub-channel]
+            msc_valid.append(np.stack([v for _, v in subs], axis=1))      # [nb_cifs, sub-channels]
+            status.append(g.chan_status(i))
+        out.update(fic=np.stack(fic), fic_crc_ok=np.stack(fic_ok), msc=np.stack(msc), msc_valid=np.stack(msc_valid),
+                   chan_status=np.array(status))
+    out = {k: v.astype(np.float32) for k, v in out.items()}
+    total = sum(v.nbytes for v in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def timed_pass(torch, dist, world, stream, step, K, finish=None, start=None):
     """K steps bracketed by barrier + synchronize, CUDA events on `stream`; returns ms (this rank)."""
     torch.cuda.synchronize()
@@ -404,6 +447,8 @@ def main():
     ap.add_argument("--no-channel-leg", action="store_true", help="skip the channel-decode-only sub-legs (BASELINE configs[2])")
     ap.add_argument("--no-c32-leg", action="store_true", help="skip the OFDM-only sub-leg with complex<float> input (256 streams)")
     ap.add_argument("--wc-host", action="store_true", help="e2e: write-combined pinned memory for the IQ the host feeds in")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps of the main leg, write what its last step computed "
+                                                           "(seeded sample of rank 0's streams) to DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -527,8 +572,9 @@ def main():
         def join(self):
             pass
 
-    def run_leg(with_chan, K=K, c32=None, n_streams=None):
-        """W warm-up steps, K timed steps (device-resident), K profiled steps.  Returns a dict of raw measurements."""
+    def run_leg(with_chan, K=K, c32=None, n_streams=None, dump_dir=None):
+        """W warm-up steps, K timed steps (device-resident), K profiled steps.  Returns a dict of raw measurements.
+        dump_dir: write the outputs of the last timed step there (dump_outputs) before the profiled steps change them."""
         g = CtxGroup(with_chan, n_streams) if c32 is None else C32Group(c32)
 
         def step():
@@ -544,6 +590,8 @@ def main():
         ms = timed_pass(torch, dist, world, stream, step, K, finish=g.join, start=g.fork)
         c1 = g.counters()
         launches = g.launch_count - launches0
+        if dump_dir and rank == 0:
+            dump_outputs(dump_dir, np, g.ctxs, len(subs) if with_chan else 0)
         # second pass with CUDA events around every kernel launch (dabgpu_profile_*): per-kernel times for the roofline.  The
         # library keeps the channel decode on the main stream while profiling, so this pass is slower than the one above.
         g.profile_enable(True)
@@ -558,7 +606,7 @@ def main():
     sampler.start()
     sampler.ready.wait(timeout=20)   # NVML initialisation on a fresh box can take longer than the whole timed region
     sampler.samples.clear()          # keep only what is sampled while the kernels run
-    main_leg = run_leg(full)
+    main_leg = run_leg(full, dump_dir=args.dump_outputs)
     sampler.stop_flag = True
     sampler.join(timeout=2)
     clocks = sampler.summary()

@@ -195,7 +195,9 @@ def test_aac_frame_processor_class(driver, tx, pyref):
 
 def test_radio_block_chain(driver, tx, pyref):
     """Radio_Block: complex<float> blocks into OFDM_Demod::Process, soft bits stay on the device, FIBs and sub-channel bytes
-    come out of the BasicRadio observers; everything equals the reference chain on the same recording."""
+    come out of the BasicRadio observers.  The frames and soft bits match the reference OFDM_Demod on the same recording (one LSB);
+    the FIBs and bytes equal the reference's FIC and MSC decoders fed the frames the adapter emitted and, where the reference build
+    is the oracle, fed the reference's own frames."""
     mode, block = 1, 65536
     subs = [tx.Subchannel(0, 0, 48, eep_level=2), tx.Subchannel(1, 48, 54, eep_level=2, eep_type_b=True, dabplus=False)]
     ens = tx.EnsembleTx(mode, subs, seed=77)
@@ -215,9 +217,22 @@ def test_radio_block_chain(driver, tx, pyref):
     for off in range(0, n, block):
         o.process_c32(c32[off:off + block])
     exp_frames = o.pop_frames()
-    o_fic = pyref.RefFic() if use_ref else pyref.PortFic()
-    mk = pyref.RefMsc if use_ref else pyref.PortMsc
-    o_msc = [mk(sc.start_address, sc.length, sc.is_uep, sc.uep_index, sc.eep_level, sc.eep_type_b) for sc in subs]
+
+    def decode(soft_frames):
+        """FIBs and per-sub-channel bytes of the oracle's FIC and MSC decoders over these soft-bit frames"""
+        o_fic = pyref.RefFic() if use_ref else pyref.PortFic()
+        mk = pyref.RefMsc if use_ref else pyref.PortMsc
+        o_msc = [mk(sc.start_address, sc.length, sc.is_uep, sc.uep_index, sc.eep_level, sc.eep_type_b) for sc in subs]
+        exp_fibs, exp_msc = [], [[] for _ in subs]
+        for b in soft_frames:
+            for c in range(4):
+                exp_fibs += o_fic.decode_group(b[c * 2304:(c + 1) * 2304], c)
+            for k in range(len(subs)):
+                for c in range(4):
+                    e = o_msc[k].decode_cif(b[9216 + c * 55296:9216 + (c + 1) * 55296])
+                    if e.size:
+                        exp_msc[k].append(e)
+        return exp_fibs, exp_msc
 
     # the reference order per frame would be FIBs then sub-channels (BasicRadio::Process); the adapter decodes the frame
     # on the device first and then reports the soft bits, so the records are grouped by tag before comparing
@@ -244,22 +259,20 @@ def test_radio_block_chain(driver, tx, pyref):
             off += 8 + ln
     assert len(frames) == len(exp_frames) >= n_frames - 2
     assert total_read == len(exp_frames)
-    exp_fibs, exp_msc = [], [[] for _ in subs]
     for (bits, fto), (eb, _, _, et) in zip(frames, exp_frames):
         assert fto == et
         assert np.abs(bits.astype(np.int32) - eb.astype(np.int32)).max() <= 1
-        for c in range(4):
-            exp_fibs += o_fic.decode_group(eb[c * 2304:(c + 1) * 2304], c)
+    # one LSB can flip a Viterbi decision, so the exact comparison feeds the oracle's decoders the soft bits the adapter reported
+    # (the ones it decoded).  The C restatement's OFDM is itself only within one LSB of the reference's, so the end-to-end
+    # comparison with the oracle's own frames is made where the reference build is the oracle.
+    sources = [[b for b, _ in frames]] + ([[e[0] for e in exp_frames]] if use_ref else [])
+    for src in sources:
+        exp_fibs, exp_msc = decode(src)
+        assert fibs == exp_fibs
         for k in range(len(subs)):
-            for c in range(4):
-                e = o_msc[k].decode_cif(eb[9216 + c * 55296:9216 + (c + 1) * 55296])
-                if e.size:
-                    exp_msc[k].append(e)
-    assert fibs == exp_fibs
-    for k in range(len(subs)):
-        assert len(msc[k]) == len(exp_msc[k])
-        for a, b in zip(msc[k], exp_msc[k]):
-            assert np.array_equal(a, b)
+            assert len(msc[k]) == len(exp_msc[k])
+            for a, b in zip(msc[k], exp_msc[k]):
+                assert np.array_equal(a, b)
 
 
 def test_basic_radio_configures_itself_from_the_fic(driver, tx, pyref):
