@@ -151,6 +151,45 @@ DABGPU_API int dabgpu_ofdm_attach_device_input(dabgpu_ctx* ctx, const void* d_iq
                                                size_t capacity_samples);
 DABGPU_API int dabgpu_ofdm_advance(dabgpu_ctx* ctx, int first_stream, int n_streams, int n_samples, int block_size);
 
+/* ---------------------------------------------------------------------------------------------
+ * Wideband front end.  Replaces, for every ensemble of a multi-ensemble capture at once, the 2.048 MHz VFO that
+ * DABModule::enable puts in front of OFDM_Demod in the plugin (SURVEY.md 3.1) and the reference's
+ * examples/apply_frequency_shift (SURVEY.md 2.1): mix each ensemble to baseband, low-pass filter and decimate to 2.048 MS/s.
+ *
+ * A source is one capture at fs = D x 2 048 000 Hz, D in {1, 2, 4, 8, 16}, in one of the formats below, scaled exactly as
+ * dabgpu_iq_convert scales it.  Channel c (= context stream c) is the ensemble of source[c] centred offset_hz[c] above the
+ * capture centre, |offset_hz[c]| + 768 000 <= fs / 2.  With h = firwin(64 D + 1, 856 kHz, Kaiser beta = kaiser_beta(70 dB))
+ * (unit DC gain, computed in double on the host), f^ = 4000 round(f / 4000) (half away from zero), delta = f - f^, input before
+ * sample 0 = 0, output n of a channel is
+ *     y[n] = exp(-j 2 pi delta n D / fs) * sum_{i=0}^{64 D} h[i] x[n D - i] exp(-j 2 pi f^ (n D - i) / fs)
+ * up to the aliasing beyond 1.024 MHz that the frequency-domain decimation drops (>= 75 dB down).  Every phase comes from the
+ * absolute sample index in exact integer arithmetic modulo fs, so nothing drifts.  After n_in input samples per source, every
+ * channel holds 448 floor(n_in / (448 D)) output samples; output n depends only on the input and n, whatever the call sizes.
+ * ------------------------------------------------------------------------------------------- */
+enum { DABGPU_WB_RAW_U8 = 0, DABGPU_WB_RAW_S8 = 1, DABGPU_WB_RAW_S16L = 2, DABGPU_WB_RAW_F32L = 3 };   /* the reference's mode strings */
+typedef struct {
+    int sample_rate;        /* Hz, 2 048 000 x {1, 2, 4, 8, 16}, shared by every source */
+    int format;             /* DABGPU_WB_*, shared by every source */
+    int n_sources;
+    int n_channels;         /* <= max_streams of the context */
+    const int* source;      /* [n_channels] source of channel c */
+    const int* offset_hz;   /* [n_channels] centre of channel c relative to the capture centre, Hz */
+} dabgpu_wideband_config;
+typedef struct dabgpu_wideband dabgpu_wideband;
+/* Validates cfg and attaches d_out (c32, channel c sample k at d_out[c * capacity_samples + (k mod capacity_samples)], the layout
+ * of dabgpu_ofdm_attach_device_input with stride = capacity) to the context: every stream is reset, and dabgpu_ofdm_process /
+ * dabgpu_submit return DABGPU_ERR_STATE from then on.  capacity_samples: power of two that holds a transmission frame, the
+ * NULL + PRS window and a margin of 1472 samples.  The context must be created with DABGPU_IQ_C32; one front end per context
+ * (a second open returns DABGPU_ERR_STATE).  Close it before destroying the context. */
+DABGPU_API int dabgpu_wideband_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, void* d_out, size_t capacity_samples,
+                                    dabgpu_wideband** out);
+/* Copies n_samples raw samples of every source (source s at iq_host + s * source_stride_bytes) to the device, filters them into
+ * d_out and runs OFDM_Demod::Process on channels [0, n_channels) over the new output samples, presented as Process() blocks of
+ * block_size (<= 0: one block).  Returns once the host buffer may be reused; *n_out = output samples per channel this call. */
+DABGPU_API int dabgpu_wideband_process(dabgpu_wideband* w, const void* iq_host, size_t source_stride_bytes, size_t n_samples,
+                                       int block_size, size_t* n_out);
+DABGPU_API int dabgpu_wideband_close(dabgpu_wideband* w);
+
 /* On_OFDM_Frame: number of undelivered soft-bit frames per stream, then copy them out in order.
  * Each frame is nb_frame_bits int8.  infos (optional) receives per-frame {coarse, fine} offsets
  * and fine time offset as observed when the frame was emitted. */

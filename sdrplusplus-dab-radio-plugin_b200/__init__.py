@@ -19,6 +19,9 @@ OK, ERR_INVALID, ERR_CUDA, ERR_NOMEM, ERR_STATE, ERR_OVERFLOW = 0, -1, -2, -3, -
 IQ_U8, IQ_C32 = 0, 1
 MAX_SEGMENTS = 5
 EV_FIRECODE_ERROR, EV_RS_ERROR, EV_SUPERFRAME_HEADER, EV_AU_CRC_ERROR, EV_ACCESS_UNIT = 1, 2, 3, 4, 5
+WB_RAW_U8, WB_RAW_S8, WB_RAW_S16L, WB_RAW_F32L = 0, 1, 2, 3
+WB_FORMATS = {"raw_u8": WB_RAW_U8, "raw_s8": WB_RAW_S8, "raw_s16l": WB_RAW_S16L, "raw_f32l": WB_RAW_F32L}
+WB_BYTES_PER_SAMPLE = {WB_RAW_U8: 2, WB_RAW_S8: 2, WB_RAW_S16L: 4, WB_RAW_F32L: 8}
 
 
 class DabGpuError(RuntimeError):
@@ -88,6 +91,11 @@ class Step(C.Structure):
                 ("fic_crc_host", C.c_void_p), ("chan_status_host", C.c_void_p)]
 
 
+class WidebandConfig(C.Structure):
+    _fields_ = [("sample_rate", C.c_int), ("format", C.c_int), ("n_sources", C.c_int), ("n_channels", C.c_int),
+                ("source", C.POINTER(C.c_int)), ("offset_hz", C.POINTER(C.c_int))]
+
+
 CIF_OUT_STRIDE, FIC_GROUP_STRIDE, PIPELINE_DEPTH = 6912, 128, 2
 
 PROF_CLASSES = ("ofdm_ctl", "ofdm_demod", "viterbi", "dabplus", "chan_misc")
@@ -104,7 +112,7 @@ EXPORTS = [
     "dabgpu_autocfg_create", "dabgpu_autocfg_destroy", "dabgpu_autocfg_push_fibs", "dabgpu_autocfg_dump", "dabgpu_autocfg_runnable",
     "dabgpu_host_alloc", "dabgpu_host_free", "dabgpu_ofdm_get_frame_data_vec", "dabgpu_ofdm_get_correlation_buffer", "dabgpu_autocfg_applied", "dabgpu_msc_add_subchannel", "dabgpu_msc_remove_subchannel", "dabgpu_chan_join",
     "dabgpu_autocfg_apply", "dabgpu_ofdm_get_response", "dabgpu_ofdm_get_frame_fft", "dabgpu_iq_convert", "dabgpu_softbits_to_bytes", "dabgpu_bytes_to_softbits",
-    "dabgpu_packet_fec_decode",
+    "dabgpu_packet_fec_decode", "dabgpu_wideband_open", "dabgpu_wideband_process", "dabgpu_wideband_close",
 ]
 
 _lib = None
@@ -181,6 +189,9 @@ def load_library() -> C.CDLL:
     L.dabgpu_iq_convert.argtypes = [C.c_char_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
     L.dabgpu_softbits_to_bytes.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p]
     L.dabgpu_bytes_to_softbits.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p]
+    L.dabgpu_wideband_open.argtypes = [C.c_void_p, C.POINTER(WidebandConfig), C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]
+    L.dabgpu_wideband_process.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_int, C.POINTER(C.c_size_t)]
+    L.dabgpu_wideband_close.argtypes = [C.c_void_p]
     _lib = L
     return L
 
@@ -252,6 +263,8 @@ class DabGpu:
         self._subs = {}
 
     def close(self):
+        if getattr(self, "_wideband", None) is not None:
+            self._wideband.close()
         if getattr(self, "h", None):
             self.L.dabgpu_ctx_destroy(self.h)
             self.h = None
@@ -446,6 +459,14 @@ class DabGpu:
         _check(self.L.dabgpu_ofdm_advance(self.h, first_stream, self.max_streams - first_stream if n_streams is None else n_streams,
                                           n_samples, block_size))
 
+    def wideband_open(self, sample_rate: int, fmt, sources: Sequence[int], offsets_hz: Sequence[int], d_out: int,
+                      capacity_samples: int, n_sources: Optional[int] = None) -> "Wideband":
+        """dabgpu_wideband_open: channel c = ensemble of capture sources[c] at offsets_hz[c] from its centre, written as c32 to the
+        device buffer d_out ([channel][capacity_samples], e.g. a torch.complex64 tensor's data_ptr()) and fed to stream c."""
+        w = Wideband(self, sample_rate, fmt, sources, offsets_hz, d_out, capacity_samples, n_sources)
+        self._wideband = w
+        return w
+
     def submit(self, iq_ptr: int, iq_stride_bytes: int, n_samples: int, block_size: int = 65536, first_stream: int = 0,
                n_streams: Optional[int] = None, run_chan_decode: bool = False, **out_ptrs) -> int:
         """dabgpu_submit: queue H2D + OFDM (+ channel decode) + D2H without blocking; returns the ticket.
@@ -511,6 +532,43 @@ class DabGpu:
         produced = np.zeros(n, dtype=np.uint8)
         _check(self.L.dabgpu_ofdm_fetch_latest(self.h, first_stream, n, _ptr(frames), _ptr(produced)))
         return frames, produced
+
+
+class Wideband:
+    """Wideband front end of one context (dabgpu_wideband_*): splits multi-ensemble captures into the context's streams."""
+
+    def __init__(self, ctx: DabGpu, sample_rate: int, fmt, sources: Sequence[int], offsets_hz: Sequence[int], d_out: int,
+                 capacity_samples: int, n_sources: Optional[int] = None):
+        self.L, self.ctx = ctx.L, ctx
+        self.format = WB_FORMATS[fmt] if isinstance(fmt, str) else int(fmt)
+        self.n_sources = (max(sources) + 1 if len(sources) else 0) if n_sources is None else n_sources
+        src = (C.c_int * max(len(sources), 1))(*sources)
+        off = (C.c_int * max(len(offsets_hz), 1))(*offsets_hz)
+        cfg = WidebandConfig(sample_rate, self.format, self.n_sources, len(sources), src, off)
+        self.h = C.c_void_p()
+        _check(self.L.dabgpu_wideband_open(ctx.h, C.byref(cfg), C.c_void_p(d_out), capacity_samples, C.byref(self.h)))
+
+    def process(self, iq: np.ndarray, block_size: int = 65536) -> int:
+        """iq: [n_sources, ...] host array, each row one source's raw samples (u8 / s8 / s16 I,Q pairs, f32 I,Q or complex64).
+        Returns the new output samples per channel."""
+        assert iq.ndim == 2 and iq.shape[0] == self.n_sources and iq.strides[1] == iq.itemsize
+        n = (iq.shape[1] * iq.itemsize) // WB_BYTES_PER_SAMPLE[self.format]
+        n_out = C.c_size_t(0)
+        _check(self.L.dabgpu_wideband_process(self.h, C.c_void_p(iq.ctypes.data), iq.strides[0], n, block_size, C.byref(n_out)))
+        return n_out.value
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.dabgpu_wideband_close(self.h)
+            self.h = None
+            if getattr(self.ctx, "_wideband", None) is self:
+                self.ctx._wideband = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class FicAutoConfig:

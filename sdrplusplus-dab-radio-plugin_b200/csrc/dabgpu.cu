@@ -6,6 +6,7 @@
 #include "chan.cuh"
 #include "dabplus.cuh"
 #include "ofdm_host.cuh"
+#include "wideband.cuh"
 #include "../host/fic_autoconfig.hpp"
 #include "../host/capture_formats.hpp"
 #include <algorithm>
@@ -67,6 +68,7 @@ struct dabgpu_ctx {
 
     // OFDM
     OfdmState ofdm;
+    dabgpu_wideband* wb = nullptr;   // open wideband front end feeding the OFDM stage (dabgpu_wideband_open)
 
     // dabgpu_submit / dabgpu_wait pipeline
     struct PipeSlot {
@@ -93,6 +95,8 @@ static cudaError_t sync_ctx(dabgpu_ctx* ctx) {
     if (e != cudaSuccess) return e;
     return cudaStreamSynchronize(ctx->stream);
 }
+
+static void wb_detach(dabgpu_wideband* w);
 
 extern "C" {
 
@@ -328,6 +332,7 @@ void dabgpu_ctx_destroy(dabgpu_ctx* ctx) {
     if (ctx->ev_dp) cudaEventDestroy(ctx->ev_dp);
     if (ctx->ev_dp_fork) cudaEventDestroy(ctx->ev_dp_fork);
     if (ctx->s_h2d) { cudaStreamSynchronize(ctx->s_h2d); cudaStreamDestroy(ctx->s_h2d); }
+    if (ctx->wb) wb_detach(ctx->wb);
     if (ctx->s_d2h) { cudaStreamSynchronize(ctx->s_d2h); cudaStreamDestroy(ctx->s_d2h); }
     ofdm_destroy(ctx->ofdm);
     dabplus_destroy(ctx->dabplus);
@@ -1400,6 +1405,257 @@ int dabgpu_msc_get_layout(dabgpu_ctx* ctx, int stream, int sub_index, int* offse
     if (sub_index < 0 || size_t(sub_index) >= hs.size() || !hs[size_t(sub_index)].active) return set_error(DABGPU_ERR_INVALID, "sub-channel index %d not configured", sub_index);
     if (offset) *offset = int(hs[size_t(sub_index)].out_offset);
     if (bytes_per_cif) *bytes_per_cif = int(hs[size_t(sub_index)].n_out_bytes);
+    return DABGPU_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Wideband front end (kernel in wideband.cuh)
+// ---------------------------------------------------------------------------------------------
+}  // extern "C"
+
+struct dabgpu_wideband {
+    dabgpu_ctx* ctx = nullptr;   // null once the context was destroyed
+    int D = 1, fmt = 0, bps = 2, n_sources = 0, n_channels = 0;
+    long long fs = 0;
+    DevBuf d_ring, d_H, d_twf, d_twi, d_dposf, d_dposi, d_chans, d_first;
+    int ring_log2 = 0;
+    size_t ring_cap = 0, out_cap = 0, headroom = 0;
+    unsigned long long max_pass_blocks = 0;
+    float2* d_out = nullptr;
+    unsigned long long n_in = 0, blocks_done = 0, out_consumed = 0;   // input samples per source, blocks filtered, outputs handed to OFDM
+};
+
+static void wb_detach(dabgpu_wideband* w) {
+    DevBuf* bufs[] = {&w->d_ring, &w->d_H, &w->d_twf, &w->d_twi, &w->d_dposf, &w->d_dposi, &w->d_chans, &w->d_first};
+    for (DevBuf* b : bufs) b->release();
+    if (w->ctx) w->ctx->wb = nullptr;
+    w->ctx = nullptr;
+}
+
+// Kaiser-windowed sinc low-pass, unit DC gain: scipy.signal.firwin(64 D + 1, 856e3, window=('kaiser', kaiser_beta(70)), fs)
+static void wb_design_taps(int D, std::vector<double>& h) {
+    const int T = 64 * D + 1;
+    const double c = 856e3 / (0.5 * 2048000.0 * D), beta = 0.1102 * (70.0 - 8.7), alpha = 0.5 * (T - 1);
+    auto i0 = [](double x) {
+        double sum = 1.0, term = 1.0;
+        for (int k = 1; k < 200 && term > 1e-18 * sum; k++) { const double q = x / (2.0 * k); term *= q * q; sum += term; }
+        return sum;
+    };
+    h.assign(size_t(T), 0.0);
+    double sum = 0.0;
+    for (int n = 0; n < T; n++) {
+        const double m = n - alpha, r = m / alpha;
+        const double sinc = (m == 0.0) ? 1.0 : sin(M_PI * c * m) / (M_PI * c * m);
+        h[size_t(n)] = c * sinc * i0(beta * sqrt(std::max(0.0, 1.0 - r * r))) / i0(beta);
+        sum += h[size_t(n)];
+    }
+    for (double& v : h) v /= sum;
+}
+
+// padded position of natural index k in the digit-reversed output of fft_cta<n> (DIF radices 8, 8, ..., then 4 or 2)
+static void wb_dpos(int n, std::vector<uint16_t>& dpos) {
+    std::vector<int> radices;
+    int m = n;
+    while (m % 8 == 0 && m > 1) { radices.push_back(8); m /= 8; }
+    if (m > 1) radices.push_back(m);
+    dpos.resize(size_t(n));
+    for (int k = 0; k < n; k++) {
+        int a = 0, rem = n, kk = k;
+        for (int R : radices) { const int d = kk % R; kk /= R; rem /= R; a += d * rem; }
+        dpos[size_t(k)] = uint16_t(OFDM_PAD(a));
+    }
+}
+
+static void wb_roots(int n, std::vector<float2>& tw) {
+    tw.resize(size_t(n / 8));
+    for (int k = 0; k < n / 8; k++) tw[size_t(k)] = make_float2(float(cos(-2.0 * M_PI * k / n)), float(sin(-2.0 * M_PI * k / n)));
+}
+
+// one entry per (D, format): W == nullptr sets the kernel's shared-memory attribute, otherwise launches nb blocks of every source
+typedef int (*WbKernelFn)(const WbDev* W, unsigned long long block0, unsigned nb, int n_sources, cudaStream_t cs);
+template <int D, int FMT> static int wb_kernel_t(const WbDev* W, unsigned long long block0, unsigned nb, int n_sources, cudaStream_t cs) {
+    if (!W) {
+        CUDA_TRY(cudaFuncSetAttribute(k_wideband<D, FMT>, cudaFuncAttributeMaxDynamicSharedMemorySize, WbCfg<D>::SMEM));
+        return DABGPU_OK;
+    }
+    k_wideband<D, FMT><<<dim3(nb, unsigned(n_sources)), 64 * D, WbCfg<D>::SMEM, cs>>>(*W, block0);
+    CUDA_TRY(cudaGetLastError());
+    return DABGPU_OK;
+}
+#define WB_ROW(D) {wb_kernel_t<D, 0>, wb_kernel_t<D, 1>, wb_kernel_t<D, 2>, wb_kernel_t<D, 3>}
+static const WbKernelFn kWbKernels[5][4] = {WB_ROW(1), WB_ROW(2), WB_ROW(4), WB_ROW(8), WB_ROW(16)};
+#undef WB_ROW
+static WbKernelFn wb_kernel(int D, int fmt) { return kWbKernels[__builtin_ctz(unsigned(D))][fmt]; }
+
+extern "C" {
+
+int dabgpu_wideband_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, void* d_out, size_t capacity, dabgpu_wideband** out) {
+    if (!ctx || !cfg || !d_out || !out) return set_error(DABGPU_ERR_INVALID, "null argument");
+    *out = nullptr;
+    if (ctx->wb) return set_error(DABGPU_ERR_STATE, "a wideband front end is already open on this context");
+    if (ctx->cfg.iq_format != DABGPU_IQ_C32) return set_error(DABGPU_ERR_INVALID, "the wideband front end writes c32: the context needs DABGPU_IQ_C32");
+    const int D = cfg->sample_rate / 2048000;
+    if (cfg->sample_rate <= 0 || cfg->sample_rate % 2048000 != 0 || (D != 1 && D != 2 && D != 4 && D != 8 && D != 16))
+        return set_error(DABGPU_ERR_INVALID, "sample rate %d Hz is not 2.048 MHz x 1, 2, 4, 8 or 16", cfg->sample_rate);
+    if (cfg->format < DABGPU_WB_RAW_U8 || cfg->format > DABGPU_WB_RAW_F32L) return set_error(DABGPU_ERR_INVALID, "bad wideband format %d", cfg->format);
+    if (cfg->n_sources < 1 || cfg->n_sources > 65535) return set_error(DABGPU_ERR_INVALID, "n_sources %d out of range", cfg->n_sources);
+    if (cfg->n_channels < 1 || cfg->n_channels > ctx->cfg.max_streams)
+        return set_error(DABGPU_ERR_INVALID, "n_channels %d: the context holds %d streams", cfg->n_channels, ctx->cfg.max_streams);
+    if (!cfg->source || !cfg->offset_hz) return set_error(DABGPU_ERR_INVALID, "null channel table");
+    const long long fs = cfg->sample_rate;
+    for (int c = 0; c < cfg->n_channels; c++) {
+        if (cfg->source[c] < 0 || cfg->source[c] >= cfg->n_sources) return set_error(DABGPU_ERR_INVALID, "channel %d: source %d out of range", c, cfg->source[c]);
+        if (std::llabs((long long)cfg->offset_hz[c]) + 768000 > fs / 2)
+            return set_error(DABGPU_ERR_INVALID, "channel %d: offset %d Hz puts the ensemble outside +-fs/2", c, cfg->offset_hz[c]);
+    }
+    const size_t min_cap = size_t(ctx->P.nb_frame_samples) + size_t(ctx->P.nb_null_period + ctx->P.nb_symbol_period) + 1024 + WB_OUT;
+    if (!is_pow2(capacity) || capacity < min_cap || capacity > (size_t(1) << 30))
+        return set_error(DABGPU_ERR_INVALID, "capacity %zu: must be a power of two in [%zu, 2^30]", capacity, min_cap);
+
+    dabgpu_wideband* w = new dabgpu_wideband();
+    w->D = D; w->fmt = cfg->format; w->fs = fs;
+    w->bps = (cfg->format == DABGPU_WB_RAW_F32L) ? 8 : (cfg->format == DABGPU_WB_RAW_S16L) ? 4 : 2;
+    w->n_sources = cfg->n_sources; w->n_channels = cfg->n_channels;
+    w->out_cap = capacity;
+    w->headroom = ofdm_ring_headroom(ctx->P, capacity);
+    w->max_pass_blocks = std::min<unsigned long long>(512, w->headroom / WB_OUT);
+    w->d_out = static_cast<float2*>(d_out);
+    while ((size_t(1) << w->ring_log2) < (w->max_pass_blocks + 2) * WB_OUT * size_t(D)) w->ring_log2++;
+    w->ring_cap = size_t(1) << w->ring_log2;
+
+    // channels grouped by source, in channel order
+    std::vector<WbChan> chans;
+    std::vector<int> first(size_t(cfg->n_sources) + 1, 0);
+    for (int s = 0; s < cfg->n_sources; s++) {
+        first[size_t(s)] = int(chans.size());
+        for (int c = 0; c < cfg->n_channels; c++) {
+            if (cfg->source[c] != s) continue;
+            const int f = cfg->offset_hz[c];
+            const int bin = f >= 0 ? (f + 2000) / 4000 : -((2000 - f) / 4000);   // round half away from zero
+            chans.push_back(WbChan{bin, f - 4000 * bin, c, 0});
+        }
+    }
+    first[size_t(cfg->n_sources)] = int(chans.size());
+
+    const int N = 512 * D;
+    std::vector<double> h;
+    wb_design_taps(D, h);
+    std::vector<float2> H(WB_IFFT), twf, twi;
+    for (int i = 0; i < WB_IFFT; i++) {
+        const int u = i < WB_IFFT / 2 ? i : i - WB_IFFT;
+        double re = 0.0, im = 0.0;
+        for (size_t n = 0; n < h.size(); n++) {
+            const long long k = ((long long)u * (long long)n) % N;
+            re += h[n] * cos(-2.0 * M_PI * double(k) / N);
+            im += h[n] * sin(-2.0 * M_PI * double(k) / N);
+        }
+        H[size_t(i)] = make_float2(float(re / N), float(im / N));
+    }
+    wb_roots(N, twf);
+    wb_roots(WB_IFFT, twi);
+    std::vector<uint16_t> dposf, dposi;
+    wb_dpos(N, dposf);
+    wb_dpos(WB_IFFT, dposi);
+
+    int rc = DABGPU_OK;
+#define WB_TRY(expr) do { if ((rc = (expr))) { wb_detach(w); delete w; return rc; } } while (0)
+    cudaError_t e = cudaSetDevice(ctx->cfg.device);
+    if (e != cudaSuccess) { delete w; return set_error(DABGPU_ERR_CUDA, "cudaSetDevice: %s", cudaGetErrorString(e)); }
+    WB_TRY(w->d_ring.alloc(size_t(cfg->n_sources) * w->ring_cap * size_t(w->bps)));
+    WB_TRY(w->d_H.alloc(H.size() * sizeof(float2)));
+    WB_TRY(w->d_twf.alloc(twf.size() * sizeof(float2)));
+    WB_TRY(w->d_twi.alloc(twi.size() * sizeof(float2)));
+    WB_TRY(w->d_dposf.alloc(dposf.size() * 2));
+    WB_TRY(w->d_dposi.alloc(dposi.size() * 2));
+    WB_TRY(w->d_chans.alloc(chans.size() * sizeof(WbChan)));
+    WB_TRY(w->d_first.alloc(first.size() * sizeof(int)));
+    const std::pair<DevBuf*, std::pair<const void*, size_t>> up[] = {
+        {&w->d_H, {H.data(), H.size() * sizeof(float2)}}, {&w->d_twf, {twf.data(), twf.size() * sizeof(float2)}},
+        {&w->d_twi, {twi.data(), twi.size() * sizeof(float2)}}, {&w->d_dposf, {dposf.data(), dposf.size() * 2}},
+        {&w->d_dposi, {dposi.data(), dposi.size() * 2}}, {&w->d_chans, {chans.data(), chans.size() * sizeof(WbChan)}},
+        {&w->d_first, {first.data(), first.size() * sizeof(int)}}};
+    for (const auto& u : up) {
+        e = cudaMemcpy(u.first->p, u.second.first, u.second.second, cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) { wb_detach(w); delete w; return set_error(DABGPU_ERR_CUDA, "cudaMemcpy: %s", cudaGetErrorString(e)); }
+    }
+    WB_TRY(wb_kernel(D, w->fmt)(nullptr, 0, 0, 0, ctx->stream));
+    WB_TRY(ofdm_attach(ctx->ofdm, d_out, capacity, capacity, ctx->stream));
+#undef WB_TRY
+    w->ctx = ctx;
+    ctx->wb = w;
+    *out = w;
+    return DABGPU_OK;
+}
+
+int dabgpu_wideband_process(dabgpu_wideband* w, const void* iq_host, size_t stride, size_t n_samples, int block_size, size_t* n_out) {
+    if (!w) return set_error(DABGPU_ERR_INVALID, "null wideband front end");
+    if (n_out) *n_out = 0;
+    dabgpu_ctx* ctx = w->ctx;
+    if (!ctx) return set_error(DABGPU_ERR_STATE, "the context of this wideband front end was destroyed");
+    if (!iq_host && n_samples) return set_error(DABGPU_ERR_INVALID, "null input");
+    if (w->n_sources > 1 && stride < n_samples * size_t(w->bps)) return set_error(DABGPU_ERR_INVALID, "source stride %zu is shorter than a source", stride);
+    const unsigned long long blk_in = WB_OUT * (unsigned long long)w->D, hist = 64ull * w->D;
+    const size_t new_out = size_t((w->n_in + n_samples) / blk_in - w->blocks_done) * WB_OUT;
+    const size_t bs = block_size > 0 ? size_t(block_size) : std::max<size_t>(new_out, 1);
+    if (bs + WB_OUT > w->headroom)
+        return set_error(DABGPU_ERR_INVALID, "block_size %zu does not fit the output ring (%zu samples of headroom)", bs, w->headroom);
+    CUDA_TRY(cudaSetDevice(ctx->cfg.device));
+    CUDA_TRY(join_if_many_frames(ctx, long(std::min<size_t>(new_out, 1ul << 40))));
+    ctx->ofdm.demod_ctas_cap = ctx->dp_pending ? 3 : 0;   // a channel decode is running on its stream: share the SMs with it
+    const WbKernelFn kern = wb_kernel(w->D, w->fmt);
+    WbDev W;
+    W.ring = w->d_ring.as<uint8_t>(); W.ring_log2 = w->ring_log2; W.ring_mask = w->ring_cap - 1;
+    W.out = w->d_out; W.out_cap = w->out_cap;
+    W.H = w->d_H.as<float2>(); W.tw_fwd = w->d_twf.as<float2>(); W.tw_inv = w->d_twi.as<float2>();
+    W.dpos_fwd = w->d_dposf.as<uint16_t>(); W.dpos_inv = w->d_dposi.as<uint16_t>();
+    W.chans = w->d_chans.as<WbChan>(); W.chan_first = w->d_first.as<int>(); W.fs = w->fs;
+    const uint8_t* src = static_cast<const uint8_t*>(iq_host);
+    size_t done = 0;
+    for (;;) {
+        // input: the ring keeps everything from the first sample the next block reads (its 64 D samples of history)
+        const unsigned long long keep = w->blocks_done * blk_in >= hist ? w->blocks_done * blk_in - hist : 0;
+        const size_t take = std::min<size_t>(n_samples - done, size_t(keep + w->ring_cap - w->n_in));
+        for (size_t left = take, off = done; left > 0;) {
+            const size_t pos = size_t(w->n_in & (w->ring_cap - 1)), run = std::min(left, w->ring_cap - pos);
+            const size_t bytes = run * size_t(w->bps);
+            CUDA_TRY(cudaMemcpy2DAsync(w->d_ring.as<uint8_t>() + pos * size_t(w->bps), w->ring_cap * size_t(w->bps), src + off * size_t(w->bps),
+                                       w->n_sources > 1 ? stride : bytes, bytes, size_t(w->n_sources), cudaMemcpyHostToDevice, ctx->stream));
+            w->n_in += run; off += run; left -= run;
+        }
+        done += take;
+        // filter: whole blocks, never more than the OFDM stage's headroom ahead of what it consumed
+        const size_t pending = size_t(w->blocks_done * WB_OUT - w->out_consumed);
+        const unsigned long long nb = std::min({w->n_in / blk_in - w->blocks_done, w->max_pass_blocks, (unsigned long long)((w->headroom - pending) / WB_OUT)});
+        if (nb) {
+            int rc = kern(&W, w->blocks_done, unsigned(nb), w->n_sources, ctx->stream);
+            if (rc) return rc;
+            ctx->launches++;
+            w->blocks_done += nb;
+        }
+        // OFDM_Demod::Process over the new outputs in blocks of bs; a partial block only at the end of the call
+        const size_t avail = size_t(w->blocks_done * WB_OUT - w->out_consumed);
+        const bool last = done == n_samples && w->n_in / blk_in == w->blocks_done;
+        const size_t present = last ? avail : (avail / bs) * bs;
+        if (present) {
+            int rc = ofdm_run(ctx->ofdm, 0, w->n_channels, int(present), int(bs), ctx->stream);
+            if (rc) return rc;
+            w->out_consumed += present;
+        }
+        if (last) break;
+    }
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    if (n_out) *n_out = new_out;
+    return DABGPU_OK;
+}
+
+int dabgpu_wideband_close(dabgpu_wideband* w) {
+    if (!w) return set_error(DABGPU_ERR_INVALID, "null wideband front end");
+    if (w->ctx) {
+        cudaSetDevice(w->ctx->cfg.device);
+        sync_ctx(w->ctx);
+    }
+    wb_detach(w);
+    delete w;
     return DABGPU_OK;
 }
 

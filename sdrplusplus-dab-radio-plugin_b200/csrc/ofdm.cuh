@@ -214,7 +214,7 @@ __device__ __forceinline__ void fft_cta(float2 (&x)[8], float* __restrict__ re, 
             re[a] = v.x; im[a] = v.y;
         }
     }
-    constexpr int RF = (N == 2048 || N == 256) ? 4 : (N == 1024 ? 2 : 1);
+    constexpr int RF = (N == 2048 || N == 256) ? 4 : ((N == 1024 || N == 8192) ? 2 : 1);   // N / 8^stages
     if (RF == 4) {
         __syncthreads();
 #pragma unroll

@@ -413,9 +413,10 @@ static int ofdm_upload(OfdmState& O, const void* iq_host, size_t stride_bytes, i
 }
 
 // samples that may be written ahead of the consumer without touching the frame being assembled or the correlation window
-static size_t ofdm_ring_headroom(const OfdmState& O) {
-    return O.ring_cap - size_t(O.P.nb_frame_samples) - size_t(O.P.nb_null_period + O.P.nb_symbol_period) - 1024;
+static size_t ofdm_ring_headroom(const dabgpu_params& P, size_t ring_cap) {
+    return ring_cap - size_t(P.nb_frame_samples) - size_t(P.nb_null_period + P.nb_symbol_period) - 1024;
 }
+static size_t ofdm_ring_headroom(const OfdmState& O) { return ofdm_ring_headroom(O.P, O.ring_cap); }
 
 static int ofdm_process(OfdmState& O, const void* iq_host, size_t stride_bytes, int first, int n, int n_samples, int block_size, cudaStream_t cs) {
     if (O.external_ring) return set_error(DABGPU_ERR_STATE, "a device input buffer is attached: use dabgpu_ofdm_advance");

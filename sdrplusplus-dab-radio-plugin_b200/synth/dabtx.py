@@ -648,3 +648,47 @@ def periodic_frames(mode: int, subchannels: Sequence[Subchannel], seed: int, per
     if return_logical:
         return np.stack(frames[period_frames:]), {k: np.stack(v) for k, v in cache.items()}
     return np.stack(frames[period_frames:])
+
+
+def wideband_capture(mode: int, ensembles: Sequence[np.ndarray], D: int, offsets_hz: Sequence[int], snr_db: float = 15.0,
+                     cfo_hz: Sequence[float] = (), shifts: Sequence[int] = (), gains_db: Sequence[float] = (), seed: int = 0,
+                     mask_hz: float = 800e3) -> np.ndarray:
+    """One period of a periodic multi-ensemble capture at D x 2.048 MS/s (complex128; np.take(..., mode="wrap") continues it).
+    ensembles[k] = the coded frames of one period of periodic_frames(); ensemble k gets AWGN at snr_db, a band limit of
+    +-mask_hz (a transmitter's spectrum mask), a CFO of cfo_hz[k] and a time shift of shifts[k] samples (both cyclic), the gain
+    gains_db[k], and sits offsets_hz[k] above the capture centre.  Built in the frequency domain over the whole period, so the
+    CFO and the offsets are rounded to the period's bin spacing (2.048 MHz / period samples, about 2 Hz)."""
+    p = MODES[mode]
+    L = len(ensembles[0]) * p.nb_frame_samples
+    M = D * L
+    Y = np.zeros(M, dtype=np.complex128)
+    fb = np.fft.fftfreq(L, 1.0 / L).astype(np.int64)
+    keep = np.nonzero(np.abs(fb) * 2048000.0 / L <= mask_hz)[0]
+    rng = np.random.default_rng(seed)
+    sigma = np.sqrt(0.5 * 10 ** (-snr_db / 10))
+    for k, f in enumerate(offsets_hz):
+        x = ofdm_modulate(list(ensembles[k]), mode).astype(np.complex128)
+        assert x.size == L
+        x = x + sigma * (rng.standard_normal(L) + 1j * rng.standard_normal(L))
+        if k < len(shifts):
+            x = np.roll(x, shifts[k])
+        X = np.fft.fft(x)
+        shift = int(round(f * L / 2048000.0)) + (int(round(cfo_hz[k] * L / 2048000.0)) if k < len(cfo_hz) else 0)
+        g = 10 ** ((gains_db[k] if k < len(gains_db) else 0.0) / 20)
+        np.add.at(Y, (fb[keep] + shift) % M, X[keep] * (D * g))
+    return np.fft.ifft(Y)
+
+
+def quantize(iq: np.ndarray, fmt: str, rms: float) -> np.ndarray:
+    """complex samples scaled to `rms` (LSB, or full scale for raw_f32l) -> raw interleaved I,Q of a reader mode
+    (examples/app_helpers/app_iq_readers.h); values beyond the format's range clip."""
+    v = np.empty(iq.size * 2, dtype=np.float64)
+    v[0::2], v[1::2] = iq.real, iq.imag
+    v *= rms / np.sqrt(np.mean(np.abs(iq) ** 2))
+    if fmt == "raw_u8":
+        return np.clip(np.round(v + 127.5), 0, 255).astype(np.uint8)
+    if fmt == "raw_s8":
+        return np.clip(np.round(v), -127, 127).astype(np.int8)
+    if fmt == "raw_s16l":
+        return np.clip(np.round(v), -32767, 32767).astype("<i2")
+    return v.astype("<f4")
