@@ -146,6 +146,8 @@ __device__ __forceinline__ uint32_t crc_mulmod(const uint32_t a, const uint32_t 
 // CRC16-CCITT (init 0xFFFF, final inversion; crc.h:46-67) of n bytes by a whole warp: lane l runs the table loop over its chunk
 // of ceil(n / 32) bytes (lane 0 carries the initial value), weighs the result with x^(8 * bytes that follow) and the lanes XOR
 // their shares.  A 300-byte access unit is a dependent chain of 10 table steps instead of 300.  Every lane returns the CRC.
+// Lane 0 reads weight n - ceil(n / 32); n is at most a superframe (5 logical frames of up to CIF_OUT_STRIDE bytes).
+static_assert(CRC_XP8_ENTRIES >= 5 * CIF_OUT_STRIDE, "g_crc_xp8 must hold a weight for every access-unit length");
 __device__ __forceinline__ uint16_t crc16_ccitt_warp(const uint16_t* tab, const uint8_t* p, const int n, const uint32_t lane) {
     const int c = (n + 31) >> 5;
     const int b0 = min(n, int(lane) * c), b1 = min(n, b0 + c);

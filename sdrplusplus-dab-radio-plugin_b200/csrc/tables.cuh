@@ -34,9 +34,10 @@ __constant__ uint32_t c_branch[32];
 __constant__ uint16_t c_crc_ccitt[256];
 __constant__ uint16_t c_crc_fire[256];
 
-// x^(8m) mod the CCITT polynomial, m = 0..2047: the weight of a partial CRC that is followed by m more bytes (k_dabplus splits
-// the CRC of an access unit over the 32 lanes of a warp).  In global memory: every lane reads a different entry.
-#define CRC_XP8_ENTRIES 2048
+// x^(8m) mod the CCITT polynomial, m = 0..34559: the weight of a partial CRC that is followed by m more bytes (k_dabplus splits
+// the CRC of an access unit over the 32 lanes of a warp).  An access unit lies inside one superframe of at most 5 * 6912 bytes,
+// so m stays below that (static_assert next to crc16_ccitt_warp).  In global memory: every lane reads a different entry.
+#define CRC_XP8_ENTRIES 34560
 __device__ uint16_t g_crc_xp8[CRC_XP8_ENTRIES];
 
 // Time de-interleaver: age (0 = newest CIF) of the CIF that carries bit i of the oldest complete
