@@ -165,6 +165,17 @@ DABGPU_API int dabgpu_ofdm_advance(dabgpu_ctx* ctx, int first_stream, int n_stre
  * up to the aliasing beyond 1.024 MHz that the frequency-domain decimation drops (>= 75 dB down).  Every phase comes from the
  * absolute sample index in exact integer arithmetic modulo fs, so nothing drifts.  After n_in input samples per source, every
  * channel holds 448 floor(n_in / (448 D)) output samples; output n depends only on the input and n, whatever the call sizes.
+ *
+ * dabgpu_wideband_open_any_rate accepts every integer fs that dabgpu_wideband_plan supports (2.048 to 32.768 MS/s, e.g. the
+ * 2.4, 2.5, 3, 6, 8, 10, 12.5 and 20 MS/s of common tuners) under the same offset rule.  With the plan's bin spacing Delta, T
+ * taps h = firwin(T, 856 kHz, same Kaiser window, unit DC gain) at fs, f^ = Delta round(f / Delta) (half away from zero),
+ * delta = f - f^ and input before sample 0 = 0, let
+ *     v[m] = sum_{i<T} h[i] x[m - i] exp(-j 2 pi f^ (m - i) / fs).
+ * Output n is exp(-j 2 pi delta n / 2 048 000) times the band-limited (|f| < 1.024 MHz) interpolation of v evaluated at input
+ * time n fs / 2 048 000, up to the same >= 75 dB aliasing; where n fs / 2 048 000 is an integer this is the formula above.  All
+ * phases are exact integers modulo N_in and 2 048 000.  After n_in input samples per source every channel holds
+ * step_out floor(n_in / step_in) output samples, whatever the call sizes.  At fs = 2.048 MHz x 2^d the output is bit-identical
+ * to dabgpu_wideband_open's.
  * ------------------------------------------------------------------------------------------- */
 enum { DABGPU_WB_RAW_U8 = 0, DABGPU_WB_RAW_S8 = 1, DABGPU_WB_RAW_S16L = 2, DABGPU_WB_RAW_F32L = 3 };   /* the reference's mode strings */
 typedef struct {
@@ -176,6 +187,16 @@ typedef struct {
     const int* offset_hz;   /* [n_channels] centre of channel c relative to the capture centre, Hz */
 } dabgpu_wideband_config;
 typedef struct dabgpu_wideband dabgpu_wideband;
+/* Block geometry of the filter bank at one rate.  bin_hz = Delta in {4000, 2000, 1000}; fft_in = fs / Delta (<= 8192, no prime
+ * factor above 5) forward-FFT points per block; fft_out = 2 048 000 / Delta inverse-FFT points per channel; each block advances
+ * step_in input and step_out output samples (step_in / step_out = fs / 2 048 000); taps = T = 2 ceil(fs / 64 000) + 1.  Of
+ * the Delta that qualify, the plan takes the one with the fewest inverse-FFT operations per output sample.  At
+ * 2.048 MHz x D: Delta = 4000, fft_in = 512 D, steps 448 D / 448, T = 64 D + 1. */
+typedef struct {
+    int bin_hz, fft_in, fft_out, step_in, step_out, taps;
+} dabgpu_wideband_geometry;
+/* Fills *g for sample_rate, or returns DABGPU_ERR_INVALID (with a message) when the rate is not supported.  Needs no device. */
+DABGPU_API int dabgpu_wideband_plan(int sample_rate, dabgpu_wideband_geometry* g);
 /* Validates cfg and attaches d_out (c32, channel c sample k at d_out[c * capacity_samples + (k mod capacity_samples)], the layout
  * of dabgpu_ofdm_attach_device_input with stride = capacity) to the context: every stream is reset, and dabgpu_ofdm_process /
  * dabgpu_submit return DABGPU_ERR_STATE from then on.  capacity_samples: power of two that holds a transmission frame, the
@@ -183,6 +204,10 @@ typedef struct dabgpu_wideband dabgpu_wideband;
  * (a second open returns DABGPU_ERR_STATE).  Close it before destroying the context. */
 DABGPU_API int dabgpu_wideband_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, void* d_out, size_t capacity_samples,
                                     dabgpu_wideband** out);
+/* dabgpu_wideband_open for any rate dabgpu_wideband_plan supports (cfg->sample_rate); capacity_samples must hold a transmission
+ * frame, the NULL + PRS window and a margin of 1024 + step_out samples.  Process and close as for dabgpu_wideband_open. */
+DABGPU_API int dabgpu_wideband_open_any_rate(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, void* d_out,
+                                             size_t capacity_samples, dabgpu_wideband** out);
 /* Copies n_samples raw samples of every source (source s at iq_host + s * source_stride_bytes) to the device, filters them into
  * d_out and runs OFDM_Demod::Process on channels [0, n_channels) over the new output samples, presented as Process() blocks of
  * block_size (<= 0: one block).  Returns once the host buffer may be reused; *n_out = output samples per channel this call. */

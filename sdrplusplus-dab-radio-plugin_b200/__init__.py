@@ -96,6 +96,10 @@ class WidebandConfig(C.Structure):
                 ("source", C.POINTER(C.c_int)), ("offset_hz", C.POINTER(C.c_int))]
 
 
+class WidebandGeometry(C.Structure):
+    _fields_ = [(n, C.c_int) for n in ("bin_hz", "fft_in", "fft_out", "step_in", "step_out", "taps")]
+
+
 CIF_OUT_STRIDE, FIC_GROUP_STRIDE, PIPELINE_DEPTH = 6912, 128, 2
 
 PROF_CLASSES = ("ofdm_ctl", "ofdm_demod", "viterbi", "dabplus", "chan_misc")
@@ -113,6 +117,7 @@ EXPORTS = [
     "dabgpu_host_alloc", "dabgpu_host_free", "dabgpu_ofdm_get_frame_data_vec", "dabgpu_ofdm_get_correlation_buffer", "dabgpu_autocfg_applied", "dabgpu_msc_add_subchannel", "dabgpu_msc_remove_subchannel", "dabgpu_chan_join",
     "dabgpu_autocfg_apply", "dabgpu_ofdm_get_response", "dabgpu_ofdm_get_frame_fft", "dabgpu_iq_convert", "dabgpu_softbits_to_bytes", "dabgpu_bytes_to_softbits",
     "dabgpu_packet_fec_decode", "dabgpu_wideband_open", "dabgpu_wideband_process", "dabgpu_wideband_close",
+    "dabgpu_wideband_plan", "dabgpu_wideband_open_any_rate",
 ]
 
 _lib = None
@@ -192,6 +197,8 @@ def load_library() -> C.CDLL:
     L.dabgpu_wideband_open.argtypes = [C.c_void_p, C.POINTER(WidebandConfig), C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]
     L.dabgpu_wideband_process.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_int, C.POINTER(C.c_size_t)]
     L.dabgpu_wideband_close.argtypes = [C.c_void_p]
+    L.dabgpu_wideband_plan.argtypes = [C.c_int, C.POINTER(WidebandGeometry)]
+    L.dabgpu_wideband_open_any_rate.argtypes = L.dabgpu_wideband_open.argtypes
     _lib = L
     return L
 
@@ -228,6 +235,14 @@ def get_params(mode: int) -> Params:
     p = Params()
     _check(load_library().dabgpu_get_params(mode, C.byref(p)))
     return p
+
+
+def wideband_plan(rate: int) -> dict:
+    """dabgpu_wideband_plan: the wideband filter bank's block geometry at `rate` Hz (bin_hz, fft_in, fft_out, step_in, step_out,
+    taps); raises DabGpuError for a rate it does not support.  Needs no GPU."""
+    g = WidebandGeometry()
+    _check(load_library().dabgpu_wideband_plan(rate, C.byref(g)))
+    return {n: getattr(g, n) for n, _ in WidebandGeometry._fields_}
 
 
 def _ptr(a: np.ndarray) -> C.c_void_p:
@@ -460,10 +475,11 @@ class DabGpu:
                                           n_samples, block_size))
 
     def wideband_open(self, sample_rate: int, fmt, sources: Sequence[int], offsets_hz: Sequence[int], d_out: int,
-                      capacity_samples: int, n_sources: Optional[int] = None) -> "Wideband":
+                      capacity_samples: int, n_sources: Optional[int] = None, any_rate: bool = False) -> "Wideband":
         """dabgpu_wideband_open: channel c = ensemble of capture sources[c] at offsets_hz[c] from its centre, written as c32 to the
-        device buffer d_out ([channel][capacity_samples], e.g. a torch.complex64 tensor's data_ptr()) and fed to stream c."""
-        w = Wideband(self, sample_rate, fmt, sources, offsets_hz, d_out, capacity_samples, n_sources)
+        device buffer d_out ([channel][capacity_samples], e.g. a torch.complex64 tensor's data_ptr()) and fed to stream c.
+        any_rate=True: dabgpu_wideband_open_any_rate, which takes every rate wideband_plan() supports."""
+        w = Wideband(self, sample_rate, fmt, sources, offsets_hz, d_out, capacity_samples, n_sources, any_rate)
         self._wideband = w
         return w
 
@@ -538,7 +554,7 @@ class Wideband:
     """Wideband front end of one context (dabgpu_wideband_*): splits multi-ensemble captures into the context's streams."""
 
     def __init__(self, ctx: DabGpu, sample_rate: int, fmt, sources: Sequence[int], offsets_hz: Sequence[int], d_out: int,
-                 capacity_samples: int, n_sources: Optional[int] = None):
+                 capacity_samples: int, n_sources: Optional[int] = None, any_rate: bool = False):
         self.L, self.ctx = ctx.L, ctx
         self.format = WB_FORMATS[fmt] if isinstance(fmt, str) else int(fmt)
         self.n_sources = (max(sources) + 1 if len(sources) else 0) if n_sources is None else n_sources
@@ -546,7 +562,8 @@ class Wideband:
         off = (C.c_int * max(len(offsets_hz), 1))(*offsets_hz)
         cfg = WidebandConfig(sample_rate, self.format, self.n_sources, len(sources), src, off)
         self.h = C.c_void_p()
-        _check(self.L.dabgpu_wideband_open(ctx.h, C.byref(cfg), C.c_void_p(d_out), capacity_samples, C.byref(self.h)))
+        fn = self.L.dabgpu_wideband_open_any_rate if any_rate else self.L.dabgpu_wideband_open
+        _check(fn(ctx.h, C.byref(cfg), C.c_void_p(d_out), capacity_samples, C.byref(self.h)))
 
     def process(self, iq: np.ndarray, block_size: int = 65536) -> int:
         """iq: [n_sources, ...] host array, each row one source's raw samples (u8 / s8 / s16 I,Q pairs, f32 I,Q or complex64).

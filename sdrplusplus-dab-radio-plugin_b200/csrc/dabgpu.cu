@@ -10,6 +10,7 @@
 #include "../host/fic_autoconfig.hpp"
 #include "../host/capture_formats.hpp"
 #include <algorithm>
+#include <numeric>
 
 #define DABGPU_VERSION "dabgpu 0.1 (sm_100a)"
 
@@ -1417,6 +1418,9 @@ struct dabgpu_wideband {
     dabgpu_ctx* ctx = nullptr;   // null once the context was destroyed
     int D = 1, fmt = 0, bps = 2, n_sources = 0, n_channels = 0;
     long long fs = 0;
+    dabgpu_wideband_geometry geo{};   // block geometry (dabgpu_wideband_plan)
+    bool mixed = false;               // k_wideband_mixed (fft_in not a power of two) instead of k_wideband<D>
+    std::vector<int> radices;         // forward FFT passes of k_wideband_mixed
     DevBuf d_ring, d_H, d_twf, d_twi, d_dposf, d_dposi, d_chans, d_first;
     int ring_log2 = 0;
     size_t ring_cap = 0, out_cap = 0, headroom = 0;
@@ -1432,10 +1436,9 @@ static void wb_detach(dabgpu_wideband* w) {
     w->ctx = nullptr;
 }
 
-// Kaiser-windowed sinc low-pass, unit DC gain: scipy.signal.firwin(64 D + 1, 856e3, window=('kaiser', kaiser_beta(70)), fs)
-static void wb_design_taps(int D, std::vector<double>& h) {
-    const int T = 64 * D + 1;
-    const double c = 856e3 / (0.5 * 2048000.0 * D), beta = 0.1102 * (70.0 - 8.7), alpha = 0.5 * (T - 1);
+// Kaiser-windowed sinc low-pass, unit DC gain: scipy.signal.firwin(T, 856e3, window=('kaiser', kaiser_beta(70)), fs)
+static void wb_design_taps(int T, long long fs, std::vector<double>& h) {
+    const double c = 856e3 / (0.5 * double(fs)), beta = 0.1102 * (70.0 - 8.7), alpha = 0.5 * (T - 1);
     auto i0 = [](double x) {
         double sum = 1.0, term = 1.0;
         for (int k = 1; k < 200 && term > 1e-18 * sum; k++) { const double q = x / (2.0 * k); term *= q * q; sum += term; }
@@ -1452,12 +1455,21 @@ static void wb_design_taps(int D, std::vector<double>& h) {
     for (double& v : h) v /= sum;
 }
 
-// padded position of natural index k in the digit-reversed output of fft_cta<n> (DIF radices 8, 8, ..., then 4 or 2)
-static void wb_dpos(int n, std::vector<uint16_t>& dpos) {
+// DIF pass radices: those of fft_cta<n> for a power of two (8, 8, ..., then 4 or 2), else 8s, then 4 or 2, then 3s, then 5s
+// (fft_mixed_fwd)
+static std::vector<int> wb_radices(int n) {
     std::vector<int> radices;
     int m = n;
-    while (m % 8 == 0 && m > 1) { radices.push_back(8); m /= 8; }
-    if (m > 1) radices.push_back(m);
+    while (m % 8 == 0) { radices.push_back(8); m /= 8; }
+    if (m % 4 == 0) { radices.push_back(4); m /= 4; }
+    if (m % 2 == 0) { radices.push_back(2); m /= 2; }
+    while (m % 3 == 0) { radices.push_back(3); m /= 3; }
+    while (m % 5 == 0) { radices.push_back(5); m /= 5; }
+    return radices;
+}
+
+// padded position of natural index k in the digit-reversed output of an in-place DIF FFT of n points with these pass radices
+static void wb_dpos(int n, const std::vector<int>& radices, std::vector<uint16_t>& dpos) {
     dpos.resize(size_t(n));
     for (int k = 0; k < n; k++) {
         int a = 0, rem = n, kk = k;
@@ -1466,9 +1478,38 @@ static void wb_dpos(int n, std::vector<uint16_t>& dpos) {
     }
 }
 
-static void wb_roots(int n, std::vector<float2>& tw) {
-    tw.resize(size_t(n / 8));
-    for (int k = 0; k < n / 8; k++) tw[size_t(k)] = make_float2(float(cos(-2.0 * M_PI * k / n)), float(sin(-2.0 * M_PI * k / n)));
+// exp(-j 2 pi k / n), k < count
+static void wb_roots(int n, int count, std::vector<float2>& tw) {
+    tw.resize(size_t(count));
+    for (int k = 0; k < count; k++) tw[size_t(k)] = make_float2(float(cos(-2.0 * M_PI * k / n)), float(sin(-2.0 * M_PI * k / n)));
+}
+
+// block geometry at fs (include/dabgpu.h): among the bin spacings 4, 2 and 1 kHz that divide fs and give an N_in <= 8192 with
+// no prime factor above 5, the one with the fewest inverse-FFT operations per output sample
+static bool wb_plan(long long fs, dabgpu_wideband_geometry& out) {
+    if (fs < 2048000 || fs > 32768000) return false;
+    bool found = false;
+    double best = 0.0;
+    for (const int bin : {4000, 2000, 1000}) {
+        if (fs % bin) continue;
+        const int n_in = int(fs / bin);
+        int m = n_in;
+        for (const int p : {2, 3, 5})
+            while (m % p == 0) m /= p;
+        if (n_in > WB_MIX_MAX_FFT || m != 1) continue;
+        const int n_out = 2048000 / bin, T = int(2 * ((fs + 63999) / 64000) + 1);
+        const int ov_out = int(((long long)(T - 1) * 2048000 + fs - 1) / fs);
+        const long long g = 2048000 / std::gcd(fs, 2048000LL), l = g / std::gcd(g, 64LL) * 64;
+        const int step_out = int((n_out - ov_out) / l * l);
+        if (step_out <= 0) continue;
+        const double cost = 5.0 * n_out * std::log2(double(n_out)) / step_out;
+        if (found && cost >= best) continue;
+        found = true;
+        best = cost;
+        out.bin_hz = bin; out.fft_in = n_in; out.fft_out = n_out; out.taps = T;
+        out.step_out = step_out; out.step_in = int((long long)step_out * fs / 2048000);
+    }
+    return found;
 }
 
 // one entry per (D, format): W == nullptr sets the kernel's shared-memory attribute, otherwise launches nb blocks of every source
@@ -1487,16 +1528,66 @@ static const WbKernelFn kWbKernels[5][4] = {WB_ROW(1), WB_ROW(2), WB_ROW(4), WB_
 #undef WB_ROW
 static WbKernelFn wb_kernel(int D, int fmt) { return kWbKernels[__builtin_ctz(unsigned(D))][fmt]; }
 
+// the same for k_wideband_mixed, one entry per (NOUT, format)
+typedef int (*WbMixKernelFn)(const WbMixDev* W, unsigned long long block0, unsigned nb, int n_sources, cudaStream_t cs);
+template <int NOUT, int FMT> static int wb_mix_kernel_t(const WbMixDev* W, unsigned long long block0, unsigned nb, int n_sources, cudaStream_t cs) {
+    if (!W) {
+        CUDA_TRY(cudaFuncSetAttribute(k_wideband_mixed<NOUT, FMT>, cudaFuncAttributeMaxDynamicSharedMemorySize, WbMixCfg<NOUT>::SMEM_MAX));
+        return DABGPU_OK;
+    }
+    const int smem = (2 * OFDM_PAD(W->n_fft) + WbMixCfg<NOUT>::GROUP_FLOATS) * int(sizeof(float));
+    k_wideband_mixed<NOUT, FMT><<<dim3(nb, unsigned(n_sources)), WB_MIX_THREADS, smem, cs>>>(*W, block0);
+    CUDA_TRY(cudaGetLastError());
+    return DABGPU_OK;
+}
+#define WB_MIX_ROW(NOUT) {wb_mix_kernel_t<NOUT, 0>, wb_mix_kernel_t<NOUT, 1>, wb_mix_kernel_t<NOUT, 2>, wb_mix_kernel_t<NOUT, 3>}
+static const WbMixKernelFn kWbMixKernels[3][4] = {WB_MIX_ROW(512), WB_MIX_ROW(1024), WB_MIX_ROW(2048)};
+#undef WB_MIX_ROW
+static WbMixKernelFn wb_mix_kernel(int n_out, int fmt) { return kWbMixKernels[__builtin_ctz(unsigned(n_out / 512))][fmt]; }
+
+static int wb_check_ctx(const dabgpu_ctx* ctx) {
+    if (ctx->wb) return set_error(DABGPU_ERR_STATE, "a wideband front end is already open on this context");
+    if (ctx->cfg.iq_format != DABGPU_IQ_C32) return set_error(DABGPU_ERR_INVALID, "the wideband front end writes c32: the context needs DABGPU_IQ_C32");
+    return DABGPU_OK;
+}
+static int wb_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, const dabgpu_wideband_geometry& geo, void* d_out,
+                   size_t capacity, dabgpu_wideband** out);
+
 extern "C" {
+
+int dabgpu_wideband_plan(int sample_rate, dabgpu_wideband_geometry* g) {
+    if (!g) return set_error(DABGPU_ERR_INVALID, "null argument");
+    if (!wb_plan(sample_rate, *g))
+        return set_error(DABGPU_ERR_INVALID, "sample rate %d Hz is not supported: it must lie in [2 048 000, 32 768 000] and be "
+                         "N x 4000, 2000 or 1000 Hz with N <= 8192 and no prime factor of N above 5", sample_rate);
+    return DABGPU_OK;
+}
 
 int dabgpu_wideband_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, void* d_out, size_t capacity, dabgpu_wideband** out) {
     if (!ctx || !cfg || !d_out || !out) return set_error(DABGPU_ERR_INVALID, "null argument");
     *out = nullptr;
-    if (ctx->wb) return set_error(DABGPU_ERR_STATE, "a wideband front end is already open on this context");
-    if (ctx->cfg.iq_format != DABGPU_IQ_C32) return set_error(DABGPU_ERR_INVALID, "the wideband front end writes c32: the context needs DABGPU_IQ_C32");
+    if (int rc = wb_check_ctx(ctx)) return rc;
     const int D = cfg->sample_rate / 2048000;
     if (cfg->sample_rate <= 0 || cfg->sample_rate % 2048000 != 0 || (D != 1 && D != 2 && D != 4 && D != 8 && D != 16))
         return set_error(DABGPU_ERR_INVALID, "sample rate %d Hz is not 2.048 MHz x 1, 2, 4, 8 or 16", cfg->sample_rate);
+    dabgpu_wideband_geometry geo;
+    wb_plan(cfg->sample_rate, geo);
+    return wb_open(ctx, cfg, geo, d_out, capacity, out);
+}
+
+int dabgpu_wideband_open_any_rate(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, void* d_out, size_t capacity, dabgpu_wideband** out) {
+    if (!ctx || !cfg || !d_out || !out) return set_error(DABGPU_ERR_INVALID, "null argument");
+    *out = nullptr;
+    if (int rc = wb_check_ctx(ctx)) return rc;
+    dabgpu_wideband_geometry geo;
+    if (int rc = dabgpu_wideband_plan(cfg->sample_rate, &geo)) return rc;
+    return wb_open(ctx, cfg, geo, d_out, capacity, out);
+}
+
+}  // extern "C"
+
+static int wb_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, const dabgpu_wideband_geometry& geo, void* d_out,
+                   size_t capacity, dabgpu_wideband** out) {
     if (cfg->format < DABGPU_WB_RAW_U8 || cfg->format > DABGPU_WB_RAW_F32L) return set_error(DABGPU_ERR_INVALID, "bad wideband format %d", cfg->format);
     if (cfg->n_sources < 1 || cfg->n_sources > 65535) return set_error(DABGPU_ERR_INVALID, "n_sources %d out of range", cfg->n_sources);
     if (cfg->n_channels < 1 || cfg->n_channels > ctx->cfg.max_streams)
@@ -1508,19 +1599,23 @@ int dabgpu_wideband_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, voi
         if (std::llabs((long long)cfg->offset_hz[c]) + 768000 > fs / 2)
             return set_error(DABGPU_ERR_INVALID, "channel %d: offset %d Hz puts the ensemble outside +-fs/2", c, cfg->offset_hz[c]);
     }
-    const size_t min_cap = size_t(ctx->P.nb_frame_samples) + size_t(ctx->P.nb_null_period + ctx->P.nb_symbol_period) + 1024 + WB_OUT;
+    const size_t min_cap = size_t(ctx->P.nb_frame_samples) + size_t(ctx->P.nb_null_period + ctx->P.nb_symbol_period) + 1024 + size_t(geo.step_out);
     if (!is_pow2(capacity) || capacity < min_cap || capacity > (size_t(1) << 30))
         return set_error(DABGPU_ERR_INVALID, "capacity %zu: must be a power of two in [%zu, 2^30]", capacity, min_cap);
 
     dabgpu_wideband* w = new dabgpu_wideband();
-    w->D = D; w->fmt = cfg->format; w->fs = fs;
+    w->D = int(fs / 2048000); w->fmt = cfg->format; w->fs = fs;
+    w->geo = geo;
+    w->mixed = !is_pow2(size_t(geo.fft_in));
     w->bps = (cfg->format == DABGPU_WB_RAW_F32L) ? 8 : (cfg->format == DABGPU_WB_RAW_S16L) ? 4 : 2;
     w->n_sources = cfg->n_sources; w->n_channels = cfg->n_channels;
     w->out_cap = capacity;
     w->headroom = ofdm_ring_headroom(ctx->P, capacity);
-    w->max_pass_blocks = std::min<unsigned long long>(512, w->headroom / WB_OUT);
+    w->max_pass_blocks = std::min<unsigned long long>(512, w->headroom / size_t(geo.step_out));
     w->d_out = static_cast<float2*>(d_out);
-    while ((size_t(1) << w->ring_log2) < (w->max_pass_blocks + 2) * WB_OUT * size_t(D)) w->ring_log2++;
+    // the history of the first block of a pass, the pass, and the input held back until the next block is complete
+    const size_t ov_in = size_t(geo.fft_in - geo.step_in);
+    while ((size_t(1) << w->ring_log2) < ov_in + (w->max_pass_blocks + 1) * size_t(geo.step_in)) w->ring_log2++;
     w->ring_cap = size_t(1) << w->ring_log2;
 
     // channels grouped by source, in channel order
@@ -1531,18 +1626,19 @@ int dabgpu_wideband_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, voi
         for (int c = 0; c < cfg->n_channels; c++) {
             if (cfg->source[c] != s) continue;
             const int f = cfg->offset_hz[c];
-            const int bin = f >= 0 ? (f + 2000) / 4000 : -((2000 - f) / 4000);   // round half away from zero
-            chans.push_back(WbChan{bin, f - 4000 * bin, c, 0});
+            const int half = geo.bin_hz / 2;
+            const int bin = f >= 0 ? (f + half) / geo.bin_hz : -((half - f) / geo.bin_hz);   // round half away from zero
+            chans.push_back(WbChan{bin, f - geo.bin_hz * bin, c, 0});
         }
     }
     first[size_t(cfg->n_sources)] = int(chans.size());
 
-    const int N = 512 * D;
+    const int N = geo.fft_in, NO = geo.fft_out;
     std::vector<double> h;
-    wb_design_taps(D, h);
-    std::vector<float2> H(WB_IFFT), twf, twi;
-    for (int i = 0; i < WB_IFFT; i++) {
-        const int u = i < WB_IFFT / 2 ? i : i - WB_IFFT;
+    wb_design_taps(geo.taps, fs, h);
+    std::vector<float2> H(static_cast<size_t>(NO)), twf, twi;
+    for (int i = 0; i < NO; i++) {
+        const int u = i < NO / 2 ? i : i - NO;
         double re = 0.0, im = 0.0;
         for (size_t n = 0; n < h.size(); n++) {
             const long long k = ((long long)u * (long long)n) % N;
@@ -1551,11 +1647,12 @@ int dabgpu_wideband_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, voi
         }
         H[size_t(i)] = make_float2(float(re / N), float(im / N));
     }
-    wb_roots(N, twf);
-    wb_roots(WB_IFFT, twi);
+    wb_roots(N, w->mixed ? N : N / 8, twf);
+    wb_roots(NO, NO / 8, twi);
+    w->radices = wb_radices(N);
     std::vector<uint16_t> dposf, dposi;
-    wb_dpos(N, dposf);
-    wb_dpos(WB_IFFT, dposi);
+    wb_dpos(N, w->radices, dposf);
+    wb_dpos(NO, wb_radices(NO), dposi);
 
     int rc = DABGPU_OK;
 #define WB_TRY(expr) do { if ((rc = (expr))) { wb_detach(w); delete w; return rc; } } while (0)
@@ -1578,7 +1675,7 @@ int dabgpu_wideband_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, voi
         e = cudaMemcpy(u.first->p, u.second.first, u.second.second, cudaMemcpyHostToDevice);
         if (e != cudaSuccess) { wb_detach(w); delete w; return set_error(DABGPU_ERR_CUDA, "cudaMemcpy: %s", cudaGetErrorString(e)); }
     }
-    WB_TRY(wb_kernel(D, w->fmt)(nullptr, 0, 0, 0, ctx->stream));
+    WB_TRY(w->mixed ? wb_mix_kernel(NO, w->fmt)(nullptr, 0, 0, 0, ctx->stream) : wb_kernel(w->D, w->fmt)(nullptr, 0, 0, 0, ctx->stream));
     WB_TRY(ofdm_attach(ctx->ofdm, d_out, capacity, capacity, ctx->stream));
 #undef WB_TRY
     w->ctx = ctx;
@@ -1587,6 +1684,8 @@ int dabgpu_wideband_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, voi
     return DABGPU_OK;
 }
 
+extern "C" {
+
 int dabgpu_wideband_process(dabgpu_wideband* w, const void* iq_host, size_t stride, size_t n_samples, int block_size, size_t* n_out) {
     if (!w) return set_error(DABGPU_ERR_INVALID, "null wideband front end");
     if (n_out) *n_out = 0;
@@ -1594,25 +1693,29 @@ int dabgpu_wideband_process(dabgpu_wideband* w, const void* iq_host, size_t stri
     if (!ctx) return set_error(DABGPU_ERR_STATE, "the context of this wideband front end was destroyed");
     if (!iq_host && n_samples) return set_error(DABGPU_ERR_INVALID, "null input");
     if (w->n_sources > 1 && stride < n_samples * size_t(w->bps)) return set_error(DABGPU_ERR_INVALID, "source stride %zu is shorter than a source", stride);
-    const unsigned long long blk_in = WB_OUT * (unsigned long long)w->D, hist = 64ull * w->D;
-    const size_t new_out = size_t((w->n_in + n_samples) / blk_in - w->blocks_done) * WB_OUT;
+    const unsigned long long blk_in = (unsigned long long)w->geo.step_in, hist = (unsigned long long)(w->geo.fft_in - w->geo.step_in);
+    const size_t blk_out = size_t(w->geo.step_out);
+    const size_t new_out = size_t((w->n_in + n_samples) / blk_in - w->blocks_done) * blk_out;
     const size_t bs = block_size > 0 ? size_t(block_size) : std::max<size_t>(new_out, 1);
-    if (bs + WB_OUT > w->headroom)
+    if (bs + blk_out > w->headroom)
         return set_error(DABGPU_ERR_INVALID, "block_size %zu does not fit the output ring (%zu samples of headroom)", bs, w->headroom);
     CUDA_TRY(cudaSetDevice(ctx->cfg.device));
     CUDA_TRY(join_if_many_frames(ctx, long(std::min<size_t>(new_out, 1ul << 40))));
     ctx->ofdm.demod_ctas_cap = ctx->dp_pending ? 3 : 0;   // a channel decode is running on its stream: share the SMs with it
-    const WbKernelFn kern = wb_kernel(w->D, w->fmt);
     WbDev W;
     W.ring = w->d_ring.as<uint8_t>(); W.ring_log2 = w->ring_log2; W.ring_mask = w->ring_cap - 1;
     W.out = w->d_out; W.out_cap = w->out_cap;
     W.H = w->d_H.as<float2>(); W.tw_fwd = w->d_twf.as<float2>(); W.tw_inv = w->d_twi.as<float2>();
     W.dpos_fwd = w->d_dposf.as<uint16_t>(); W.dpos_inv = w->d_dposi.as<uint16_t>();
     W.chans = w->d_chans.as<WbChan>(); W.chan_first = w->d_first.as<int>(); W.fs = w->fs;
+    WbMixDev M;
+    M.w = W; M.n_fft = w->geo.fft_in; M.step_in = w->geo.step_in; M.ov_in = int(hist); M.step_out = w->geo.step_out;
+    M.n_pass = int(w->radices.size());
+    for (int p = 0; p < WB_MIX_MAX_PASSES; p++) M.radix[p] = p < M.n_pass ? w->radices[size_t(p)] : 1;
     const uint8_t* src = static_cast<const uint8_t*>(iq_host);
     size_t done = 0;
     for (;;) {
-        // input: the ring keeps everything from the first sample the next block reads (its 64 D samples of history)
+        // input: the ring keeps everything from the first sample the next block reads (its fft_in - step_in samples of history)
         const unsigned long long keep = w->blocks_done * blk_in >= hist ? w->blocks_done * blk_in - hist : 0;
         const size_t take = std::min<size_t>(n_samples - done, size_t(keep + w->ring_cap - w->n_in));
         for (size_t left = take, off = done; left > 0;) {
@@ -1624,16 +1727,17 @@ int dabgpu_wideband_process(dabgpu_wideband* w, const void* iq_host, size_t stri
         }
         done += take;
         // filter: whole blocks, never more than the OFDM stage's headroom ahead of what it consumed
-        const size_t pending = size_t(w->blocks_done * WB_OUT - w->out_consumed);
-        const unsigned long long nb = std::min({w->n_in / blk_in - w->blocks_done, w->max_pass_blocks, (unsigned long long)((w->headroom - pending) / WB_OUT)});
+        const size_t pending = size_t(w->blocks_done * blk_out - w->out_consumed);
+        const unsigned long long nb = std::min({w->n_in / blk_in - w->blocks_done, w->max_pass_blocks, (unsigned long long)((w->headroom - pending) / blk_out)});
         if (nb) {
-            int rc = kern(&W, w->blocks_done, unsigned(nb), w->n_sources, ctx->stream);
+            int rc = w->mixed ? wb_mix_kernel(w->geo.fft_out, w->fmt)(&M, w->blocks_done, unsigned(nb), w->n_sources, ctx->stream)
+                              : wb_kernel(w->D, w->fmt)(&W, w->blocks_done, unsigned(nb), w->n_sources, ctx->stream);
             if (rc) return rc;
             ctx->launches++;
             w->blocks_done += nb;
         }
         // OFDM_Demod::Process over the new outputs in blocks of bs; a partial block only at the end of the call
-        const size_t avail = size_t(w->blocks_done * WB_OUT - w->out_consumed);
+        const size_t avail = size_t(w->blocks_done * blk_out - w->out_consumed);
         const bool last = done == n_samples && w->n_in / blk_in == w->blocks_done;
         const size_t present = last ? avail : (avail / bs) * bs;
         if (present) {

@@ -652,15 +652,22 @@ def periodic_frames(mode: int, subchannels: Sequence[Subchannel], seed: int, per
 
 def wideband_capture(mode: int, ensembles: Sequence[np.ndarray], D: int, offsets_hz: Sequence[int], snr_db: float = 15.0,
                      cfo_hz: Sequence[float] = (), shifts: Sequence[int] = (), gains_db: Sequence[float] = (), seed: int = 0,
-                     mask_hz: float = 800e3) -> np.ndarray:
-    """One period of a periodic multi-ensemble capture at D x 2.048 MS/s (complex128; np.take(..., mode="wrap") continues it).
+                     mask_hz: float = 800e3, sample_rate: Optional[int] = None) -> np.ndarray:
+    """One period of a periodic multi-ensemble capture at D x 2.048 MS/s, or at sample_rate Hz when given (then D is ignored; the
+    period must be a whole number of samples at that rate, as it is for 5 Mode I frames at every multiple of 25 Hz)
+    (complex128; np.take(..., mode="wrap") continues it).
     ensembles[k] = the coded frames of one period of periodic_frames(); ensemble k gets AWGN at snr_db, a band limit of
     +-mask_hz (a transmitter's spectrum mask), a CFO of cfo_hz[k] and a time shift of shifts[k] samples (both cyclic), the gain
     gains_db[k], and sits offsets_hz[k] above the capture centre.  Built in the frequency domain over the whole period, so the
     CFO and the offsets are rounded to the period's bin spacing (2.048 MHz / period samples, about 2 Hz)."""
     p = MODES[mode]
     L = len(ensembles[0]) * p.nb_frame_samples
-    M = D * L
+    if sample_rate is None:
+        M, scale = D * L, D
+    else:
+        assert (L * sample_rate) % 2048000 == 0, "the period is not a whole number of samples at this rate"
+        M = L * sample_rate // 2048000
+        scale = M / L
     Y = np.zeros(M, dtype=np.complex128)
     fb = np.fft.fftfreq(L, 1.0 / L).astype(np.int64)
     keep = np.nonzero(np.abs(fb) * 2048000.0 / L <= mask_hz)[0]
@@ -675,7 +682,7 @@ def wideband_capture(mode: int, ensembles: Sequence[np.ndarray], D: int, offsets
         X = np.fft.fft(x)
         shift = int(round(f * L / 2048000.0)) + (int(round(cfo_hz[k] * L / 2048000.0)) if k < len(cfo_hz) else 0)
         g = 10 ** ((gains_db[k] if k < len(gains_db) else 0.0) / 20)
-        np.add.at(Y, (fb[keep] + shift) % M, X[keep] * (D * g))
+        np.add.at(Y, (fb[keep] + shift) % M, X[keep] * (scale * g))
     return np.fft.ifft(Y)
 
 
