@@ -213,6 +213,7 @@ DABGPU_API int dabgpu_wideband_open_any_rate(dabgpu_ctx* ctx, const dabgpu_wideb
  * block_size (<= 0: one block).  Returns once the host buffer may be reused; *n_out = output samples per channel this call. */
 DABGPU_API int dabgpu_wideband_process(dabgpu_wideband* w, const void* iq_host, size_t source_stride_bytes, size_t n_samples,
                                        int block_size, size_t* n_out);
+/* Closes the front end once every queued call and the copy-out of every ticket in flight have finished. */
 DABGPU_API int dabgpu_wideband_close(dabgpu_wideband* w);
 
 /* On_OFDM_Frame: number of undelivered soft-bit frames per stream, then copy them out in order.
@@ -276,6 +277,32 @@ DABGPU_API int dabgpu_submit(dabgpu_ctx* ctx, const dabgpu_step* step, uint64_t*
 DABGPU_API int dabgpu_wait(dabgpu_ctx* ctx, uint64_t ticket);
 /* byte offset and length of sub-channel sub_index inside one CIF row of the msc_host arena */
 DABGPU_API int dabgpu_msc_get_layout(dabgpu_ctx* ctx, int stream, int sub_index, int* offset, int* bytes_per_cif);
+
+/* Pipelined wideband front end (dabgpu_wideband_open above, the pipeline of dabgpu_submit).
+ *
+ * dabgpu_wideband_reserve sizes the device input ring for tickets of up to max_submit_samples raw samples per source: it holds
+ * the fft_in - step_in samples of history of the next block, fewer than step_in samples held back until that block is
+ * complete, and two tickets, rounded up to a power of two (one 96 ms frame per ticket at 16.384 MS/s raw_s16l for 128 sources
+ * is about 2 GB).  Valid only before the first input (dabgpu_wideband_process or _submit), DABGPU_ERR_STATE after it; a failed
+ * allocation is reported here (DABGPU_ERR_NOMEM) and leaves the front end as it was.  Outputs do not depend on the ring size.
+ *
+ * dabgpu_wideband_submit queues one ticket without blocking: (1) the copy of step->n_samples (1 .. the reserved size) raw
+ * samples of every source (source s at step->iq_host + s * step->iq_stride_bytes) into the ring on the copy stream, (2) the
+ * filter bank and OFDM_Demod::Process over every channel as dabgpu_wideband_process runs them (Process() blocks of
+ * step->block_size), then, if step->run_chan_decode != 0, one dabgpu_chan_decode of channels [first_stream, first_stream +
+ * n_streams) on the compute stream, (3) the copy of the non-NULL result pointers of step on the copy-out stream, in the layouts
+ * of dabgpu_submit with row 0 = channel first_stream.  Tickets retire with dabgpu_wait and share the context's
+ * DABGPU_PIPELINE_DEPTH slots.  Contract: after the same sequence of n_samples and block_size, ticket i leaves the device
+ * state and the copied arenas exactly as dabgpu_wideband_process(n_i) followed by dabgpu_chan_decode(first, n) would.
+ * produced_host[c] is 1 when channel first_stream + c emitted at least one frame during this ticket (which can span several
+ * OFDM runs), and frames_host row c then holds the newest such frame.
+ *
+ * Ordering: the input must stay valid until the ticket was waited for and be pinned (dabgpu_host_alloc) for the copies to
+ * overlap.  The upload of ticket t + 1 overlaps the compute of ticket t; the upload of ticket t + 2 waits for the compute of
+ * ticket t.  dabgpu_wideband_process and _submit may be mixed in any order: each call's work is ordered after the previous
+ * one's.  dabgpu_submit keeps returning DABGPU_ERR_STATE while a front end is attached. */
+DABGPU_API int dabgpu_wideband_reserve(dabgpu_wideband* w, size_t max_submit_samples);
+DABGPU_API int dabgpu_wideband_submit(dabgpu_wideband* w, const dabgpu_step* step, uint64_t* ticket);
 
 /* ---------------------------------------------------------------------------------------------
  * Viterbi.  Replaces DAB_Viterbi_Decoder::{reset,update,chainback}

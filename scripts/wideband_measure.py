@@ -3,8 +3,12 @@ streams, one transmission frame (96 ms of signal) per step.  With --rate, captur
 supports, through dabgpu_wideband_open_any_rate) with the Band III offsets (multiples of 1.712 MHz) that fit it and enough
 sources for about 1 024 streams, e.g. 204 sources x 5 ensembles at 10 MS/s.  Prints one JSON line per input format with the
 step time of process + chan_decode (CUDA events), the channelizer kernel time from torch.profiler in a separate run, the
-achieved FLOP/s and bytes/s of the kernel, the host->device rate and the rate's plan.  Needs a GPU; writes nothing but the
-traces asked for with --out."""
+achieved FLOP/s and bytes/s of the kernel, the host->device rate and the rate's plan.  With --pipelined the same run also drives
+the workload through dabgpu_wideband_reserve + dabgpu_wideband_submit / dabgpu_wait on a second context, two tickets in flight,
+each with its channel decode and the channel status and MSC bytes copied into pinned buffers, as a receiver would, and adds the
+wall-clock time per ticket, the real-time streams it gives, the pinned host->device time of a step and whether the counter
+deltas over the timed tickets equal those of the timed serial steps.  Needs a GPU; writes nothing but the traces asked for with
+--out."""
 import argparse
 import importlib
 import json
@@ -50,7 +54,66 @@ def design_counts(n_in, bps, plan, offs, n_src):
     return float(flop), float(byts)
 
 
-def run(fmt, steps, warmup, out_dir, rate=DEFAULT_RATE):
+COUNTERS = ("frames_demodulated", "fibs_crc_ok", "fibs_total", "superframes_ok", "superframes_rs_fail", "au_ok", "au_crc_fail")
+
+
+def delta(c1, c0):
+    return {k: c1[k] - c0[k] for k in COUNTERS}
+
+
+def run_pipelined(dab, h, hb, S, E, offs, subs, fmt, rate, step, bps, steps, warmup, out_dir):
+    """the serial leg's steps as tickets of dabgpu_wideband_submit on a fresh context: (wall-clock ms per ticket, counter deltas
+    over the timed tickets)"""
+    import torch
+    g = dab.DabGpu(mode=1, max_streams=S * E, iq_format=dab.IQ_C32)
+    out = torch.zeros((S * E, 1 << 19), dtype=torch.complex64, device="cuda:0")
+    w = g.wideband_open(rate, fmt, [s for s in range(S) for _ in offs], offs * S, out.data_ptr(), 1 << 19,
+                        any_rate=rate != DEFAULT_RATE)
+    for c in range(S * E):
+        g.msc_configure(c, subs)
+    w.reserve(step)
+    nc = g.P.nb_cifs
+    outs = [(dab.HostBuffer(S * E * 8), dab.HostBuffer(S * E * nc * dab.CIF_OUT_STRIDE)) for _ in range(2)]
+    row = h.strides[0]
+
+    def submit(i):
+        st, msc = outs[i % 2]
+        return w.submit(hb.ptr.value + (i % PERIOD) * step * bps, row, step, block_size=65536, run_chan_decode=True,
+                        chan_status_host=st.ptr.value, msc_host=msc.ptr.value)
+
+    def drive(first, n, stamps=None):
+        prev = None
+        for i in range(first, first + n):
+            t = submit(i)
+            if prev is not None:
+                g.wait(prev)
+                if stamps is not None:
+                    stamps.append(time.perf_counter())
+            prev = t
+        g.wait(prev)
+        if stamps is not None:
+            stamps.append(time.perf_counter())
+
+    drive(0, warmup)
+    c0 = g.counters()
+    stamps = [time.perf_counter()]
+    drive(warmup, steps, stamps)
+    c1 = g.counters()
+    if out_dir:
+        from torch.profiler import profile, ProfilerActivity
+        with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
+            drive(warmup + steps, 10)
+        name = f"wideband_pipelined_trace_{fmt}.json" if rate == DEFAULT_RATE else f"wideband_pipelined_trace_{rate}_{fmt}.json"
+        prof.export_chrome_trace(os.path.join(out_dir, name))
+    w.close()
+    g.close()
+    for a, b in outs:
+        a.close()
+        b.close()
+    return np.diff(np.array(stamps)) * 1e3, delta(c1, c0)
+
+
+def run(fmt, steps, warmup, out_dir, rate=DEFAULT_RATE, pipelined=False):
     import torch
     dab = importlib.import_module(PKG)
     tx = importlib.import_module(PKG + ".synth.dabtx")
@@ -91,6 +154,7 @@ def run(fmt, steps, warmup, out_dir, rate=DEFAULT_RATE):
     for i in range(warmup):
         one(i)
     g.sync()
+    c_timed = g.counters()
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
     stream = torch.cuda.ExternalStream(g.cuda_stream)
     ms = []
@@ -103,6 +167,7 @@ def run(fmt, steps, warmup, out_dir, rate=DEFAULT_RATE):
         ev[1].synchronize()
         ms.append(ev[0].elapsed_time(ev[1]))
     c = g.counters()
+    serial_delta = delta(c, c_timed)
     # H2D alone: the same bytes as one step, pinned
     d_tmp = torch.empty(S * step * bps, dtype=torch.uint8, device="cuda:0")
     src = torch.from_numpy(h[:, :step * bps].reshape(-1))
@@ -136,6 +201,22 @@ def run(fmt, steps, warmup, out_dir, rate=DEFAULT_RATE):
                superframes_rs_fail=c["superframes_rs_fail"], au_crc_fail=c["au_crc_fail"])
     w.close()
     g.close()
+    if pipelined:
+        # the same step's bytes from the pinned buffer (the line above copies a pageable copy of them)
+        d_tmp = torch.empty(S * step * bps, dtype=torch.uint8, device="cuda:0")
+        src = torch.from_numpy(hb.array[:S * step * bps])
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        for _ in range(5):
+            d_tmp.copy_(src, non_blocking=True)
+        torch.cuda.synchronize()
+        pinned_h2d_ms = (time.perf_counter() - t0) / 5 * 1e3
+        del d_tmp
+        pms, pipe_delta = run_pipelined(dab, h, hb, S, E, offs, subs, fmt, rate, step, bps, steps, warmup, out_dir)
+        res.update(pipelined_tickets=steps, pipelined_step_ms_median=float(np.median(pms)), pipelined_step_ms_p90=float(np.percentile(pms, 90)),
+                   pipelined_step_ms_mean=float(np.mean(pms)), pipelined_realtime_streams=S * E * (FS / 2048.0) / float(np.median(pms)),
+                   pinned_h2d_ms_per_step=pinned_h2d_ms, serial_counter_deltas=serial_delta, pipelined_counter_deltas=pipe_delta,
+                   pipelined_counters_equal=pipe_delta == serial_delta)
     hb.close()
     return res
 
@@ -147,6 +228,7 @@ def main():
     ap.add_argument("--formats", default="raw_s16l,raw_s8")
     ap.add_argument("--rate", type=int, default=DEFAULT_RATE, help="capture rate in Hz (default: 16.384 MHz, 128 x 8 ensembles)")
     ap.add_argument("--out", default=None, help="directory for the profiler's chrome traces (none written if omitted)")
+    ap.add_argument("--pipelined", action="store_true", help="also time the workload through reserve + submit / wait (two tickets in flight)")
     a = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -154,7 +236,7 @@ def main():
     if a.out:
         os.makedirs(a.out, exist_ok=True)
     for fmt in a.formats.split(","):
-        print(json.dumps(run(fmt, a.steps, a.warmup, a.out, a.rate)), flush=True)
+        print(json.dumps(run(fmt, a.steps, a.warmup, a.out, a.rate, a.pipelined)), flush=True)
 
 
 if __name__ == "__main__":

@@ -117,7 +117,7 @@ EXPORTS = [
     "dabgpu_host_alloc", "dabgpu_host_free", "dabgpu_ofdm_get_frame_data_vec", "dabgpu_ofdm_get_correlation_buffer", "dabgpu_autocfg_applied", "dabgpu_msc_add_subchannel", "dabgpu_msc_remove_subchannel", "dabgpu_chan_join",
     "dabgpu_autocfg_apply", "dabgpu_ofdm_get_response", "dabgpu_ofdm_get_frame_fft", "dabgpu_iq_convert", "dabgpu_softbits_to_bytes", "dabgpu_bytes_to_softbits",
     "dabgpu_packet_fec_decode", "dabgpu_wideband_open", "dabgpu_wideband_process", "dabgpu_wideband_close",
-    "dabgpu_wideband_plan", "dabgpu_wideband_open_any_rate",
+    "dabgpu_wideband_plan", "dabgpu_wideband_open_any_rate", "dabgpu_wideband_reserve", "dabgpu_wideband_submit",
 ]
 
 _lib = None
@@ -199,6 +199,8 @@ def load_library() -> C.CDLL:
     L.dabgpu_wideband_close.argtypes = [C.c_void_p]
     L.dabgpu_wideband_plan.argtypes = [C.c_int, C.POINTER(WidebandGeometry)]
     L.dabgpu_wideband_open_any_rate.argtypes = L.dabgpu_wideband_open.argtypes
+    L.dabgpu_wideband_reserve.argtypes = [C.c_void_p, C.c_size_t]
+    L.dabgpu_wideband_submit.argtypes = [C.c_void_p, C.POINTER(Step), C.POINTER(C.c_uint64)]
     _lib = L
     return L
 
@@ -247,6 +249,16 @@ def wideband_plan(rate: int) -> dict:
 
 def _ptr(a: np.ndarray) -> C.c_void_p:
     return C.c_void_p(a.ctypes.data)
+
+
+def _step(iq_ptr, iq_stride_bytes, n_samples, block_size, first_stream, n_streams, run_chan_decode, out_ptrs) -> Step:
+    st = Step()
+    st.iq_host, st.iq_stride_bytes = iq_ptr, iq_stride_bytes
+    st.first_stream, st.n_streams = first_stream, n_streams
+    st.n_samples, st.block_size, st.run_chan_decode = n_samples, block_size, int(run_chan_decode)
+    for k, v in out_ptrs.items():
+        setattr(st, k, v)
+    return st
 
 
 class DabGpu:
@@ -487,13 +499,8 @@ class DabGpu:
                n_streams: Optional[int] = None, run_chan_decode: bool = False, **out_ptrs) -> int:
         """dabgpu_submit: queue H2D + OFDM (+ channel decode) + D2H without blocking; returns the ticket.
         out_ptrs: frames_host, produced_host, msc_host, msc_valid_host, fic_host, fic_crc_host, chan_status_host (raw addresses)."""
-        st = Step()
-        st.iq_host, st.iq_stride_bytes = iq_ptr, iq_stride_bytes
-        st.first_stream = first_stream
-        st.n_streams = self.max_streams - first_stream if n_streams is None else n_streams
-        st.n_samples, st.block_size, st.run_chan_decode = n_samples, block_size, int(run_chan_decode)
-        for k, v in out_ptrs.items():
-            setattr(st, k, v)
+        st = _step(iq_ptr, iq_stride_bytes, n_samples, block_size, first_stream,
+                   self.max_streams - first_stream if n_streams is None else n_streams, run_chan_decode, out_ptrs)
         t = C.c_uint64(0)
         _check(self.L.dabgpu_submit(self.h, C.byref(st), C.byref(t)))
         return int(t.value)
@@ -558,6 +565,7 @@ class Wideband:
         self.L, self.ctx = ctx.L, ctx
         self.format = WB_FORMATS[fmt] if isinstance(fmt, str) else int(fmt)
         self.n_sources = (max(sources) + 1 if len(sources) else 0) if n_sources is None else n_sources
+        self.n_channels = len(sources)
         src = (C.c_int * max(len(sources), 1))(*sources)
         off = (C.c_int * max(len(offsets_hz), 1))(*offsets_hz)
         cfg = WidebandConfig(sample_rate, self.format, self.n_sources, len(sources), src, off)
@@ -573,6 +581,24 @@ class Wideband:
         n_out = C.c_size_t(0)
         _check(self.L.dabgpu_wideband_process(self.h, C.c_void_p(iq.ctypes.data), iq.strides[0], n, block_size, C.byref(n_out)))
         return n_out.value
+
+    def reserve(self, max_samples: int) -> None:
+        """dabgpu_wideband_reserve: size the input ring for submit() tickets of up to max_samples raw samples per source.
+        Only before the first input."""
+        _check(self.L.dabgpu_wideband_reserve(self.h, max_samples))
+
+    def submit(self, iq_ptr: int, source_stride_bytes: int, n_samples: int, block_size: int = 65536, first_stream: int = 0,
+               n_streams: Optional[int] = None, run_chan_decode: bool = False, **out_ptrs) -> int:
+        """dabgpu_wideband_submit: queue the upload of n_samples raw samples per source (source s at iq_ptr + s *
+        source_stride_bytes, pinned host memory that stays valid until the ticket is waited for), the filter bank and OFDM over
+        every channel, the channel decode of channels [first_stream, first_stream + n_streams) if run_chan_decode, and the
+        copy-out of out_ptrs (as DabGpu.submit, rows from first_stream) without blocking.  Returns the ticket; retire it with
+        DabGpu.wait."""
+        st = _step(iq_ptr, source_stride_bytes, n_samples, block_size, first_stream,
+                   self.n_channels - first_stream if n_streams is None else n_streams, run_chan_decode, out_ptrs)
+        t = C.c_uint64(0)
+        _check(self.L.dabgpu_wideband_submit(self.h, C.byref(st), C.byref(t)))
+        return int(t.value)
 
     def close(self):
         if getattr(self, "h", None):

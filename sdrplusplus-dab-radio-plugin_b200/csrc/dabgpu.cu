@@ -75,6 +75,7 @@ struct dabgpu_ctx {
     struct PipeSlot {
         cudaEvent_t h2d_done = nullptr, compute_done = nullptr, d2h_done = nullptr;
         DevBuf d_stage, d_produced;
+        DevBuf d_written0;   // frames_written of the ticket's streams before its first OFDM run (dabgpu_wideband_submit)
         uint64_t ticket = 0;
         bool busy = false;
     } pipe[DABGPU_PIPELINE_DEPTH];
@@ -328,6 +329,7 @@ void dabgpu_ctx_destroy(dabgpu_ctx* ctx) {
         if (sl.d2h_done) cudaEventDestroy(sl.d2h_done);
         sl.d_stage.release();
         sl.d_produced.release();
+        sl.d_written0.release();
     }
     if (ctx->s_dp) { cudaStreamSynchronize(ctx->s_dp); cudaStreamDestroy(ctx->s_dp); }
     if (ctx->ev_dp) cudaEventDestroy(ctx->ev_dp);
@@ -1329,45 +1331,38 @@ static int pipe_init(dabgpu_ctx* ctx) {
     return DABGPU_OK;
 }
 
-int dabgpu_submit(dabgpu_ctx* ctx, const dabgpu_step* st, uint64_t* ticket) {
-    if (!ctx || !st || !ticket) return set_error(DABGPU_ERR_INVALID, "null argument");
-    int rc = check_stream_range(ctx, st->first_stream, st->n_streams);
-    if (rc) return rc;
-    if (!st->iq_host || st->n_samples <= 0 || st->n_streams == 0) return set_error(DABGPU_ERR_INVALID, "bad IQ buffer");
-    OfdmState& O = ctx->ofdm;
-    if (O.external_ring) return set_error(DABGPU_ERR_STATE, "a device input buffer is attached: use dabgpu_ofdm_advance");
-    CUDA_TRY(cudaSetDevice(ctx->cfg.device));
+}  // extern "C"
+
+// The slot of the next ticket.  When the caller has not waited for the ticket that used it DABGPU_PIPELINE_DEPTH tickets ago,
+// this waits for it: everything that ticket queued has then finished, its compute included.
+static int pipe_acquire(dabgpu_ctx* ctx, dabgpu_ctx::PipeSlot** out) {
+    int rc;
     if ((rc = pipe_init(ctx))) return rc;
-    CUDA_TRY(join_if_many_frames(ctx, st->n_samples));
-    const uint64_t t = ctx->next_ticket;
-    auto& sl = ctx->pipe[t % DABGPU_PIPELINE_DEPTH];
-    auto& prev = ctx->pipe[(t + DABGPU_PIPELINE_DEPTH - 1) % DABGPU_PIPELINE_DEPTH];
-    // the copy of this step overlaps the compute of the previous one: together they must fit the ring headroom
-    const size_t prev_samples = ctx->pipe_recent_samples[(t + DABGPU_PIPELINE_DEPTH - 1) % DABGPU_PIPELINE_DEPTH];
-    if (size_t(st->n_samples) + prev_samples > ofdm_ring_headroom(O))
-        return set_error(DABGPU_ERR_INVALID, "n_samples %d (+%zu in flight) exceeds the IQ ring headroom %zu: raise ring_samples", st->n_samples,
-                         prev_samples, ofdm_ring_headroom(O));
+    auto& sl = ctx->pipe[ctx->next_ticket % DABGPU_PIPELINE_DEPTH];
     if (sl.busy) { CUDA_TRY(cudaEventSynchronize(sl.d2h_done)); sl.busy = false; }
+    *out = &sl;
+    return DABGPU_OK;
+}
+
+// Everything of a ticket after its OFDM stage, which the caller has queued on the compute stream: the newest frame of every
+// stream that produced one (during the last OFDM run, or since the counters in d_written0 when given), the channel decode,
+// and the device->host copies of the non-NULL result pointers of st on the copy-out stream.
+static int pipe_finish(dabgpu_ctx* ctx, dabgpu_ctx::PipeSlot& sl, const dabgpu_step* st, const uint32_t* d_written0, uint64_t* ticket) {
+    int rc;
+    OfdmState& O = ctx->ofdm;
     const int n = st->n_streams, first = st->first_stream;
     const size_t fb = size_t(ctx->P.nb_frame_bits);
-    // (1) copy in; the ring region being overwritten was last read by the compute two tickets ago, which d2h_done covers
-    if (prev.busy) CUDA_TRY(cudaStreamWaitEvent(ctx->s_h2d, prev.h2d_done, 0));
-    if ((rc = ofdm_upload(O, st->iq_host, st->iq_stride_bytes, first, n, 0, size_t(st->n_samples), ctx->s_h2d))) return rc;
-    CUDA_TRY(cudaEventRecord(sl.h2d_done, ctx->s_h2d));
-    // (2) compute
-    CUDA_TRY(cudaStreamWaitEvent(ctx->stream, sl.h2d_done, 0));
-    const int bs = st->block_size > 0 ? st->block_size : st->n_samples;
-    ctx->ofdm.demod_ctas_cap = ctx->dp_pending ? 3 : 0;   // a channel decode is running on its stream: share the SMs with it
-    if ((rc = ofdm_run(O, first, n, st->n_samples, bs, ctx->stream))) return rc;
     if (st->frames_host || st->produced_host) {
         if ((rc = sl.d_stage.alloc(size_t(n) * fb))) return rc;
         if ((rc = sl.d_produced.alloc(size_t(n)))) return rc;
-        if ((rc = ofdm_gather_latest(O, first, n, sl.d_stage.as<int8_t>(), sl.d_produced.as<uint8_t>(), ctx->stream))) return rc;
+        rc = d_written0 ? ofdm_gather_since(O, first, n, d_written0, sl.d_stage.as<int8_t>(), sl.d_produced.as<uint8_t>(), ctx->stream)
+                        : ofdm_gather_latest(O, first, n, sl.d_stage.as<int8_t>(), sl.d_produced.as<uint8_t>(), ctx->stream);
+        if (rc) return rc;
     }
     if (st->run_chan_decode && (rc = dabgpu_chan_decode(ctx, first, n))) return rc;
     CUDA_TRY(join_dabplus(ctx));
     CUDA_TRY(cudaEventRecord(sl.compute_done, ctx->stream));
-    // (3) copy out.  The next compute may overwrite the channel-decode arenas: it is made to wait for this copy.
+    // Copy out.  The next compute may overwrite the channel-decode arenas: it is made to wait for this copy.
     CUDA_TRY(cudaStreamWaitEvent(ctx->s_d2h, sl.compute_done, 0));
     const int nb_cifs = ctx->P.nb_cifs;
     if (st->frames_host) CUDA_TRY(cudaMemcpyAsync(st->frames_host, sl.d_stage.p, size_t(n) * fb, cudaMemcpyDeviceToHost, ctx->s_d2h));
@@ -1381,10 +1376,44 @@ int dabgpu_submit(dabgpu_ctx* ctx, const dabgpu_step* st, uint64_t* ticket) {
     CUDA_TRY(cudaEventRecord(sl.d2h_done, ctx->s_d2h));
     if (arenas) CUDA_TRY(cudaStreamWaitEvent(ctx->stream, sl.d2h_done, 0));
     sl.busy = true;
-    sl.ticket = t;
+    sl.ticket = ctx->next_ticket;
+    *ticket = ctx->next_ticket++;
+    return DABGPU_OK;
+}
+
+extern "C" {
+
+int dabgpu_submit(dabgpu_ctx* ctx, const dabgpu_step* st, uint64_t* ticket) {
+    if (!ctx || !st || !ticket) return set_error(DABGPU_ERR_INVALID, "null argument");
+    int rc = check_stream_range(ctx, st->first_stream, st->n_streams);
+    if (rc) return rc;
+    if (!st->iq_host || st->n_samples <= 0 || st->n_streams == 0) return set_error(DABGPU_ERR_INVALID, "bad IQ buffer");
+    OfdmState& O = ctx->ofdm;
+    if (O.external_ring) return set_error(DABGPU_ERR_STATE, "a device input buffer is attached: use dabgpu_ofdm_advance");
+    CUDA_TRY(cudaSetDevice(ctx->cfg.device));
+    CUDA_TRY(join_if_many_frames(ctx, st->n_samples));
+    const uint64_t t = ctx->next_ticket;
+    auto& prev = ctx->pipe[(t + DABGPU_PIPELINE_DEPTH - 1) % DABGPU_PIPELINE_DEPTH];
+    // the copy of this step overlaps the compute of the previous one: together they must fit the ring headroom
+    const size_t prev_samples = ctx->pipe_recent_samples[(t + DABGPU_PIPELINE_DEPTH - 1) % DABGPU_PIPELINE_DEPTH];
+    if (size_t(st->n_samples) + prev_samples > ofdm_ring_headroom(O))
+        return set_error(DABGPU_ERR_INVALID, "n_samples %d (+%zu in flight) exceeds the IQ ring headroom %zu: raise ring_samples", st->n_samples,
+                         prev_samples, ofdm_ring_headroom(O));
+    dabgpu_ctx::PipeSlot* sl;
+    if ((rc = pipe_acquire(ctx, &sl))) return rc;
+    const int n = st->n_streams, first = st->first_stream;
+    // (1) copy in; the ring region being overwritten was last read by the compute two tickets ago, which pipe_acquire covers
+    if (prev.busy) CUDA_TRY(cudaStreamWaitEvent(ctx->s_h2d, prev.h2d_done, 0));
+    if ((rc = ofdm_upload(O, st->iq_host, st->iq_stride_bytes, first, n, 0, size_t(st->n_samples), ctx->s_h2d))) return rc;
+    CUDA_TRY(cudaEventRecord(sl->h2d_done, ctx->s_h2d));
+    // (2) compute
+    CUDA_TRY(cudaStreamWaitEvent(ctx->stream, sl->h2d_done, 0));
+    const int bs = st->block_size > 0 ? st->block_size : st->n_samples;
+    ctx->ofdm.demod_ctas_cap = ctx->dp_pending ? 3 : 0;   // a channel decode is running on its stream: share the SMs with it
+    if ((rc = ofdm_run(O, first, n, st->n_samples, bs, ctx->stream))) return rc;
+    // (3) channel decode and copy out
+    if ((rc = pipe_finish(ctx, *sl, st, nullptr, ticket))) return rc;
     ctx->pipe_recent_samples[t % DABGPU_PIPELINE_DEPTH] = size_t(st->n_samples);
-    ctx->next_ticket = t + 1;
-    *ticket = t;
     return DABGPU_OK;
 }
 
@@ -1427,7 +1456,20 @@ struct dabgpu_wideband {
     unsigned long long max_pass_blocks = 0;
     float2* d_out = nullptr;
     unsigned long long n_in = 0, blocks_done = 0, out_consumed = 0;   // input samples per source, blocks filtered, outputs handed to OFDM
+    size_t max_submit = 0;            // samples per source a ticket may carry (dabgpu_wideband_reserve); 0: none
 };
+
+// Input ring size (log2) for tickets of up to max_submit samples per source.  The ring keeps the history of the next block
+// (fft_in - step_in samples), the input held back until that block is complete (< step_in) and either one pass of
+// max_pass_blocks blocks, or two tickets: the upload of ticket t + 1 then writes none of the samples the filter passes of
+// ticket t still read.
+static int wb_ring_log2(const dabgpu_wideband* w, size_t max_submit) {
+    const size_t ov_in = size_t(w->geo.fft_in - w->geo.step_in), step_in = size_t(w->geo.step_in);
+    const size_t need = std::max<size_t>(ov_in + (w->max_pass_blocks + 1) * step_in, ov_in + step_in - 1 + 2 * max_submit);
+    int log2 = 0;
+    while ((size_t(1) << log2) < need) log2++;
+    return log2;
+}
 
 static void wb_detach(dabgpu_wideband* w) {
     DevBuf* bufs[] = {&w->d_ring, &w->d_H, &w->d_twf, &w->d_twi, &w->d_dposf, &w->d_dposi, &w->d_chans, &w->d_first};
@@ -1613,9 +1655,7 @@ static int wb_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, const dab
     w->headroom = ofdm_ring_headroom(ctx->P, capacity);
     w->max_pass_blocks = std::min<unsigned long long>(512, w->headroom / size_t(geo.step_out));
     w->d_out = static_cast<float2*>(d_out);
-    // the history of the first block of a pass, the pass, and the input held back until the next block is complete
-    const size_t ov_in = size_t(geo.fft_in - geo.step_in);
-    while ((size_t(1) << w->ring_log2) < ov_in + (w->max_pass_blocks + 1) * size_t(geo.step_in)) w->ring_log2++;
+    w->ring_log2 = wb_ring_log2(w, 0);
     w->ring_cap = size_t(1) << w->ring_log2;
 
     // channels grouped by source, in channel order
@@ -1684,6 +1724,70 @@ static int wb_open(dabgpu_ctx* ctx, const dabgpu_wideband_config* cfg, const dab
     return DABGPU_OK;
 }
 
+// Validation and set-up shared by dabgpu_wideband_process and _submit for a call of n_samples per source: the Process() block
+// size (*bs) and the output samples per channel the call yields (*new_out).
+static int wb_begin(dabgpu_wideband* w, size_t n_samples, int block_size, size_t* bs, size_t* new_out) {
+    dabgpu_ctx* ctx = w->ctx;
+    const size_t blk_out = size_t(w->geo.step_out);
+    *new_out = size_t((w->n_in + n_samples) / (unsigned long long)w->geo.step_in - w->blocks_done) * blk_out;
+    *bs = block_size > 0 ? size_t(block_size) : std::max<size_t>(*new_out, 1);
+    if (*bs + blk_out > w->headroom)
+        return set_error(DABGPU_ERR_INVALID, "block_size %zu does not fit the output ring (%zu samples of headroom)", *bs, w->headroom);
+    CUDA_TRY(cudaSetDevice(ctx->cfg.device));
+    CUDA_TRY(join_if_many_frames(ctx, long(std::min<size_t>(*new_out, 1ul << 40))));
+    ctx->ofdm.demod_ctas_cap = ctx->dp_pending ? 3 : 0;   // a channel decode is running on its stream: share the SMs with it
+    return DABGPU_OK;
+}
+
+// Queues the copy of n samples of every source (source s at src + s * stride) into the ring at n_in on cs.
+static int wb_upload(dabgpu_wideband* w, const uint8_t* src, size_t stride, size_t n, cudaStream_t cs) {
+    for (size_t left = n, off = 0; left > 0;) {
+        const size_t pos = size_t(w->n_in & (w->ring_cap - 1)), run = std::min(left, w->ring_cap - pos);
+        const size_t bytes = run * size_t(w->bps);
+        CUDA_TRY(cudaMemcpy2DAsync(w->d_ring.as<uint8_t>() + pos * size_t(w->bps), w->ring_cap * size_t(w->bps), src + off * size_t(w->bps),
+                                   w->n_sources > 1 ? stride : bytes, bytes, size_t(w->n_sources), cudaMemcpyHostToDevice, cs));
+        w->n_in += run; off += run; left -= run;
+    }
+    return DABGPU_OK;
+}
+
+// One pass on the compute stream over the input in the ring: the filter bank over its whole blocks, at most max_pass_blocks
+// and never more than the OFDM stage's headroom ahead of what that consumed, then OFDM_Demod::Process over the new outputs in
+// blocks of bs.  A partial block only at the end of the call: once input_done and every complete block is filtered (*last).
+static int wb_pass(dabgpu_wideband* w, size_t bs, bool input_done, bool* last) {
+    dabgpu_ctx* ctx = w->ctx;
+    const unsigned long long blk_in = (unsigned long long)w->geo.step_in;
+    const size_t blk_out = size_t(w->geo.step_out);
+    WbDev W;
+    W.ring = w->d_ring.as<uint8_t>(); W.ring_log2 = w->ring_log2; W.ring_mask = w->ring_cap - 1;
+    W.out = w->d_out; W.out_cap = w->out_cap;
+    W.H = w->d_H.as<float2>(); W.tw_fwd = w->d_twf.as<float2>(); W.tw_inv = w->d_twi.as<float2>();
+    W.dpos_fwd = w->d_dposf.as<uint16_t>(); W.dpos_inv = w->d_dposi.as<uint16_t>();
+    W.chans = w->d_chans.as<WbChan>(); W.chan_first = w->d_first.as<int>(); W.fs = w->fs;
+    WbMixDev M;
+    M.w = W; M.n_fft = w->geo.fft_in; M.step_in = w->geo.step_in; M.ov_in = w->geo.fft_in - w->geo.step_in; M.step_out = w->geo.step_out;
+    M.n_pass = int(w->radices.size());
+    for (int p = 0; p < WB_MIX_MAX_PASSES; p++) M.radix[p] = p < M.n_pass ? w->radices[size_t(p)] : 1;
+    const size_t pending = size_t(w->blocks_done * blk_out - w->out_consumed);
+    const unsigned long long nb = std::min({w->n_in / blk_in - w->blocks_done, w->max_pass_blocks, (unsigned long long)((w->headroom - pending) / blk_out)});
+    if (nb) {
+        int rc = w->mixed ? wb_mix_kernel(w->geo.fft_out, w->fmt)(&M, w->blocks_done, unsigned(nb), w->n_sources, ctx->stream)
+                          : wb_kernel(w->D, w->fmt)(&W, w->blocks_done, unsigned(nb), w->n_sources, ctx->stream);
+        if (rc) return rc;
+        ctx->launches++;
+        w->blocks_done += nb;
+    }
+    const size_t avail = size_t(w->blocks_done * blk_out - w->out_consumed);
+    *last = input_done && w->n_in / blk_in == w->blocks_done;
+    const size_t present = *last ? avail : (avail / bs) * bs;
+    if (present) {
+        int rc = ofdm_run(ctx->ofdm, 0, w->n_channels, int(present), int(bs), ctx->stream);
+        if (rc) return rc;
+        w->out_consumed += present;
+    }
+    return DABGPU_OK;
+}
+
 extern "C" {
 
 int dabgpu_wideband_process(dabgpu_wideband* w, const void* iq_host, size_t stride, size_t n_samples, int block_size, size_t* n_out) {
@@ -1693,63 +1797,83 @@ int dabgpu_wideband_process(dabgpu_wideband* w, const void* iq_host, size_t stri
     if (!ctx) return set_error(DABGPU_ERR_STATE, "the context of this wideband front end was destroyed");
     if (!iq_host && n_samples) return set_error(DABGPU_ERR_INVALID, "null input");
     if (w->n_sources > 1 && stride < n_samples * size_t(w->bps)) return set_error(DABGPU_ERR_INVALID, "source stride %zu is shorter than a source", stride);
-    const unsigned long long blk_in = (unsigned long long)w->geo.step_in, hist = (unsigned long long)(w->geo.fft_in - w->geo.step_in);
-    const size_t blk_out = size_t(w->geo.step_out);
-    const size_t new_out = size_t((w->n_in + n_samples) / blk_in - w->blocks_done) * blk_out;
-    const size_t bs = block_size > 0 ? size_t(block_size) : std::max<size_t>(new_out, 1);
-    if (bs + blk_out > w->headroom)
-        return set_error(DABGPU_ERR_INVALID, "block_size %zu does not fit the output ring (%zu samples of headroom)", bs, w->headroom);
-    CUDA_TRY(cudaSetDevice(ctx->cfg.device));
-    CUDA_TRY(join_if_many_frames(ctx, long(std::min<size_t>(new_out, 1ul << 40))));
-    ctx->ofdm.demod_ctas_cap = ctx->dp_pending ? 3 : 0;   // a channel decode is running on its stream: share the SMs with it
-    WbDev W;
-    W.ring = w->d_ring.as<uint8_t>(); W.ring_log2 = w->ring_log2; W.ring_mask = w->ring_cap - 1;
-    W.out = w->d_out; W.out_cap = w->out_cap;
-    W.H = w->d_H.as<float2>(); W.tw_fwd = w->d_twf.as<float2>(); W.tw_inv = w->d_twi.as<float2>();
-    W.dpos_fwd = w->d_dposf.as<uint16_t>(); W.dpos_inv = w->d_dposi.as<uint16_t>();
-    W.chans = w->d_chans.as<WbChan>(); W.chan_first = w->d_first.as<int>(); W.fs = w->fs;
-    WbMixDev M;
-    M.w = W; M.n_fft = w->geo.fft_in; M.step_in = w->geo.step_in; M.ov_in = int(hist); M.step_out = w->geo.step_out;
-    M.n_pass = int(w->radices.size());
-    for (int p = 0; p < WB_MIX_MAX_PASSES; p++) M.radix[p] = p < M.n_pass ? w->radices[size_t(p)] : 1;
+    size_t bs, new_out;
+    int rc = wb_begin(w, n_samples, block_size, &bs, &new_out);
+    if (rc) return rc;
     const uint8_t* src = static_cast<const uint8_t*>(iq_host);
+    const unsigned long long hist = (unsigned long long)(w->geo.fft_in - w->geo.step_in);
     size_t done = 0;
-    for (;;) {
+    for (bool last = false; !last;) {
         // input: the ring keeps everything from the first sample the next block reads (its fft_in - step_in samples of history)
-        const unsigned long long keep = w->blocks_done * blk_in >= hist ? w->blocks_done * blk_in - hist : 0;
+        const unsigned long long keep = w->blocks_done * (unsigned long long)w->geo.step_in >= hist ? w->blocks_done * w->geo.step_in - hist : 0;
         const size_t take = std::min<size_t>(n_samples - done, size_t(keep + w->ring_cap - w->n_in));
-        for (size_t left = take, off = done; left > 0;) {
-            const size_t pos = size_t(w->n_in & (w->ring_cap - 1)), run = std::min(left, w->ring_cap - pos);
-            const size_t bytes = run * size_t(w->bps);
-            CUDA_TRY(cudaMemcpy2DAsync(w->d_ring.as<uint8_t>() + pos * size_t(w->bps), w->ring_cap * size_t(w->bps), src + off * size_t(w->bps),
-                                       w->n_sources > 1 ? stride : bytes, bytes, size_t(w->n_sources), cudaMemcpyHostToDevice, ctx->stream));
-            w->n_in += run; off += run; left -= run;
-        }
+        if ((rc = wb_upload(w, src + done * size_t(w->bps), stride, take, ctx->stream))) return rc;
         done += take;
-        // filter: whole blocks, never more than the OFDM stage's headroom ahead of what it consumed
-        const size_t pending = size_t(w->blocks_done * blk_out - w->out_consumed);
-        const unsigned long long nb = std::min({w->n_in / blk_in - w->blocks_done, w->max_pass_blocks, (unsigned long long)((w->headroom - pending) / blk_out)});
-        if (nb) {
-            int rc = w->mixed ? wb_mix_kernel(w->geo.fft_out, w->fmt)(&M, w->blocks_done, unsigned(nb), w->n_sources, ctx->stream)
-                              : wb_kernel(w->D, w->fmt)(&W, w->blocks_done, unsigned(nb), w->n_sources, ctx->stream);
-            if (rc) return rc;
-            ctx->launches++;
-            w->blocks_done += nb;
-        }
-        // OFDM_Demod::Process over the new outputs in blocks of bs; a partial block only at the end of the call
-        const size_t avail = size_t(w->blocks_done * blk_out - w->out_consumed);
-        const bool last = done == n_samples && w->n_in / blk_in == w->blocks_done;
-        const size_t present = last ? avail : (avail / bs) * bs;
-        if (present) {
-            int rc = ofdm_run(ctx->ofdm, 0, w->n_channels, int(present), int(bs), ctx->stream);
-            if (rc) return rc;
-            w->out_consumed += present;
-        }
-        if (last) break;
+        if ((rc = wb_pass(w, bs, done == n_samples, &last))) return rc;
     }
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (n_out) *n_out = new_out;
     return DABGPU_OK;
+}
+
+int dabgpu_wideband_reserve(dabgpu_wideband* w, size_t max_submit_samples) {
+    if (!w) return set_error(DABGPU_ERR_INVALID, "null wideband front end");
+    if (!w->ctx) return set_error(DABGPU_ERR_STATE, "the context of this wideband front end was destroyed");
+    if (w->n_in > 0) return set_error(DABGPU_ERR_STATE, "dabgpu_wideband_reserve must come before the first input");
+    if (max_submit_samples < 1 || max_submit_samples > size_t(INT_MAX))
+        return set_error(DABGPU_ERR_INVALID, "max_submit_samples %zu out of range [1, %d]", max_submit_samples, INT_MAX);
+    CUDA_TRY(cudaSetDevice(w->ctx->cfg.device));
+    const int log2 = wb_ring_log2(w, max_submit_samples);
+    if (log2 != w->ring_log2) {
+        // the ring holds no input yet: nothing to keep
+        const size_t row = size_t(w->n_sources) * size_t(w->bps);
+        w->d_ring.release();
+        if (int rc = w->d_ring.alloc(row << log2)) {
+            w->d_ring.alloc(row << w->ring_log2);   // leave the front end as it was
+            return rc;
+        }
+        w->ring_log2 = log2;
+        w->ring_cap = size_t(1) << log2;
+    }
+    w->max_submit = max_submit_samples;
+    return DABGPU_OK;
+}
+
+// Pipelined dabgpu_wideband_process + dabgpu_chan_decode: (1) the upload on the copy stream, (2) the filter bank and OFDM
+// passes, the newest frames and the channel decode on the compute stream, (3) the copy-out, as in dabgpu_submit (pipe_finish).
+int dabgpu_wideband_submit(dabgpu_wideband* w, const dabgpu_step* st, uint64_t* ticket) {
+    if (!w || !st || !ticket) return set_error(DABGPU_ERR_INVALID, "null argument");
+    dabgpu_ctx* ctx = w->ctx;
+    if (!ctx) return set_error(DABGPU_ERR_STATE, "the context of this wideband front end was destroyed");
+    const int first = st->first_stream, n = st->n_streams;
+    if (first < 0 || n < 1 || first > w->n_channels - n)
+        return set_error(DABGPU_ERR_INVALID, "channel range [%d,%d) is empty or outside [0,%d)", first, first + n, w->n_channels);
+    if (!st->iq_host || st->n_samples <= 0) return set_error(DABGPU_ERR_INVALID, "bad input buffer");
+    const size_t n_samples = size_t(st->n_samples);
+    if (n_samples > w->max_submit)
+        return set_error(DABGPU_ERR_INVALID, "n_samples %zu exceeds the %zu samples per ticket set with dabgpu_wideband_reserve", n_samples, w->max_submit);
+    if (w->n_sources > 1 && st->iq_stride_bytes < n_samples * size_t(w->bps))
+        return set_error(DABGPU_ERR_INVALID, "source stride %zu is shorter than a source", st->iq_stride_bytes);
+    size_t bs, new_out;
+    int rc = wb_begin(w, n_samples, st->block_size, &bs, &new_out);
+    if (rc) return rc;
+    dabgpu_ctx::PipeSlot* sl;
+    if ((rc = pipe_acquire(ctx, &sl))) return rc;
+    const bool gather = st->frames_host || st->produced_host;
+    if (gather && (rc = sl->d_written0.alloc(size_t(n) * 4))) return rc;
+    // (1) copy in.  Ticket t - 1 may still be filtering: the reserve keeps this ticket's samples clear of what it reads.  The
+    // ticket before that used this slot; its compute must have read its samples before they are overwritten.
+    CUDA_TRY(cudaStreamWaitEvent(ctx->s_h2d, sl->compute_done, 0));
+    if ((rc = wb_upload(w, static_cast<const uint8_t*>(st->iq_host), st->iq_stride_bytes, n_samples, ctx->s_h2d))) return rc;
+    CUDA_TRY(cudaEventRecord(sl->h2d_done, ctx->s_h2d));
+    // (2) compute
+    CUDA_TRY(cudaStreamWaitEvent(ctx->stream, sl->h2d_done, 0));
+    if (gather)
+        CUDA_TRY(cudaMemcpyAsync(sl->d_written0.p, ctx->d_frames_written.as<uint32_t>() + first, size_t(n) * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+    for (bool last = false; !last;)
+        if ((rc = wb_pass(w, bs, true, &last))) return rc;
+    // (3) channel decode and copy out
+    return pipe_finish(ctx, *sl, st, sl->d_written0.as<uint32_t>(), ticket);
 }
 
 int dabgpu_wideband_close(dabgpu_wideband* w) {
@@ -1757,6 +1881,7 @@ int dabgpu_wideband_close(dabgpu_wideband* w) {
     if (w->ctx) {
         cudaSetDevice(w->ctx->cfg.device);
         sync_ctx(w->ctx);
+        if (w->ctx->s_d2h) cudaStreamSynchronize(w->ctx->s_d2h);   // the copy-out of tickets still in flight
     }
     wb_detach(w);
     delete w;

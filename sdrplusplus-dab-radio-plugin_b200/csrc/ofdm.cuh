@@ -678,6 +678,22 @@ __global__ void k_ofdm_gather_latest(const OfdmDev D, const int first_stream, in
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += gridDim.x * blockDim.x) frame_convert_group(src, dst, i, D.fg, false);
 }
 
+// The same over a step that spans several runs (produced_last only covers the last one): stream first_stream + y has produced
+// when its frame counter moved past written0[y], the counter as it stood before the step's first run.
+__global__ void k_ofdm_gather_since(const OfdmDev D, const int first_stream, const uint32_t* __restrict__ written0, int8_t* __restrict__ stage,
+                                    uint8_t* __restrict__ produced) {
+    const int s = first_stream + blockIdx.y;
+    const uint32_t written = D.frames_written[s];
+    const bool has = written != written0[blockIdx.y];
+    if (blockIdx.x == 0 && threadIdx.x == 0) produced[blockIdx.y] = has ? 1 : 0;
+    if (!has) return;
+    const uint32_t slot = (written - 1u) & D.slot_mask;
+    const int8_t* src = D.frames + (size_t(s) * (D.slot_mask + 1u) + slot) * D.g.frame_bits;
+    int8_t* dst = stage + size_t(blockIdx.y) * D.g.frame_bits;
+    const uint32_t n16 = uint32_t(D.g.frame_bits) / 16u;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += gridDim.x * blockDim.x) frame_convert_group(src, dst, i, D.fg, false);
+}
+
 // OFDM_Demod::GetFrameFFT (ofdm_demodulator.h:135, filled by PipelineThread, ofdm_demodulator.cpp:673-700): the spectra of the
 // PRS and the data symbols of the last emitted frame, natural bin order, recomputed on demand from the IQ that is still in the
 // ring (the demodulation kernel keeps its spectra in registers).  One CTA per symbol; same PLL and FFT as the control kernel.

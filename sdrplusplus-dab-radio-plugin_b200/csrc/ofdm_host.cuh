@@ -515,6 +515,15 @@ static int ofdm_gather_latest(OfdmState& O, int first, int n, int8_t* d_stage, u
     return DABGPU_OK;
 }
 
+// the same for the streams whose frame counter moved past d_written0 (a device copy of frames_written[first, first + n))
+static int ofdm_gather_since(OfdmState& O, int first, int n, const uint32_t* d_written0, int8_t* d_stage, uint8_t* d_produced, cudaStream_t cs) {
+    const dim3 grid(32, n);
+    k_ofdm_gather_since<<<grid, 256, 0, cs>>>(O.dev, first, d_written0, d_stage, d_produced);
+    O.launches++;
+    CUDA_TRY(cudaGetLastError());
+    return DABGPU_OK;
+}
+
 static int ofdm_fetch_latest(OfdmState& O, int first, int n, int8_t* frames_host, uint8_t* produced, cudaStream_t cs) {
     int rc;
     const size_t fb = size_t(O.P.nb_frame_bits);
