@@ -1,7 +1,8 @@
 """Wideband front end at any tuner rate (dabgpu_wideband_plan, dabgpu_wideband_open_any_rate), CPU side: the library's plan
 agrees with a restatement of the rule in include/dabgpu.h at every multiple of 1 kHz, the channel filter meets its mask at every
-supported rate, and a numpy model of the mixed-radix filter bank the kernel implements (k_wideband_mixed, wideband.cuh) agrees
-with a float64 long-FFT evaluation of the header's output contract."""
+supported rate, a numpy model of the mixed-radix filter bank the kernel implements (k_wideband_mixed, wideband.cuh) agrees
+with a float64 long-FFT evaluation of the header's output contract at every supported rate, and the windowed form of that
+evaluation the long-run GPU tests use agrees with the evaluation over the whole input."""
 from math import ceil, gcd, log2
 
 import numpy as np
@@ -42,7 +43,6 @@ def plan(fs):
 
 GRID = [f for f in range(FS_OUT, 16 * FS_OUT + 1, 1000)]
 SUPPORTED = [f for f in GRID if plan(f)]
-MODEL_RATES = [2400000, 2500000, 3000000, 6000000, 10000000, 12500000, 20000000, 2250000, 8000000]
 
 
 def taps(fs):
@@ -55,14 +55,18 @@ def split_offset(f, d):
     return b, f - d * b
 
 
-def reference(x, fs, f):
+def reference(x, fs, f, a0=0):
     """the header's contract in float64 over one long FFT: mix by f^, filter with the DFT of h, keep |f| < 1.024 MHz, evaluate
-    at input times n fs / 2.048 MHz, rotate by delta.  x holds input beyond the outputs asked for, so the tail is realistic."""
+    at input times n fs / 2.048 MHz, rotate by delta.  x holds input beyond the outputs asked for, so the tail is realistic.
+    x may instead be a window of the input from absolute sample a0, a multiple of q = fs / gcd(fs, 2.048 MHz): the mixing
+    phase then takes absolute input indices and the rotation absolute output indices, so output i is output
+    a0 2.048 MHz / fs + i of the whole input wherever the window has MARGIN samples of input on either side of it."""
     p = plan(fs)
     b, delta = split_offset(f, p["bin_hz"])
-    m = np.arange(x.size, dtype=np.int64)
-    z = x * np.exp(-2j * np.pi * ((b * m) % p["fft_in"]) / p["fft_in"])
     q = fs // gcd(fs, FS_OUT)                        # P a multiple of q: P * 2.048 MHz / fs is an integer
+    assert a0 % q == 0
+    m = a0 + np.arange(x.size, dtype=np.int64)
+    z = x * np.exp(-2j * np.pi * ((b * m) % p["fft_in"]) / p["fft_in"])
     P = -(-(x.size + p["taps"]) // q) * q
     Q = P * FS_OUT // fs
     V = np.fft.fft(z, P) * np.fft.fft(taps(fs), P)
@@ -71,8 +75,24 @@ def reference(x, fs, f):
     Y = np.zeros(Q, dtype=np.complex128)
     Y[k[keep] % Q] = V[keep]
     y = np.fft.ifft(Y) * (Q / P)
-    n = np.arange(Q, dtype=np.int64)
+    n = a0 * FS_OUT // fs + np.arange(Q, dtype=np.int64)
     return y * np.exp(-2j * np.pi * ((n % FS_OUT) * delta % FS_OUT) / FS_OUT)
+
+
+MARGIN = 20000   # input samples of the reference before and after the outputs it is asked for
+
+
+def reference_outputs(x_at, fs, f, n_lo, n_hi):
+    """outputs n_lo .. n_hi - 1 of the contract from a window of the input: x_at(a, b) returns absolute input samples
+    a .. b - 1.  The window starts MARGIN samples (rounded to a multiple of q, or at 0) before the input time of output n_lo
+    and ends MARGIN samples after that of output n_hi - 1."""
+    q = fs // gcd(fs, FS_OUT)
+    a_s = n_lo * fs // FS_OUT // q * q               # a_s 2.048 MHz / fs is an output index <= n_lo
+    a_e = -(-n_hi * fs // FS_OUT)
+    a0 = max(0, a_s - -(-MARGIN // q) * q)
+    y = reference(x_at(a0, a_e + MARGIN), fs, f, a0)
+    n0 = a0 * FS_OUT // fs
+    return y[n_lo - n0: n_hi - n0]
 
 
 def model(x, fs, f):
@@ -142,7 +162,7 @@ def test_filter_mask_every_supported_rate():
     assert worst_944 > -71.2
 
 
-@pytest.mark.parametrize("fs", MODEL_RATES)
+@pytest.mark.parametrize("fs", SUPPORTED)
 def test_mixed_radix_model_matches_long_fft_reference(fs):
     p = plan(fs)
     rng = np.random.default_rng(fs % 9973)
@@ -155,6 +175,29 @@ def test_mixed_radix_model_matches_long_fft_reference(fs):
         ref = reference(x, fs, f)[:got.size]
         err = np.abs(got - ref)
         assert np.sqrt(np.mean(err ** 2)) < 1e-5 and err.max() < 1e-4, (f, np.sqrt(np.mean(err ** 2)), err.max())
+
+
+@pytest.mark.parametrize("fs", [2400000, 8748000, 12500000])   # q = 75, 2 187, 3 125
+def test_windowed_reference_is_the_long_one(fs):
+    """reference_outputs, as the long-run GPU tests use it, equals one reference() over the whole input in the window's
+    interior.  The two differ where their bin grids meet the 1.024 MHz band edge: a bin of a record of P samples carries
+    |H(1.024 MHz)| rms / sqrt(P) of it, |H(1.024 MHz)| between -75 and -83 dB over the supported rates.  The difference
+    shrinks as the record grows; at the MARGIN of 20 000 samples on either side it is bounded by 1.8e-4 / sqrt(2 MARGIN) =
+    9e-7 (measured: <= 4.6e-7), so 1e-7 is out of reach there, but it is 500 times below the worst sample the GPU tests
+    allow."""
+    p = plan(fs)
+    rng = np.random.default_rng(fs % 8191)
+    n_lo = 3 * MARGIN * FS_OUT // fs + 12345        # the window starts past sample 0
+    n_hi = n_lo + 3 * p["step_out"] + 77
+    n_tot = -(-n_hi * fs // FS_OUT) + MARGIN + 999
+    x = (rng.standard_normal(n_tot) + 1j * rng.standard_normal(n_tot)) / np.sqrt(2)
+    lim = fs // 2 - 768000
+    for f in (-lim, (7 * p["bin_hz"]) // 2, 6001):
+        full = reference(x, fs, f)[n_lo:n_hi]
+        win = reference_outputs(lambda a, b: x[a:b], fs, f, n_lo, n_hi)
+        assert win.size == n_hi - n_lo
+        err = np.abs(win - full)
+        assert err.max() <= 1e-6, (f, err.max())
 
 
 def test_model_is_the_power_of_two_formula():

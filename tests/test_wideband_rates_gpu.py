@@ -1,17 +1,66 @@
 """Wideband front end at the tuners' own rates (dabgpu_wideband_open_any_rate, k_wideband_mixed) on the GPU: parity of d_out with
-the float64 long-FFT evaluation of the header's contract at 2.4 to 20 MS/s in every format, bit-identical output to
-dabgpu_wideband_open at 2.048 MHz x 2^d, bit-identical output however the input is split into calls, no phase drift over 2^27
-input samples, round trips of synthetic multi-ensemble captures through the whole chain, and argument validation."""
+the float64 long-FFT evaluation of the header's contract at every one of the 105 planned rates (2.4 to 20 MS/s in every format,
+each other rate in one, so that every format meets every kept-bin count of k_wideband_mixed and k_wideband<D>), with channels
+listed out of source order, a source without channels, a second round of channel groups per CTA, offsets on rounding ties and
+coinciding channels; bit-identical output to dabgpu_wideband_open at 2.048 MHz x 2^d, bit-identical output however the input is
+split into calls at every rate, no phase drift over 2^27 input samples, round trips of synthetic multi-ensemble captures
+through the whole chain, and argument validation."""
 import numpy as np
 import pytest
 
 from test_wideband_gpu import CAP, PERIOD, SCALE, WARM, _hash, _tx, dequantize
-from test_wideband_rates_cpu import FS_OUT, plan, reference, split_offset, taps
+from test_wideband_rates_cpu import FS_OUT, MARGIN, SUPPORTED, plan, reference, split_offset, taps
 
 pytestmark = pytest.mark.gpu
 
 RATES = [2400000, 2500000, 3000000, 6000000, 10000000, 12500000, 20000000]
 FORMATS = ["raw_u8", "raw_s8", "raw_s16l", "raw_f32l"]
+WB_MIX_THREADS = 256   # threads of a k_wideband_mixed CTA (wideband.cuh)
+
+
+def kernel_of(fs):
+    """the filter bank dabgpu_wideband_open_any_rate runs at fs: k_wideband<D> where fft_in = 512 D, else k_wideband_mixed
+    with its kept-bin count"""
+    n = plan(fs)["fft_in"]
+    return "k_wideband" if n & (n - 1) == 0 else plan(fs)["fft_out"]
+
+
+def groups_per_cta(fs):
+    """channels a CTA filters at once: D groups of 64 threads in k_wideband<D>, WB_MIX_THREADS / (fft_out / 8) in k_wideband_mixed"""
+    p = plan(fs)
+    return p["fft_in"] // 512 if kernel_of(fs) == "k_wideband" else WB_MIX_THREADS // (p["fft_out"] // 8)
+
+
+# the seven tuner rates in every format, every other planned rate in one, the formats taken in turn over the sorted rates
+OTHER_RATES = [fs for fs in SUPPORTED if fs not in RATES]
+PARITY = [(fmt, fs) for fmt in FORMATS for fs in RATES] + [(FORMATS[i % len(FORMATS)], fs) for i, fs in enumerate(OTHER_RATES)]
+assert len(SUPPORTED) == 105 and sorted({fs for _, fs in PARITY}) == SUPPORTED
+assert {(fmt, kernel_of(fs)) for fmt, fs in PARITY} == {(fmt, k) for fmt in FORMATS for k in (512, 1024, 2048, "k_wideband")}
+
+
+def layout(fs):
+    """(source, offset) per channel for n_sources = 3: source 0 holds groups_per_cta + 1 channels (a second round, partly
+    filled where a CTA runs more than one group), source 1 every offset below plus a duplicate, source 2 none; the channels of
+    sources 0 and 1 alternate, source 1 first.  Offsets: the edges +-lim, rounding ties +(3 + 1/2) and -(5 + 1/2) bins (the
+    largest residual rotation, of either sign), 0, a non-zero whole bin, just below a tie, 6001 Hz, and next to the edges with
+    a non-zero residual rotation: lim - bin/2 (a tie where lim is a whole bin) and -lim + bin + 777."""
+    d, lim = plan(fs)["bin_hz"], fs // 2 - 768000
+    offs = [-lim, lim, 7 * d // 2, -11 * d // 2, 0, 3 * d, d // 2 - 1 - 2 * d, 6001, lim - d // 2, -lim + d + 777]
+    on0 = [offs[i % len(offs)] for i in range(groups_per_cta(fs) + 1)]
+    on1 = offs + offs[2:3]
+    chans = []
+    for i in range(max(len(on0), len(on1))):
+        chans += [(1, on1[i])] if i < len(on1) else []
+        chans += [(0, on0[i])] if i < len(on0) else []
+    return chans
+
+
+def full_scale_noise(dtype, n_values, rng):
+    """raw values over the whole range of the format (+-1 for raw_f32l)"""
+    if np.dtype(dtype).kind == "f":
+        return rng.uniform(-1.0, 1.0, n_values).astype(dtype)
+    info = np.iinfo(dtype)
+    return rng.integers(info.min, info.max, n_values, endpoint=True).astype(dtype)
 
 
 def noise_and_tones(n, fs, rng):
@@ -22,11 +71,11 @@ def noise_and_tones(n, fs, rng):
     return x
 
 
-def open_any(dab, fs, fmt, sources, offsets, cap=CAP, any_rate=True):
+def open_any(dab, fs, fmt, sources, offsets, cap=CAP, any_rate=True, n_sources=None):
     import torch
     g = dab.DabGpu(mode=1, max_streams=len(sources), iq_format=dab.IQ_C32)
     out = torch.zeros((len(sources), cap), dtype=torch.complex64, device="cuda:0")
-    w = g.wideband_open(fs, fmt, sources, offsets, out.data_ptr(), cap, any_rate=any_rate)
+    w = g.wideband_open(fs, fmt, list(sources), list(offsets), out.data_ptr(), cap, n_sources=n_sources, any_rate=any_rate)
     return g, w, out
 
 
@@ -35,34 +84,36 @@ def n_out_after(fs, n_in):
     return p["step_out"] * (n_in // p["step_in"])
 
 
-@pytest.mark.parametrize("fs", RATES)
-@pytest.mark.parametrize("fmt", FORMATS)
-def test_parity_with_formula(gpu_ctx, fs, fmt):
-    import torch
+@pytest.mark.parametrize("fmt,fs", PARITY)
+def test_parity_with_formula(gpu_ctx, fmt, fs):
     p = plan(fs)
     rng = np.random.default_rng(fs % 7919 + FORMATS.index(fmt))
     n_in = p["step_in"] * 40 + 1234
-    n_tot = n_in + 20000                      # the reference's interpolation near the last output sees realistic input after it
+    n_tot = n_in + MARGIN                      # the reference's interpolation near the last output sees realistic input after it
     raws, xs = [], []
     for _ in range(2):
         raw = _tx().quantize(noise_and_tones(n_tot, fs, rng), fmt, 0.25 if fmt == "raw_f32l" else SCALE[fmt] / 5)
         raws.append(raw)
         xs.append(dequantize(raw, fmt))
-    lim = fs // 2 - 768000
-    d = p["bin_hz"]
-    sources = [0, 0, 0, 1, 1, 1]
-    offsets = [-lim, d // 2 - 1 - 2 * d, lim - d // 2, -lim + d + 777, 6001, lim]
-    g, w, out = open_any(gpu_ctx, fs, fmt, sources, offsets)
+    raws.append(full_scale_noise(raws[0].dtype, raws[0].size, rng))   # source 2 feeds no channel: it must change nothing
+    chans = layout(fs)
+    sources, offsets = zip(*chans)
+    g, w, out = open_any(gpu_ctx, fs, fmt, sources, offsets, n_sources=3)
     got_n = w.process(np.stack(raws), block_size=65536)
     assert got_n == n_out_after(fs, n_tot)
     n_out = n_out_after(fs, n_in)
-    torch.cuda.synchronize()
-    got = out[:, :n_out].cpu().numpy().astype(np.complex128)
-    for c, (s, f) in enumerate(zip(sources, offsets)):
+    got = out[:, :n_out].cpu().numpy()
+    first = {}
+    for c, (s, f) in enumerate(chans):
+        if (s, f) in first:                    # the same channel again: the same arithmetic in another group or round
+            assert np.array_equal(got[c].view(np.float32), got[first[s, f]].view(np.float32)), (c, first[s, f], f)
+            continue
+        first[s, f] = c
         ref = reference(xs[s], fs, f)[:n_out]
         rms_in = np.sqrt(np.mean(np.abs(xs[s]) ** 2))
-        err = np.abs(got[c] - ref) / rms_in
-        assert np.sqrt(np.mean(err ** 2)) <= 1e-4 and err.max() <= 5e-4, (c, f, np.sqrt(np.mean(err ** 2)), err.max())
+        err = np.abs(got[c].astype(np.complex128) - ref) / rms_in
+        assert np.sqrt(np.mean(err ** 2)) <= 1e-4 and err.max() <= 5e-4, (c, s, f, np.sqrt(np.mean(err ** 2)), err.max())
+    assert len(first) < len(chans)
     w.close()
     g.close()
 
@@ -86,20 +137,26 @@ def test_same_output_as_power_of_two_entry_point(gpu_ctx, D):
         o.close()
 
 
-@pytest.mark.parametrize("fs", [10000000, 2400000])
+@pytest.mark.parametrize("fs", SUPPORTED)
 def test_call_partition_invariance(gpu_ctx, fs):
+    """calls of 1 sample and of sizes that are no multiple of step_in put block and call boundaries in different places at
+    every step_in"""
     import torch
     fmt = "raw_s16l"
     rng = np.random.default_rng(fs % 101)
-    n_in = 600000
-    raw = np.stack([_tx().quantize(noise_and_tones(n_in, fs, rng), fmt, 3000.0) for _ in range(2)])
-    lim = fs // 2 - 768000
-    sources, offsets = [0, 1, 1], [-lim + 1234, 0, lim - 4321]
-    g1, w1, out1 = open_any(gpu_ctx, fs, fmt, sources, offsets)
+    si = plan(fs)["step_in"]
+    n_in = 30 * si + si // 2 + 3
+    raw = [_tx().quantize(noise_and_tones(n_in, fs, rng), fmt, 3000.0) for _ in range(2)]
+    raw = np.stack(raw + [full_scale_noise(raw[0].dtype, raw[0].size, rng)])
+    sources, offsets = zip(*layout(fs))
+    g1, w1, out1 = open_any(gpu_ctx, fs, fmt, sources, offsets, n_sources=3)
     assert w1.process(raw) == n_out_after(fs, n_in)
-    g2, w2, out2 = open_any(gpu_ctx, fs, fmt, sources, offsets)
+    g2, w2, out2 = open_any(gpu_ctx, fs, fmt, sources, offsets, n_sources=3)
+    sizes = [1, si - 1, si + 1, 2 * si + si // 3, 7 * si + 11]
+    sizes.append(n_in - sum(sizes))
+    assert all(n % si for n in sizes)
     done, total = 0, 0
-    for n in (1, 4095, 65536, 333333, n_in - 1 - 4095 - 65536 - 333333):
+    for n in sizes:
         got = w2.process(np.ascontiguousarray(raw[:, 2 * done: 2 * (done + n)]))
         assert got == n_out_after(fs, done + n) - n_out_after(fs, done)
         done += n
