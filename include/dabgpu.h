@@ -445,6 +445,34 @@ typedef struct { int32_t type, a, b, c, d, n_bytes; } dabgpu_event_header;  /* f
 DABGPU_API int dabgpu_chan_get_dabplus_events(dabgpu_ctx* ctx, int stream, int sub_index, uint8_t* log_host,
                                               size_t log_cap, size_t* log_bytes);
 
+/* DAB+ output of every sub-channel of streams [first, first+n) at once, packed on the GPU.
+ * index_host: [n][max_subchannels][2] int32 = {byte offset into log_host, byte length}.  The log of (stream, sub) is
+ * byte-identical to what dabgpu_chan_get_dabplus_events(stream, sub) returns after the same decode: dabgpu_event_header
+ * records + payload padded to 4.  Length 0 = no events, not a DAB+ sub-channel, or an unused index.  Where the logs sit inside
+ * log_host is not part of the contract: read it through the index.
+ *
+ * dabgpu_dabplus_out_bound: the log_cap one decode of those streams can never exceed.  It follows from the sub-channel tables
+ * (active DAB+ entries and their bytes per CIF): a decode runs one frame of at most 4 CIFs per stream and a superframe takes 5,
+ * so each (stream, sub) fires at most 7 events and 5 x bytes-per-CIF of AU payload.  It changes with dabgpu_msc_configure /
+ * _add_subchannel / _remove_subchannel.  A log_cap below it gives DABGPU_ERR_OVERFLOW; NULL log_host or index_host gives
+ * DABGPU_ERR_INVALID.  Both are refused before anything is queued and leave the context as it was.
+ *
+ * dabgpu_chan_get_dabplus_all: the output of the last dabgpu_chan_decode that covered each stream; synchronises the context.
+ * dabgpu_submit_ex / dabgpu_wideband_submit_ex: dabgpu_submit / dabgpu_wideband_submit that also copy the DAB+ output of the
+ * ticket's channel decode into *dabplus (which needs run_chan_decode != 0, else DABGPU_ERR_INVALID).  The buffers must stay
+ * valid until the ticket was waited for and be pinned for the copy to overlap.  dabplus = NULL is exactly dabgpu_submit /
+ * dabgpu_wideband_submit.  The struct is read during the call only. */
+typedef struct {
+    uint8_t* log_host;
+    size_t log_cap;
+    int32_t* index_host;
+} dabgpu_dabplus_out;
+DABGPU_API int dabgpu_dabplus_out_bound(dabgpu_ctx* ctx, int first_stream, int n_streams, size_t* log_bytes);
+DABGPU_API int dabgpu_chan_get_dabplus_all(dabgpu_ctx* ctx, int first_stream, int n_streams, const dabgpu_dabplus_out* out);
+DABGPU_API int dabgpu_submit_ex(dabgpu_ctx* ctx, const dabgpu_step* step, const dabgpu_dabplus_out* dabplus, uint64_t* ticket);
+DABGPU_API int dabgpu_wideband_submit_ex(dabgpu_wideband* w, const dabgpu_step* step, const dabgpu_dabplus_out* dabplus,
+                                         uint64_t* ticket);
+
 /* Stand-alone AAC_Frame_Processor (dab/audio/aac_frame_processor.h:37-82): one object per DAB+ sub-channel that is
  * fed decoded logical frames from the host.  process() consumes one logical frame (MSC_Decoder::DecodeCIF output) and
  * returns the observer events it fired, in order, in the same flat log format as dabgpu_chan_get_dabplus_events. */

@@ -91,6 +91,11 @@ class Step(C.Structure):
                 ("fic_crc_host", C.c_void_p), ("chan_status_host", C.c_void_p)]
 
 
+class DabPlusOut(C.Structure):
+    """dabgpu_dabplus_out (include/dabgpu.h): host buffers of one DAB+ output, log + [n][max_subchannels][2] int32 index."""
+    _fields_ = [("log_host", C.c_void_p), ("log_cap", C.c_size_t), ("index_host", C.c_void_p)]
+
+
 class WidebandConfig(C.Structure):
     _fields_ = [("sample_rate", C.c_int), ("format", C.c_int), ("n_sources", C.c_int), ("n_channels", C.c_int),
                 ("source", C.POINTER(C.c_int)), ("offset_hz", C.POINTER(C.c_int))]
@@ -118,6 +123,7 @@ EXPORTS = [
     "dabgpu_autocfg_apply", "dabgpu_ofdm_get_response", "dabgpu_ofdm_get_frame_fft", "dabgpu_iq_convert", "dabgpu_softbits_to_bytes", "dabgpu_bytes_to_softbits",
     "dabgpu_packet_fec_decode", "dabgpu_wideband_open", "dabgpu_wideband_process", "dabgpu_wideband_close",
     "dabgpu_wideband_plan", "dabgpu_wideband_open_any_rate", "dabgpu_wideband_reserve", "dabgpu_wideband_submit",
+    "dabgpu_dabplus_out_bound", "dabgpu_chan_get_dabplus_all", "dabgpu_submit_ex", "dabgpu_wideband_submit_ex",
 ]
 
 _lib = None
@@ -201,6 +207,10 @@ def load_library() -> C.CDLL:
     L.dabgpu_wideband_open_any_rate.argtypes = L.dabgpu_wideband_open.argtypes
     L.dabgpu_wideband_reserve.argtypes = [C.c_void_p, C.c_size_t]
     L.dabgpu_wideband_submit.argtypes = [C.c_void_p, C.POINTER(Step), C.POINTER(C.c_uint64)]
+    L.dabgpu_dabplus_out_bound.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_size_t)]
+    L.dabgpu_chan_get_dabplus_all.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(DabPlusOut)]
+    L.dabgpu_submit_ex.argtypes = [C.c_void_p, C.POINTER(Step), C.POINTER(DabPlusOut), C.POINTER(C.c_uint64)]
+    L.dabgpu_wideband_submit_ex.argtypes = [C.c_void_p, C.POINTER(Step), C.POINTER(DabPlusOut), C.POINTER(C.c_uint64)]
     _lib = L
     return L
 
@@ -251,6 +261,26 @@ def _ptr(a: np.ndarray) -> C.c_void_p:
     return C.c_void_p(a.ctypes.data)
 
 
+def _dabplus_out(dabplus) -> Optional[DabPlusOut]:
+    """(log_ptr, log_cap, index_ptr) raw addresses -> dabgpu_dabplus_out, None -> NULL"""
+    if dabplus is None:
+        return None
+    log_ptr, log_cap, index_ptr = dabplus
+    return DabPlusOut(log_ptr, log_cap, index_ptr)
+
+
+def split_dabplus(log, index, first_stream: int = 0, max_subchannels: int = 64) -> dict:
+    """One DAB+ output (log bytes, index [n][max_subchannels][2] int32, or the same bytes flat) -> {(stream, sub): event log
+    bytes} for every entry with a non-empty log; streams are numbered from first_stream."""
+    log = np.ascontiguousarray(log).view(np.uint8).reshape(-1)
+    index = np.ascontiguousarray(index).view(np.int32).reshape(-1, max_subchannels, 2)
+    out = {}
+    for i, k in zip(*np.nonzero(index[..., 1] > 0)):
+        off, n = int(index[i, k, 0]), int(index[i, k, 1])
+        out[(first_stream + int(i), int(k))] = log[off:off + n].tobytes()
+    return out
+
+
 def _step(iq_ptr, iq_stride_bytes, n_samples, block_size, first_stream, n_streams, run_chan_decode, out_ptrs) -> Step:
     st = Step()
     st.iq_host, st.iq_stride_bytes = iq_ptr, iq_stride_bytes
@@ -287,6 +317,7 @@ class DabGpu:
         self.max_streams = max_streams
         self.iq_format = iq_format
         self.P = get_params(mode)
+        self._max_subs = max_subchannels if max_subchannels > 0 else 64
         self._subs = {}
 
     def close(self):
@@ -413,6 +444,27 @@ class DabGpu:
         _check(self.L.dabgpu_chan_get_dabplus_events(self.h, stream, sub_index, _ptr(buf), buf.size, C.byref(n)))
         return buf[:n.value].tobytes()
 
+    def dabplus_out_bound(self, first_stream: int = 0, n_streams: Optional[int] = None) -> int:
+        """dabgpu_dabplus_out_bound: the DAB+ log bytes one decode of these streams can produce (the log_cap to allocate)."""
+        n = self.max_streams - first_stream if n_streams is None else n_streams
+        b = C.c_size_t(0)
+        _check(self.L.dabgpu_dabplus_out_bound(self.h, first_stream, n, C.byref(b)))
+        return b.value
+
+    @property
+    def max_subchannels(self) -> int:
+        return self._max_subs
+
+    def get_dabplus_all(self, first_stream: int = 0, n_streams: Optional[int] = None) -> dict:
+        """dabgpu_chan_get_dabplus_all: {(stream, sub): event log} of the last decode, every non-empty log of the range, each
+        byte-identical to get_dabplus_events(stream, sub)."""
+        n = self.max_streams - first_stream if n_streams is None else n_streams
+        log = np.zeros(max(self.dabplus_out_bound(first_stream, n), 1), dtype=np.uint8)
+        index = np.zeros((max(n, 1), self._max_subs, 2), dtype=np.int32)
+        out = DabPlusOut(log.ctypes.data, log.size, index.ctypes.data)
+        _check(self.L.dabgpu_chan_get_dabplus_all(self.h, first_stream, n, C.byref(out)))
+        return split_dabplus(log, index[:n], first_stream, self._max_subs)
+
     def rs_decode(self, codewords: np.ndarray, nroots: int = 10, pad: int = 135):
         cw = np.ascontiguousarray(codewords, dtype=np.uint8).copy()
         assert cw.ndim == 2 and cw.shape[1] == 255 - pad
@@ -496,13 +548,19 @@ class DabGpu:
         return w
 
     def submit(self, iq_ptr: int, iq_stride_bytes: int, n_samples: int, block_size: int = 65536, first_stream: int = 0,
-               n_streams: Optional[int] = None, run_chan_decode: bool = False, **out_ptrs) -> int:
+               n_streams: Optional[int] = None, run_chan_decode: bool = False, dabplus=None, **out_ptrs) -> int:
         """dabgpu_submit: queue H2D + OFDM (+ channel decode) + D2H without blocking; returns the ticket.
-        out_ptrs: frames_host, produced_host, msc_host, msc_valid_host, fic_host, fic_crc_host, chan_status_host (raw addresses)."""
+        out_ptrs: frames_host, produced_host, msc_host, msc_valid_host, fic_host, fic_crc_host, chan_status_host (raw addresses).
+        dabplus=(log_ptr, log_cap, index_ptr): also copy the DAB+ output of the ticket's decode there (dabgpu_submit_ex;
+        split_dabplus reads it once the ticket was waited for)."""
         st = _step(iq_ptr, iq_stride_bytes, n_samples, block_size, first_stream,
                    self.max_streams - first_stream if n_streams is None else n_streams, run_chan_decode, out_ptrs)
         t = C.c_uint64(0)
-        _check(self.L.dabgpu_submit(self.h, C.byref(st), C.byref(t)))
+        dp = _dabplus_out(dabplus)
+        if dp is None:
+            _check(self.L.dabgpu_submit(self.h, C.byref(st), C.byref(t)))
+        else:
+            _check(self.L.dabgpu_submit_ex(self.h, C.byref(st), C.byref(dp), C.byref(t)))
         return int(t.value)
 
     def wait(self, ticket: int) -> None:
@@ -588,16 +646,20 @@ class Wideband:
         _check(self.L.dabgpu_wideband_reserve(self.h, max_samples))
 
     def submit(self, iq_ptr: int, source_stride_bytes: int, n_samples: int, block_size: int = 65536, first_stream: int = 0,
-               n_streams: Optional[int] = None, run_chan_decode: bool = False, **out_ptrs) -> int:
+               n_streams: Optional[int] = None, run_chan_decode: bool = False, dabplus=None, **out_ptrs) -> int:
         """dabgpu_wideband_submit: queue the upload of n_samples raw samples per source (source s at iq_ptr + s *
         source_stride_bytes, pinned host memory that stays valid until the ticket is waited for), the filter bank and OFDM over
         every channel, the channel decode of channels [first_stream, first_stream + n_streams) if run_chan_decode, and the
         copy-out of out_ptrs (as DabGpu.submit, rows from first_stream) without blocking.  Returns the ticket; retire it with
-        DabGpu.wait."""
+        DabGpu.wait.  dabplus=(log_ptr, log_cap, index_ptr): as DabGpu.submit (dabgpu_wideband_submit_ex)."""
         st = _step(iq_ptr, source_stride_bytes, n_samples, block_size, first_stream,
                    self.n_channels - first_stream if n_streams is None else n_streams, run_chan_decode, out_ptrs)
         t = C.c_uint64(0)
-        _check(self.L.dabgpu_wideband_submit(self.h, C.byref(st), C.byref(t)))
+        dp = _dabplus_out(dabplus)
+        if dp is None:
+            _check(self.L.dabgpu_wideband_submit(self.h, C.byref(st), C.byref(t)))
+        else:
+            _check(self.L.dabgpu_wideband_submit_ex(self.h, C.byref(st), C.byref(dp), C.byref(t)))
         return int(t.value)
 
     def close(self):

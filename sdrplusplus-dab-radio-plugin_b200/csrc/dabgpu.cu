@@ -76,6 +76,7 @@ struct dabgpu_ctx {
         cudaEvent_t h2d_done = nullptr, compute_done = nullptr, d2h_done = nullptr;
         DevBuf d_stage, d_produced;
         DevBuf d_written0;   // frames_written of the ticket's streams before its first OFDM run (dabgpu_wideband_submit)
+        DevBuf d_dpout;      // the ticket's packed DAB+ log, then its index (dabgpu_submit_ex / dabgpu_wideband_submit_ex)
         uint64_t ticket = 0;
         bool busy = false;
     } pipe[DABGPU_PIPELINE_DEPTH];
@@ -330,6 +331,7 @@ void dabgpu_ctx_destroy(dabgpu_ctx* ctx) {
         sl.d_stage.release();
         sl.d_produced.release();
         sl.d_written0.release();
+        sl.d_dpout.release();
     }
     if (ctx->s_dp) { cudaStreamSynchronize(ctx->s_dp); cudaStreamDestroy(ctx->s_dp); }
     if (ctx->ev_dp) cudaEventDestroy(ctx->ev_dp);
@@ -1027,6 +1029,92 @@ int dabgpu_chan_get_dabplus_events(dabgpu_ctx* ctx, int stream, int sub_index, u
     return dabplus_get_events(ctx->dabplus, stream, sub_index, log_host, log_cap, log_bytes);
 }
 
+// The packed DAB+ output layout over every stream: dp_pack_item_bound for each active DAB+ sub-channel, 0 for every other
+// entry of the [max_streams][max_subs] table.  It depends only on the sub-channel tables and is rebuilt when they change
+// (cfg_epoch).  Every table change first synchronises the context, so no queued pack still reads the device copy then.
+static const std::vector<uint64_t>& dp_layout(dabgpu_ctx* ctx) {
+    DabPlusState& D = ctx->dabplus;
+    if (D.layout_epoch != ctx->cfg_epoch) {
+        const size_t ms = size_t(ctx->max_subs);
+        D.layout.assign(ctx->subs.size() * ms + 1, 0);
+        uint64_t at = 0;
+        for (size_t s = 0; s < ctx->subs.size(); s++)
+            for (size_t k = 0; k < ms; k++) {
+                D.layout[s * ms + k] = at;
+                const SubHost* h = k < ctx->subs[s].size() ? &ctx->subs[s][k] : nullptr;
+                if (h && h->active && h->sc.is_dabplus) at += dp_pack_item_bound(h->n_out_bytes);
+            }
+        D.layout.back() = at;
+        D.layout_epoch = ctx->cfg_epoch;
+    }
+    return D.layout;
+}
+
+// Log bytes one decode of streams [first, first + n) can produce; the index holds int32 offsets, so it must stay below 2^31.
+static int dp_range_bound(dabgpu_ctx* ctx, int first, int n, size_t* bytes) {
+    const std::vector<uint64_t>& lay = dp_layout(ctx);
+    const uint64_t b = lay[size_t(first + n) * ctx->max_subs] - lay[size_t(first) * ctx->max_subs];
+    if (b > uint64_t(INT32_MAX)) return set_error(DABGPU_ERR_INVALID, "DAB+ log of streams [%d,%d) may reach %llu bytes: use smaller ranges", first, first + n, (unsigned long long)b);
+    *bytes = size_t(b);
+    return DABGPU_OK;
+}
+
+// A DAB+ output request for streams [first, first + n), checked before anything is queued.
+static int dp_check_out(dabgpu_ctx* ctx, int first, int n, const dabgpu_dabplus_out* out, size_t* log_bytes) {
+    if (!out->log_host || !out->index_host) return set_error(DABGPU_ERR_INVALID, "null DAB+ log or index buffer");
+    int rc = dp_range_bound(ctx, first, n, log_bytes);
+    if (rc) return rc;
+    if (out->log_cap < *log_bytes) return set_error(DABGPU_ERR_OVERFLOW, "DAB+ log buffer of %zu bytes, streams [%d,%d) need %zu (dabgpu_dabplus_out_bound)", out->log_cap, first, first + n, *log_bytes);
+    return DABGPU_OK;
+}
+
+// Queues k_dabplus_pack on ctx->stream into d_buf: the log (log_bytes) first, the index at dp_index_offset(log_bytes).
+static size_t dp_index_offset(size_t log_bytes) { return (log_bytes + 255u) & ~size_t(255); }
+static int dp_pack(dabgpu_ctx* ctx, int first, int n, size_t log_bytes, DevBuf& d_buf) {
+    DabPlusState& D = ctx->dabplus;
+    const std::vector<uint64_t>& lay = dp_layout(ctx);
+    int rc;
+    if (D.layout_dev_epoch != D.layout_epoch) {
+        if ((rc = D.d_layout.alloc(lay.size() * sizeof(uint64_t)))) return rc;
+        CUDA_TRY(cudaMemcpyAsync(D.d_layout.p, lay.data(), lay.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
+        D.layout_dev_epoch = D.layout_epoch;
+    }
+    const size_t at = dp_index_offset(log_bytes);
+    if ((rc = d_buf.alloc(at + size_t(n) * ctx->max_subs * 8))) return rc;
+    uint32_t subs_per_stream = 0;
+    for (int s = first; s < first + n; s++) subs_per_stream = std::max(subs_per_stream, uint32_t(ctx->subs[size_t(s)].size()));
+    return dabplus_pack(D, first, n, subs_per_stream, d_buf.as<uint8_t>(), reinterpret_cast<int32_t*>(d_buf.as<uint8_t>() + at), ctx->stream,
+                        &ctx->launches, ctx->prof);
+}
+
+static int dp_copy_out(dabgpu_ctx* ctx, int n, size_t log_bytes, const DevBuf& d_buf, const dabgpu_dabplus_out* out, cudaStream_t s) {
+    CUDA_TRY(cudaMemcpyAsync(out->log_host, d_buf.p, log_bytes, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaMemcpyAsync(out->index_host, d_buf.as<uint8_t>() + dp_index_offset(log_bytes), size_t(n) * ctx->max_subs * 8, cudaMemcpyDeviceToHost, s));
+    return DABGPU_OK;
+}
+
+int dabgpu_dabplus_out_bound(dabgpu_ctx* ctx, int first_stream, int n_streams, size_t* log_bytes) {
+    int rc = check_stream_range(ctx, first_stream, n_streams);
+    if (rc) return rc;
+    if (!log_bytes) return set_error(DABGPU_ERR_INVALID, "null output");
+    return dp_range_bound(ctx, first_stream, n_streams, log_bytes);
+}
+
+int dabgpu_chan_get_dabplus_all(dabgpu_ctx* ctx, int first_stream, int n_streams, const dabgpu_dabplus_out* out) {
+    int rc = check_stream_range(ctx, first_stream, n_streams);
+    if (rc) return rc;
+    if (!out) return set_error(DABGPU_ERR_INVALID, "null DAB+ output");
+    size_t log_bytes = 0;
+    if ((rc = dp_check_out(ctx, first_stream, n_streams, out, &log_bytes))) return rc;
+    if (n_streams == 0) return DABGPU_OK;
+    CUDA_TRY(cudaSetDevice(ctx->cfg.device));
+    CUDA_TRY(join_dabplus(ctx));
+    if ((rc = dp_pack(ctx, first_stream, n_streams, log_bytes, ctx->dabplus.d_out))) return rc;
+    if ((rc = dp_copy_out(ctx, n_streams, log_bytes, ctx->dabplus.d_out, out, ctx->stream))) return rc;
+    CUDA_TRY(sync_ctx(ctx));
+    return DABGPU_OK;
+}
+
 int dabgpu_rs_decode(dabgpu_ctx* ctx, uint8_t* codewords_host, int n_codewords, int nroots, int pad, int* counts_host, int* positions_host) {
     if (!ctx || !codewords_host || !counts_host) return set_error(DABGPU_ERR_INVALID, "null argument");
     CUDA_TRY(cudaSetDevice(ctx->cfg.device));
@@ -1346,8 +1434,10 @@ static int pipe_acquire(dabgpu_ctx* ctx, dabgpu_ctx::PipeSlot** out) {
 
 // Everything of a ticket after its OFDM stage, which the caller has queued on the compute stream: the newest frame of every
 // stream that produced one (during the last OFDM run, or since the counters in d_written0 when given), the channel decode,
-// and the device->host copies of the non-NULL result pointers of st on the copy-out stream.
-static int pipe_finish(dabgpu_ctx* ctx, dabgpu_ctx::PipeSlot& sl, const dabgpu_step* st, const uint32_t* d_written0, uint64_t* ticket) {
+// the DAB+ pack when dp is given (dp_log = its bound, checked by dp_check_out), and the device->host copies of the non-NULL
+// result pointers of st and of dp on the copy-out stream.
+static int pipe_finish(dabgpu_ctx* ctx, dabgpu_ctx::PipeSlot& sl, const dabgpu_step* st, const uint32_t* d_written0, const dabgpu_dabplus_out* dp,
+                       size_t dp_log, uint64_t* ticket) {
     int rc;
     OfdmState& O = ctx->ofdm;
     const int n = st->n_streams, first = st->first_stream;
@@ -1361,6 +1451,10 @@ static int pipe_finish(dabgpu_ctx* ctx, dabgpu_ctx::PipeSlot& sl, const dabgpu_s
     }
     if (st->run_chan_decode && (rc = dabgpu_chan_decode(ctx, first, n))) return rc;
     CUDA_TRY(join_dabplus(ctx));
+    // The pack reads the decode's event queues and superframes on the compute stream, after the join.  Ticket t + 1's channel
+    // decode, which overwrites them, forks from this stream after this point, so the output is this ticket's decode; nothing
+    // else orders the two.  It writes the slot's own buffer, so the next compute need not wait for the copy-out.
+    if (dp && (rc = dp_pack(ctx, first, n, dp_log, sl.d_dpout))) return rc;
     CUDA_TRY(cudaEventRecord(sl.compute_done, ctx->stream));
     // Copy out.  The next compute may overwrite the channel-decode arenas: it is made to wait for this copy.
     CUDA_TRY(cudaStreamWaitEvent(ctx->s_d2h, sl.compute_done, 0));
@@ -1373,6 +1467,7 @@ static int pipe_finish(dabgpu_ctx* ctx, dabgpu_ctx::PipeSlot& sl, const dabgpu_s
     if (st->fic_host) { arenas = true; CUDA_TRY(cudaMemcpyAsync(st->fic_host, ctx->d_fic_out.as<uint8_t>() + size_t(first) * nb_cifs * FIC_GROUP_BYTES, size_t(n) * nb_cifs * FIC_GROUP_BYTES, cudaMemcpyDeviceToHost, ctx->s_d2h)); }
     if (st->fic_crc_host) { arenas = true; CUDA_TRY(cudaMemcpyAsync(st->fic_crc_host, ctx->d_fic_crc.as<uint8_t>() + size_t(first) * nb_cifs * 4, size_t(n) * nb_cifs * 4, cudaMemcpyDeviceToHost, ctx->s_d2h)); }
     if (st->chan_status_host) { arenas = true; CUDA_TRY(cudaMemcpyAsync(st->chan_status_host, ctx->d_status.as<int32_t>() + 2 * size_t(first), size_t(n) * 8, cudaMemcpyDeviceToHost, ctx->s_d2h)); }
+    if (dp && (rc = dp_copy_out(ctx, n, dp_log, sl.d_dpout, dp, ctx->s_d2h))) return rc;
     CUDA_TRY(cudaEventRecord(sl.d2h_done, ctx->s_d2h));
     if (arenas) CUDA_TRY(cudaStreamWaitEvent(ctx->stream, sl.d2h_done, 0));
     sl.busy = true;
@@ -1383,11 +1478,22 @@ static int pipe_finish(dabgpu_ctx* ctx, dabgpu_ctx::PipeSlot& sl, const dabgpu_s
 
 extern "C" {
 
-int dabgpu_submit(dabgpu_ctx* ctx, const dabgpu_step* st, uint64_t* ticket) {
+int dabgpu_submit(dabgpu_ctx* ctx, const dabgpu_step* st, uint64_t* ticket) { return dabgpu_submit_ex(ctx, st, nullptr, ticket); }
+
+// DAB+ output of a ticket: asked for with the channel decode it packs, and refused before anything is queued.
+static int dp_check_step(dabgpu_ctx* ctx, const dabgpu_step* st, const dabgpu_dabplus_out* dp, size_t* dp_log) {
+    if (!dp) return DABGPU_OK;
+    if (!st->run_chan_decode) return set_error(DABGPU_ERR_INVALID, "DAB+ output needs run_chan_decode");
+    return dp_check_out(ctx, st->first_stream, st->n_streams, dp, dp_log);
+}
+
+int dabgpu_submit_ex(dabgpu_ctx* ctx, const dabgpu_step* st, const dabgpu_dabplus_out* dp, uint64_t* ticket) {
     if (!ctx || !st || !ticket) return set_error(DABGPU_ERR_INVALID, "null argument");
     int rc = check_stream_range(ctx, st->first_stream, st->n_streams);
     if (rc) return rc;
     if (!st->iq_host || st->n_samples <= 0 || st->n_streams == 0) return set_error(DABGPU_ERR_INVALID, "bad IQ buffer");
+    size_t dp_log = 0;
+    if ((rc = dp_check_step(ctx, st, dp, &dp_log))) return rc;
     OfdmState& O = ctx->ofdm;
     if (O.external_ring) return set_error(DABGPU_ERR_STATE, "a device input buffer is attached: use dabgpu_ofdm_advance");
     CUDA_TRY(cudaSetDevice(ctx->cfg.device));
@@ -1412,7 +1518,7 @@ int dabgpu_submit(dabgpu_ctx* ctx, const dabgpu_step* st, uint64_t* ticket) {
     ctx->ofdm.demod_ctas_cap = ctx->dp_pending ? 3 : 0;   // a channel decode is running on its stream: share the SMs with it
     if ((rc = ofdm_run(O, first, n, st->n_samples, bs, ctx->stream))) return rc;
     // (3) channel decode and copy out
-    if ((rc = pipe_finish(ctx, *sl, st, nullptr, ticket))) return rc;
+    if ((rc = pipe_finish(ctx, *sl, st, nullptr, dp, dp_log, ticket))) return rc;
     ctx->pipe_recent_samples[t % DABGPU_PIPELINE_DEPTH] = size_t(st->n_samples);
     return DABGPU_OK;
 }
@@ -1841,7 +1947,9 @@ int dabgpu_wideband_reserve(dabgpu_wideband* w, size_t max_submit_samples) {
 
 // Pipelined dabgpu_wideband_process + dabgpu_chan_decode: (1) the upload on the copy stream, (2) the filter bank and OFDM
 // passes, the newest frames and the channel decode on the compute stream, (3) the copy-out, as in dabgpu_submit (pipe_finish).
-int dabgpu_wideband_submit(dabgpu_wideband* w, const dabgpu_step* st, uint64_t* ticket) {
+int dabgpu_wideband_submit(dabgpu_wideband* w, const dabgpu_step* st, uint64_t* ticket) { return dabgpu_wideband_submit_ex(w, st, nullptr, ticket); }
+
+int dabgpu_wideband_submit_ex(dabgpu_wideband* w, const dabgpu_step* st, const dabgpu_dabplus_out* dp, uint64_t* ticket) {
     if (!w || !st || !ticket) return set_error(DABGPU_ERR_INVALID, "null argument");
     dabgpu_ctx* ctx = w->ctx;
     if (!ctx) return set_error(DABGPU_ERR_STATE, "the context of this wideband front end was destroyed");
@@ -1854,8 +1962,11 @@ int dabgpu_wideband_submit(dabgpu_wideband* w, const dabgpu_step* st, uint64_t* 
         return set_error(DABGPU_ERR_INVALID, "n_samples %zu exceeds the %zu samples per ticket set with dabgpu_wideband_reserve", n_samples, w->max_submit);
     if (w->n_sources > 1 && st->iq_stride_bytes < n_samples * size_t(w->bps))
         return set_error(DABGPU_ERR_INVALID, "source stride %zu is shorter than a source", st->iq_stride_bytes);
+    size_t dp_log = 0;
+    int rc = dp_check_step(ctx, st, dp, &dp_log);
+    if (rc) return rc;
     size_t bs, new_out;
-    int rc = wb_begin(w, n_samples, st->block_size, &bs, &new_out);
+    rc = wb_begin(w, n_samples, st->block_size, &bs, &new_out);
     if (rc) return rc;
     dabgpu_ctx::PipeSlot* sl;
     if ((rc = pipe_acquire(ctx, &sl))) return rc;
@@ -1873,7 +1984,7 @@ int dabgpu_wideband_submit(dabgpu_wideband* w, const dabgpu_step* st, uint64_t* 
     for (bool last = false; !last;)
         if ((rc = wb_pass(w, bs, true, &last))) return rc;
     // (3) channel decode and copy out
-    return pipe_finish(ctx, *sl, st, sl->d_written0.as<uint32_t>(), ticket);
+    return pipe_finish(ctx, *sl, st, sl->d_written0.as<uint32_t>(), dp, dp_log, ticket);
 }
 
 int dabgpu_wideband_close(dabgpu_wideband* w) {

@@ -29,6 +29,11 @@ struct DabPlusState {
     DevBuf d_st, d_sf, d_sf_out, d_events, d_nevents, d_rs_cw, d_rs_cnt, d_rs_pos;
     DabPlusDev dev;
     int max_streams = 0, max_subs = 0, nb_cifs = 0;
+    // packed output (k_dabplus_pack): item (stream, sub) starts at layout[stream * max_subs + sub] of a log that covers every
+    // stream; layout[item + 1] - layout[item] is its bound.  Built on the host from the sub-channel tables (dp_layout).
+    std::vector<uint64_t> layout;
+    uint64_t layout_epoch = 0, layout_dev_epoch = 0;
+    DevBuf d_layout, d_out;   // d_out: the pack of dabgpu_chan_get_dabplus_all
 };
 
 struct GfTables { const uint8_t* ex; const uint8_t* lg; };
@@ -404,6 +409,88 @@ k_dabplus(const ChanDev C, const DabPlusDev D, const int first_stream, const int
     }
 }
 
+// Bound of one (stream, sub-channel) log per channel decode.  A decode runs one transmission frame per stream, at most 4 CIFs
+// (mode I), and a superframe takes 5 logical frames, so at most one superframe completes per item and call.  The item then
+// fires at most 7 events: the header and 6 AUs or AU CRC errors; or an RS / fire-code failure and at most 3 fire-code errors
+// of the CIFs after it (4 fire-code errors when nothing completes).  Its AU payloads are disjoint pieces of the 5 n-byte
+// superframe, each padded to 4.  Items start 8-byte aligned.
+#define DP_PACK_MAX_CIFS 4
+#define DP_PACK_MAX_EVENTS 7
+static_assert(DP_PACK_MAX_CIFS < 5, "two superframes could complete in one decode call");
+static_assert(DP_PACK_MAX_EVENTS <= DP_MAX_EVENTS, "the event queue of an item must hold a whole decode call");
+static inline uint64_t dp_pack_item_bound(const uint32_t n_out_bytes) {
+    return (uint64_t(DP_PACK_MAX_EVENTS) * 24u + 5u * uint64_t(n_out_bytes) + 6u * 3u + 7u) & ~uint64_t(7);
+}
+
+// n payload bytes zero-padded to 4 by a warp; dst is 4-byte aligned.  AUs rarely start on 8 bytes (the AU-start table leaves
+// AU 0 at 5, 6, 8 or 11 bytes into the superframe), so outside the 8-byte path each lane assembles whole 4-byte words.
+__device__ __forceinline__ void dp_pack_payload(uint8_t* __restrict__ dst, const uint8_t* __restrict__ src, const int n, const uint32_t lane) {
+    if (((reinterpret_cast<uintptr_t>(dst) | reinterpret_cast<uintptr_t>(src) | uintptr_t(n)) & 7u) == 0u) {
+        dp_copy_bytes(dst, src, n, lane);
+        return;
+    }
+    uint32_t* d4 = reinterpret_cast<uint32_t*>(dst);
+    const int n4 = (n + 3) >> 2;
+    for (int i = int(lane); i < n4; i += 32) {
+        uint32_t v = 0u;
+#pragma unroll
+        for (int b = 0; b < 4; b++) if (4 * i + b < n) v |= uint32_t(src[4 * i + b]) << (8 * b);
+        d4[i] = v;
+    }
+}
+
+// One warp per (stream, sub-channel) of streams [first, first + n), sub-channels below subs_per_stream (the longest table of
+// those streams): the item's observer log, byte-identical to what dabplus_get_events builds on the host (24-byte headers, AU
+// payloads from sf_out padded to 4), at layout[item] - layout[first item] of `log`, and {offset, length} at its place of the
+// [n][max_subs][2] index.  Entries with an empty log (not an active DAB+ sub-channel, no events, rows from subs_per_stream on,
+// which the warp of sub-channel 0 fills) get {0, 0}.  The offsets are static, so no warp waits for another.
+__global__ void __launch_bounds__(256) k_dabplus_pack(const DabPlusDev D, const uint64_t* __restrict__ layout, const int first, const int n,
+                                                      const int max_subs, const uint32_t subs_per_stream, uint8_t* __restrict__ log,
+                                                      int32_t* __restrict__ index) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint64_t base = layout[size_t(first) * max_subs];
+    const uint32_t total = uint32_t(n) * subs_per_stream;
+    for (uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < total; w += (gridDim.x * blockDim.x) >> 5) {
+        const uint32_t si = w / subs_per_stream, sub = w - si * subs_per_stream;
+        if (sub == 0)
+            for (uint32_t k = subs_per_stream + lane; k < uint32_t(max_subs); k += 32) {
+                index[2 * (size_t(si) * max_subs + k)] = 0;
+                index[2 * (size_t(si) * max_subs + k) + 1] = 0;
+            }
+        const size_t row = size_t(si) * max_subs + sub, idx = size_t(first) * max_subs + row;
+        const uint64_t off = layout[idx] - base;
+        const int n_ev = (layout[idx + 1] > layout[idx]) ? min(D.n_events[idx], DP_MAX_EVENTS) : 0;
+        DabPlusEvent e{0, 0, 0, 0, 0, 0, 0, 0};
+        int size = 0;
+        if (int(lane) < n_ev) {
+            e = D.events[idx * DP_MAX_EVENTS + lane];
+            size = 24 + ((e.payload_len + 3) & ~3);
+        }
+        int end = size;   // inclusive prefix over the events: record k ends at lane k's value
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int v = __shfl_up_sync(FULL_MASK, end, o);
+            if (int(lane) >= o) end += v;
+        }
+        const int len = __shfl_sync(FULL_MASK, end, 31);
+        const int at = end - size;
+        uint8_t* item = log + off;
+        if (int(lane) < n_ev) {
+            int32_t* h = reinterpret_cast<int32_t*>(item + at);
+            h[0] = e.type; h[1] = e.a; h[2] = e.b; h[3] = e.c; h[4] = e.d; h[5] = e.payload_len;
+        }
+        const uint8_t* sf = D.sf_out + (size_t(first) + si) * (5u * CIF_OUT_STRIDE);
+        for (int k = 0; k < n_ev; k++) {
+            const int plen = __shfl_sync(FULL_MASK, e.payload_len, k);
+            const int poff = __shfl_sync(FULL_MASK, e.payload_off, k);
+            const int dst = __shfl_sync(FULL_MASK, at, k) + 24;
+            if (plen > 0) dp_pack_payload(item + dst, sf + poff, plen, lane);
+        }
+        if (lane == 0) { index[2 * row] = len ? int32_t(off) : 0; index[2 * row + 1] = len; }
+        __syncwarp();
+    }
+}
+
 // Stand-alone AAC_Frame_Processor objects (the C++ adapter of the same name): one warp, one logical frame per call.
 struct DabPlusProc {
     DabPlusSubState st;
@@ -494,7 +581,7 @@ static int dabplus_init(DabPlusState& S, int max_streams, int max_subs, int nb_c
 }
 
 static void dabplus_destroy(DabPlusState& S) {
-    DevBuf* bufs[] = {&S.d_st, &S.d_sf, &S.d_sf_out, &S.d_events, &S.d_nevents, &S.d_rs_cw, &S.d_rs_cnt, &S.d_rs_pos};
+    DevBuf* bufs[] = {&S.d_st, &S.d_sf, &S.d_sf_out, &S.d_events, &S.d_nevents, &S.d_rs_cw, &S.d_rs_cnt, &S.d_rs_pos, &S.d_layout, &S.d_out};
     for (DevBuf* b : bufs) b->release();
 }
 
@@ -511,6 +598,21 @@ static int dabplus_run(DabPlusState& S, const ChanDev& C, int first, int n, uint
     const uint32_t ctas = std::min((warps + DP_WARPS - 1) / DP_WARPS, uint32_t(num_sms) * 8u);
     pf.begin(PROF_DABPLUS, stream);
     k_dabplus<<<ctas, DP_WARPS * 32, 0, stream>>>(C, S.dev, first, n, subs_per_stream);
+    pf.end(stream);
+    (*launches)++;
+    CUDA_TRY(cudaGetLastError());
+    return DABGPU_OK;
+}
+
+// k_dabplus_pack over streams [first, first + n) with S.d_layout on the device, one warp per item: a warp walks its item's
+// dependent loads (layout, event count, events, payloads) in a few microseconds, so the items are spread over as many warps as
+// the GPU holds rather than looped over a persistent grid.
+static int dabplus_pack(DabPlusState& S, int first, int n, uint32_t subs_per_stream, uint8_t* d_log, int32_t* d_index, cudaStream_t stream,
+                        uint64_t* launches, Profiler& pf) {
+    const uint32_t warps = uint32_t(n) * std::max(subs_per_stream, 1u);
+    pf.begin(PROF_DABPLUS, stream);
+    k_dabplus_pack<<<(warps + 7u) / 8u, 256, 0, stream>>>(S.dev, S.d_layout.as<uint64_t>(), first, n, S.max_subs, std::max(subs_per_stream, 1u),
+                                                          d_log, d_index);
     pf.end(stream);
     (*launches)++;
     CUDA_TRY(cudaGetLastError());
