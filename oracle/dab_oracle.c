@@ -780,6 +780,13 @@ void dabo_ofdm_destroy(dabo_ofdm* d) {
     free(d->fftbuf); free(d->ifftbuf); free(d->spectra); free(d->impulse); free(d->freq_resp); free(d->phase_err);
     free(d->cmap); fft_free(d->plan); free(d->scratch); free(d);
 }
+void dabo_ofdm_set_config(dabo_ofdm* d, const dabo_ofdm_config* c) {
+    d->l1_beta = c->signal_l1_update_beta; d->l1_nb_samples = c->signal_l1_nb_samples; d->l1_decimate = c->signal_l1_nb_decimate;
+    d->thresh_null_start = c->null_thresh_start; d->thresh_null_end = c->null_thresh_end;
+    d->fine_beta = c->fine_freq_update_beta; d->coarse_enabled = c->is_coarse_freq_correction;
+    d->max_coarse_norm = c->max_coarse_freq_correction_norm; d->coarse_slow_beta = c->coarse_freq_slow_beta;
+    d->impulse_thresh_db = c->impulse_peak_threshold_db; d->impulse_dist_prob = c->impulse_peak_distance_probability;
+}
 int dabo_ofdm_frame_bits(const dabo_ofdm* d) { return (d->L - 1)*d->K*2; }
 void dabo_ofdm_keep_frames(dabo_ofdm* d, int keep) { d->keep = keep; }
 

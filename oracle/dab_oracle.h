@@ -54,7 +54,23 @@ int  dabo_aac_process(dabo_aac*, const uint8_t* frame, int n, uint8_t* log_out, 
 
 /* ---- OFDM ---- */
 typedef struct dabo_ofdm dabo_ofdm;
+/* OFDM_Demod_Config (ofdm_demodulator.h:24-45), fields in the order of dabgpu_ofdm_config */
+typedef struct {
+    float signal_l1_update_beta;
+    int   signal_l1_nb_samples;
+    int   signal_l1_nb_decimate;
+    float null_thresh_start;
+    float null_thresh_end;
+    float fine_freq_update_beta;
+    int   is_coarse_freq_correction;
+    float max_coarse_freq_correction_norm;
+    float coarse_freq_slow_beta;
+    float impulse_peak_threshold_db;
+    float impulse_peak_distance_probability;
+} dabo_ofdm_config;
 dabo_ofdm* dabo_ofdm_create(int mode);
+/* OFDM_Demod::GetConfig() = *cfg: in force from the next process call on */
+void dabo_ofdm_set_config(dabo_ofdm*, const dabo_ofdm_config* cfg);
 void dabo_ofdm_destroy(dabo_ofdm*);
 int  dabo_ofdm_frame_bits(const dabo_ofdm*);
 void dabo_ofdm_process_c32(dabo_ofdm*, const float* iq, int n_samples);

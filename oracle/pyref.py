@@ -93,6 +93,8 @@ class RefLib:
         L.ref_ofdm_get_state.argtypes = [C.c_void_p, _i32p, _f32p]
         L.ref_ofdm_reset.argtypes = [C.c_void_p]
         L.ref_ofdm_set_coarse_enabled.argtypes = [C.c_void_p, C.c_int]
+        if hasattr(L, "ref_ofdm_set_config"):
+            L.ref_ofdm_set_config.argtypes = [C.c_void_p, _f32p, _i32p]
         L.ref_ofdm_get_frame_fft.argtypes = [C.c_void_p, _f32p, C.c_int]
         L.ref_ofdm_get_impulse_response.argtypes = [C.c_void_p, _f32p, C.c_int]
         if hasattr(L, "ref_ofdm_get_correlation_buffer"):
@@ -371,11 +373,23 @@ class RefOfdm:
         if not self.h:
             raise ValueError(f"invalid transmission mode {mode}")
         self.frame_bits = self.lib.ref_ofdm_frame_bits(self.h)
+        self.config = dict(OFDM_DEFAULTS)
 
     def __del__(self):
         if getattr(self, "h", None):
             self.lib.ref_ofdm_destroy(self.h)
             self.h = None
+
+    def set_config(self, **kw):
+        """OFDM_Demod::GetConfig() edited between Process() calls; keywords as DabGpu.ofdm_set_config, unnamed knobs keep
+        their current values."""
+        self.config = _merge_config(self.config, kw)
+        c = self.config
+        f8 = np.array([c[k] for k in ("signal_l1_update_beta", "null_thresh_start", "null_thresh_end", "fine_freq_update_beta",
+                                      "max_coarse_freq_correction_norm", "coarse_freq_slow_beta", "impulse_peak_threshold_db",
+                                      "impulse_peak_distance_probability")], dtype=np.float32)
+        i3 = np.array([c["signal_l1_nb_samples"], c["signal_l1_nb_decimate"], c["is_coarse_freq_correction"]], dtype=np.int32)
+        self.lib.ref_ofdm_set_config(self.h, f8, i3)
 
     def process_u8(self, iq_u8: np.ndarray, serial: bool = True):
         iq_u8 = np.ascontiguousarray(iq_u8, dtype=np.uint8)
@@ -432,6 +446,41 @@ class RefOfdm:
         return out
 
 
+class OfdmConfig(C.Structure):
+    """dabo_ofdm_config = dabgpu_ofdm_config (include/dabgpu.h): OFDM_Demod_Config, ofdm_demodulator.h:24-45"""
+    _fields_ = [("signal_l1_update_beta", C.c_float), ("signal_l1_nb_samples", C.c_int), ("signal_l1_nb_decimate", C.c_int),
+                ("null_thresh_start", C.c_float), ("null_thresh_end", C.c_float), ("fine_freq_update_beta", C.c_float),
+                ("is_coarse_freq_correction", C.c_int), ("max_coarse_freq_correction_norm", C.c_float),
+                ("coarse_freq_slow_beta", C.c_float), ("impulse_peak_threshold_db", C.c_float),
+                ("impulse_peak_distance_probability", C.c_float)]
+
+
+OFDM_DEFAULTS = dict(signal_l1_update_beta=0.95, signal_l1_nb_samples=100, signal_l1_nb_decimate=5, null_thresh_start=0.35,
+                     null_thresh_end=0.75, fine_freq_update_beta=0.9, is_coarse_freq_correction=1,
+                     max_coarse_freq_correction_norm=0.5, coarse_freq_slow_beta=0.1, impulse_peak_threshold_db=20.0,
+                     impulse_peak_distance_probability=0.15)
+
+
+def _merge_config(cur: dict, kw: dict) -> dict:
+    unknown = set(kw) - set(OFDM_DEFAULTS)
+    if unknown:
+        raise KeyError(f"unknown OFDM knobs {sorted(unknown)}")
+    return {**cur, **kw}
+
+
+def ofdm_process_call(o, iq: np.ndarray, block_size: int, u8: bool = True) -> None:
+    """Feeds the OFDM oracle `o` one call as dabgpu_ofdm_process(n_samples, block_size) presents it: consecutive Process()
+    blocks of block_size samples (<= 0: one block), the last one partial; the next call starts a new block."""
+    n = iq.size // 2 if u8 else iq.size
+    bs = block_size if block_size > 0 else n
+    for off in range(0, n, bs):
+        end = min(n, off + bs)
+        if u8:
+            o.process_u8(iq[2 * off:2 * end])
+        else:
+            o.process_c32(iq[off:end])
+
+
 def ref_tables(mode: int):
     L = RefLib.get().L
     p = np.zeros(6, dtype=np.int32)
@@ -450,6 +499,28 @@ def ref_tables(mode: int):
 # =============================================================================================
 # Plain-C restatement (oracle/dab_oracle.c)
 # =============================================================================================
+def _refresh_port() -> None:
+    """Brings oracle/_ref/libdaboracle.so up to date with dab_oracle.c before the first load: make rebuilds it when the sources
+    are newer, and a library that lacks an entry point this module binds (built from older sources but stamped later, e.g. left
+    over from another checkout) is rebuilt unconditionally.  A library that cannot be rebuilt is loaded as it is."""
+    import subprocess
+    try:
+        subprocess.run(["make", "-s", "port"], cwd=_HERE, capture_output=True, check=False)
+        nm = subprocess.run(["nm", "-D", "--defined-only", PORT_SO], capture_output=True, text=True, check=False)
+    except OSError:
+        return
+    defined = {line.split()[-1] for line in nm.stdout.splitlines() if line.strip()}
+    src = open(os.path.join(_HERE, "dab_oracle.h")).read()
+    if nm.returncode == 0 and any(name not in defined for name in _declared(src)):
+        subprocess.run(["make", "-s", "-B", "port"], cwd=_HERE, capture_output=True, check=False)
+
+
+def _declared(header: str) -> List[str]:
+    """the dabo_* functions oracle/dab_oracle.h declares"""
+    import re
+    return sorted(set(re.findall(r"\b(dabo_\w+)\s*\(", header)))
+
+
 class PortLib:
     _inst = None
 
@@ -460,6 +531,7 @@ class PortLib:
         return cls._inst
 
     def __init__(self):
+        _refresh_port()
         L = C.CDLL(PORT_SO)
         self.L = L
         L.dabo_pi_counts.argtypes = [C.c_int, _u8p]
@@ -482,6 +554,7 @@ class PortLib:
         L.dabo_aac_destroy.argtypes = [C.c_void_p]
         L.dabo_aac_process.argtypes = [C.c_void_p, _u8p, C.c_int, _u8p, C.c_int]
         L.dabo_ofdm_create.argtypes = [C.c_int]
+        L.dabo_ofdm_set_config.argtypes = [C.c_void_p, C.POINTER(OfdmConfig)]
         L.dabo_ofdm_create.restype = C.c_void_p
         L.dabo_ofdm_destroy.argtypes = [C.c_void_p]
         L.dabo_ofdm_frame_bits.argtypes = [C.c_void_p]
@@ -695,11 +768,17 @@ class PortOfdm:
         if not self.h:
             raise ValueError(f"invalid transmission mode {mode}")
         self.frame_bits = self.lib.dabo_ofdm_frame_bits(self.h)
+        self.config = dict(OFDM_DEFAULTS)
 
     def __del__(self):
         if getattr(self, "h", None):
             self.lib.dabo_ofdm_destroy(self.h)
             self.h = None
+
+    def set_config(self, **kw):
+        """as RefOfdm.set_config"""
+        self.config = _merge_config(self.config, kw)
+        self.lib.dabo_ofdm_set_config(self.h, C.byref(OfdmConfig(**self.config)))
 
     def process_u8(self, iq_u8: np.ndarray, serial: bool = True):
         iq_u8 = np.ascontiguousarray(iq_u8, dtype=np.uint8)

@@ -485,6 +485,24 @@ API void ref_ofdm_get_state(void* h, int* state4, float* fstate3) {
 }
 API void ref_ofdm_reset(void* h) { ((RefOfdm*)h)->demod->Reset(); }
 API void ref_ofdm_set_coarse_enabled(void* h, int en) { ((RefOfdm*)h)->demod->GetConfig().sync.is_coarse_freq_correction = en != 0; }
+// OFDM_Demod::GetConfig() edited the way the plugin's GUI edits it between Process() calls; f8 / i3 in the order of
+// dabgpu_ofdm_config: f8 = {l1 update_beta, thresh_null_start, thresh_null_end, fine_freq_update_beta,
+// max_coarse_freq_correction_norm, coarse_freq_slow_beta, impulse_peak_threshold_db, impulse_peak_distance_probability},
+// i3 = {l1 nb_samples, l1 nb_decimate, is_coarse_freq_correction}
+API void ref_ofdm_set_config(void* h, const float* f8, const int* i3) {
+    auto& c = ((RefOfdm*)h)->demod->GetConfig();
+    c.signal_l1.update_beta = f8[0];
+    c.signal_l1.nb_samples = i3[0];
+    c.signal_l1.nb_decimate = i3[1];
+    c.null_l1_search.thresh_null_start = f8[1];
+    c.null_l1_search.thresh_null_end = f8[2];
+    c.sync.fine_freq_update_beta = f8[3];
+    c.sync.is_coarse_freq_correction = i3[2] != 0;
+    c.sync.max_coarse_freq_correction_norm = f8[4];
+    c.sync.coarse_freq_slow_beta = f8[5];
+    c.sync.impulse_peak_threshold_db = f8[6];
+    c.sync.impulse_peak_distance_probability = f8[7];
+}
 
 // Diagnostic taps for stage-level parity (valid after a frame callback, serial driver only)
 API void ref_ofdm_get_frame_fft(void* h, float* out, int n_complex) {

@@ -507,10 +507,11 @@ class DabGpu:
     def ofdm_set_config(self, **kw) -> None:
         cfg = Config()
         self.L.dabgpu_config_default(C.byref(cfg), self.mode)
-        for k, v in {**getattr(self, "_ofdm_cfg", {}), **kw}.items():
+        merged = {**getattr(self, "_ofdm_cfg", {}), **kw}
+        for k, v in merged.items():
             setattr(cfg.ofdm, k, v)
-        self._ofdm_cfg = {**getattr(self, "_ofdm_cfg", {}), **kw}
         _check(self.L.dabgpu_ofdm_set_config(self.h, C.byref(cfg.ofdm)))
+        self._ofdm_cfg = merged   # a rejected config leaves the knobs in force, here as in the library
 
     def counters(self) -> dict:
         c = Counters()

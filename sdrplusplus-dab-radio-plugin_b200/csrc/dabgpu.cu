@@ -101,6 +101,15 @@ static cudaError_t sync_ctx(dabgpu_ctx* ctx) {
 
 static void wb_detach(dabgpu_wideband* w);
 
+// The control kernel divides by the L1 window length and by its stride (signal_l1_nb_samples x nb_decimate): both knobs must
+// be positive wherever a configuration enters, at context creation and in dabgpu_ofdm_set_config.
+static int validate_ofdm_config(const dabgpu_ofdm_config& c) {
+    if (c.signal_l1_nb_samples < 1 || c.signal_l1_nb_decimate < 1)
+        return set_error(DABGPU_ERR_INVALID, "signal_l1 window parameters must be >= 1 (nb_samples %d, nb_decimate %d)", c.signal_l1_nb_samples,
+                         c.signal_l1_nb_decimate);
+    return DABGPU_OK;
+}
+
 extern "C" {
 
 const char* dabgpu_version(void) { return DABGPU_VERSION; }
@@ -159,6 +168,7 @@ int dabgpu_ctx_create(const dabgpu_config* cfg, dabgpu_ctx** out) {
     dabgpu_params P;
     int rc = fill_params(cfg->transmission_mode, &P);
     if (rc) return rc;
+    if ((rc = validate_ofdm_config(cfg->ofdm))) return rc;
     if (cfg->max_streams < 1) return set_error(DABGPU_ERR_INVALID, "max_streams must be >= 1");
     if (cfg->iq_format != DABGPU_IQ_U8 && cfg->iq_format != DABGPU_IQ_C32) return set_error(DABGPU_ERR_INVALID, "bad iq_format");
     int ndev = 0;
@@ -1251,7 +1261,7 @@ int dabgpu_get_counters(dabgpu_ctx* ctx, dabgpu_counters* out) {
 // ---------------------------------------------------------------------------------------------
 int dabgpu_ofdm_set_config(dabgpu_ctx* ctx, const dabgpu_ofdm_config* cfg) {
     if (!ctx || !cfg) return set_error(DABGPU_ERR_INVALID, "null argument");
-    if (cfg->signal_l1_nb_samples < 1 || cfg->signal_l1_nb_decimate < 1) return set_error(DABGPU_ERR_INVALID, "signal_l1 window parameters must be >= 1");
+    if (int rc = validate_ofdm_config(*cfg)) return rc;
     ctx->cfg.ofdm = *cfg;
     ctx->ofdm.dev.cfg = *cfg;   // OfdmDev travels by value with every launch: the next call sees the new knobs
     return DABGPU_OK;

@@ -278,8 +278,67 @@ static void run_taps(Reader& in, Writer& out) {
     out.i32(int32_t(corr.size())); out.bytes(corr.data(), corr.size() * sizeof(std::complex<float>));
 }
 
+// mode, n_edits, per edit {call index, 8 floats, 3 ints} (the fields of dabgpu_ofdm_config, floats and ints each in its order),
+// n_calls, call lengths, u8 IQ.  Each call is one OFDM_Demod::Process block; before the calls that have an edit, every field of
+// OFDM_Demod::GetConfig() is written the way the plugin's GUI writes it.  Output per call: n_frames, per frame {bits, coarse, fine,
+// fine time offset}, then GetState, GetTotalFramesRead, GetTotalFramesDesync, GetFineTimeOffset, GetSignalAverage,
+// GetCoarseFrequencyOffset, GetFineFrequencyOffset.
+static void run_ofdmcfg(Reader& in, Writer& out) {
+    const int mode = in.i32(), n_edits = in.i32();
+    struct Edit { int call; float f[8]; int i[3]; };
+    std::vector<Edit> edits(static_cast<size_t>(n_edits));
+    for (auto& e : edits) {
+        e.call = in.i32();
+        for (float& v : e.f) v = in.f32();
+        for (int& v : e.i) v = in.i32();
+    }
+    const int n_calls = in.i32();
+    std::vector<int> lens(static_cast<size_t>(n_calls));
+    for (int& l : lens) l = in.i32();
+    auto demod = Create_OFDM_Demodulator(mode, 1);
+    Writer frames;
+    int n_frames = 0;
+    demod->On_OFDM_Frame().Attach([&](span<const viterbi_bit_t> f) {
+        n_frames++;
+        frames.bytes(f.data(), f.size());
+        const dabgpu_frame_info& fi = demod->GetFrameInfo();
+        frames.f32(fi.freq_coarse_offset); frames.f32(fi.freq_fine_offset); frames.i32(fi.fine_time_offset);
+    });
+    std::vector<std::complex<float>> blockbuf;
+    for (int k = 0; k < n_calls; k++) {
+        for (const auto& e : edits) {
+            if (e.call != k) continue;
+            auto& c = demod->GetConfig();
+            c.signal_l1.update_beta = e.f[0];
+            c.signal_l1.nb_samples = e.i[0];
+            c.signal_l1.nb_decimate = e.i[1];
+            c.null_l1_search.thresh_null_start = e.f[1];
+            c.null_l1_search.thresh_null_end = e.f[2];
+            c.sync.fine_freq_update_beta = e.f[3];
+            c.sync.is_coarse_freq_correction = e.i[2] != 0;
+            c.sync.max_coarse_freq_correction_norm = e.f[4];
+            c.sync.coarse_freq_slow_beta = e.f[5];
+            c.sync.impulse_peak_threshold_db = e.f[6];
+            c.sync.impulse_peak_distance_probability = e.f[7];
+        }
+        const int n = lens[size_t(k)];
+        const uint8_t* u8 = in.bytes(size_t(n) * 2);
+        blockbuf.resize(size_t(n));
+        for (int i = 0; i < n; i++)
+            blockbuf[size_t(i)] = std::complex<float>((float(u8[2 * i]) - 127.5f) * (1.0f / 127.5f), (float(u8[2 * i + 1]) - 127.5f) * (1.0f / 127.5f));
+        n_frames = 0;
+        frames.buf.clear();
+        demod->Process(span<const std::complex<float>>(blockbuf.data(), blockbuf.size()));
+        out.i32(n_frames);
+        out.bytes(frames.buf.data(), frames.buf.size());
+        out.i32(int(demod->GetState())); out.i32(demod->GetTotalFramesRead()); out.i32(demod->GetTotalFramesDesync());
+        out.i32(demod->GetFineTimeOffset());
+        out.f32(demod->GetSignalAverage()); out.f32(demod->GetCoarseFrequencyOffset()); out.f32(demod->GetFineFrequencyOffset());
+    }
+}
+
 int main(int argc, char** argv) {
-    if (argc != 4) { std::cerr << "usage: adapter_check <viterbi|fic|msc|mscpool|rs|pktfec|aac|radio|selfcfg|taps> in.bin out.bin\n"; return 1; }
+    if (argc != 4) { std::cerr << "usage: adapter_check <viterbi|fic|msc|mscpool|rs|pktfec|aac|radio|selfcfg|taps|ofdmcfg> in.bin out.bin\n"; return 1; }
     try {
         Reader in(argv[2]);
         Writer out;
@@ -294,6 +353,7 @@ int main(int argc, char** argv) {
         else if (what == "selfcfg") run_selfcfg(in, out);
         else if (what == "mscpool") run_mscpool(in, out);
         else if (what == "taps") run_taps(in, out);
+        else if (what == "ofdmcfg") run_ofdmcfg(in, out);
         else { std::cerr << "unknown test " << what << "\n"; return 1; }
         out.save(argv[3]);
     } catch (const std::exception& e) {

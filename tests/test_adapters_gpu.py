@@ -385,3 +385,52 @@ def test_ofdm_demod_class_serves_the_gui_getters(driver, tx, pyref, ref_ok):
     exp_vec = ref.frame_data_vec((L - 1) * K)
     assert np.abs(vec[:(L - 1) * K] - exp_vec).max() < 4e-3 * np.abs(exp_vec).max()
     assert np.array_equal(corr, ref.correlation_buffer(corr.size))   # raw input samples: identical
+
+
+def test_ofdm_demod_config_edits_between_process_calls(driver, pyref):
+    """OFDM_Demod::GetConfig() edited between Process() calls of varying lengths, every field at once (host/dab_adapters.hpp
+    push_config copies them into dabgpu_ofdm_config one by one): after each call the frames and GetState / GetTotalFramesRead /
+    GetTotalFramesDesync / GetFineTimeOffset / GetSignalAverage / GetCoarseFrequencyOffset / GetFineFrequencyOffset are the
+    oracle's under the same edits.  The edits are those of tests/ofdm_config_cases.py, which tests/test_ofdm_config_cpu.py shows
+    change the oracle's output whenever two fields of the same type are exchanged."""
+    import ofdm_config_cases as C
+    mode = C.ADAPTER_MODE
+    use_ref = pyref.ref_available()
+    recs = C.recordings(mode)
+    n = recs.shape[1] // 2
+    cl = C.partition_calls(n, C.ADAPTER_BLOCKS)
+    frame_bits = importlib.import_module(PKG).get_params(mode).nb_frame_bits
+    for s in C.ADAPTER_STREAMS:
+        u8 = recs[s]
+        payload = _i32(mode, len(C.ADAPTER_EDITS))
+        for k, e in sorted(C.ADAPTER_EDITS.items()):
+            payload += _i32(k) + struct.pack("<8f", *[e[f] for f in C.FLOAT_KNOBS]) + _i32(*[e[f] for f in C.INT_KNOBS])
+        payload += _i32(len(cl), *[ln for _, ln in cl]) + u8[:2 * n].tobytes()
+        out = _run(driver, "ofdmcfg", payload)
+        exp = C.oracle_outputs(pyref, mode, C.to_c32(u8[None, :2 * n]), {}, cl, 0, u8=False, use_ref=use_ref, edits=C.ADAPTER_EDITS)[0]
+        off, frames = 0, []
+        for k in range(len(cl)):
+            nf, = struct.unpack_from("<i", out, off)
+            off += 4
+            for _ in range(nf):
+                bits = np.frombuffer(out, dtype=np.int8, count=frame_bits, offset=off)
+                coarse, fine, fto = struct.unpack_from("<2fi", out, off + frame_bits)
+                frames.append((bits, coarse, fine, fto))
+                off += frame_bits + 12
+            state, read, desync, fto = struct.unpack_from("<4i", out, off)
+            l1, coarse, fine = struct.unpack_from("<3f", out, off + 16)
+            off += 28
+            e = exp["status"][k]
+            tag = f"stream {s} after call {k}"
+            assert (state, read, desync, fto) == (e["state"], e["frames_read"], e["frames_desync"], e["fine_time_offset"]), (tag, e)
+            assert abs(l1 - e["signal_avg"]) <= C.L1_RTOL * abs(e["signal_avg"]), (tag, l1, e)
+            assert abs(coarse - e["coarse"]) <= C.FREQ_ATOL and abs(fine - e["fine"]) <= C.FREQ_ATOL, (tag, coarse, fine, e)
+        assert off == len(out)
+        assert len(frames) == len(exp["frames"]) > 0
+        for i, ((gb, gc, gf, gt), (eb, ec, ef, et)) in enumerate(zip(frames, exp["frames"])):
+            assert gt == et and abs(gc - ec) <= C.FREQ_ATOL and abs(gf - ef) <= C.FREQ_ATOL, (s, i)
+            d = np.abs(gb.astype(np.int32) - eb.astype(np.int32))
+            if (d >= 1).mean() < 1e-3:
+                assert d.max() <= 1, (s, i, d.max())
+            else:
+                assert d.max() <= 16 and (d > 1).mean() <= 5e-4, (s, i, d.max())
