@@ -364,6 +364,26 @@ DABGPU_API int dabgpu_msc_add_subchannel(dabgpu_ctx* ctx, int stream, const dabg
 /* Detach one decoder; the other entries keep their indices and state (no reference analogue: BasicRadio only ever adds). */
 DABGPU_API int dabgpu_msc_remove_subchannel(dabgpu_ctx* ctx, int stream, int sub_index);
 
+/* What a sub-channel carries, and so which stage runs on its logical frames after the MSC decode:
+ *   STREAM      nothing (the bytes are read with dabgpu_chan_get_msc)
+ *   DABPLUS     the DAB+ superframe stage (AAC_Frame_Processor)
+ *   PACKET      packet mode without FEC: every logical frame is cut into packets the way basic_data_packet_channel.cpp:49-88
+ *               walks it (length from bits 7-6 of byte 0; a tail shorter than 2 bytes or than its packet is dropped)
+ *   PACKET_FEC  packet mode with FIG 0/14 FEC scheme 1: the same walk through MSC_Reed_Solomon_Data_Packet_Processor
+ *               (msc_reed_solomon_data_packet_processor.cpp:49-258, RS(204,188) per FEC set of 2256 + 9 x 24 bytes)
+ * The packet entries report through the sub-channel event log (DABGPU_EV_PACKET / DABGPU_EV_PACKET_FEC records).  Their FEC
+ * state (ring of queued packets, last FEC counter) lives across decodes; a fresh entry starts empty.  A set of 2472 bytes spans
+ * about 26 decodes at 8 kbit/s, one decode can close several sets at high rates.
+ * dabgpu_msc_configure / _add_subchannel are the _ex calls with payload = is_dabplus ? DABPLUS : STREAM.  A packet payload
+ * with sc.is_dabplus != 0 gives DABGPU_ERR_INVALID.  An entry whose payload kind changes starts empty. */
+enum { DABGPU_PAYLOAD_STREAM = 0, DABGPU_PAYLOAD_DABPLUS = 1, DABGPU_PAYLOAD_PACKET = 2, DABGPU_PAYLOAD_PACKET_FEC = 3 };
+typedef struct {
+    dabgpu_subchannel sc;
+    int payload;         /* DABGPU_PAYLOAD_* */
+} dabgpu_subchannel_ex;
+DABGPU_API int dabgpu_msc_configure_ex(dabgpu_ctx* ctx, int stream, const dabgpu_subchannel_ex* subs, int n_subs);
+DABGPU_API int dabgpu_msc_add_subchannel_ex(dabgpu_ctx* ctx, int stream, const dabgpu_subchannel_ex* sub, int* sub_index_out);
+
 /* BasicRadio::Process: one frame of nb_frame_bits int8 per stream, stream i at frames_host + i*stride.  DABGPU_ERR_OVERFLOW when
  * the frame ring of a stream is full of frames that were not channel-decoded yet (the reference's ThreadedRingBuffer blocks its
  * producer in that case, src/radio_block.cpp:20-44). */
@@ -437,22 +457,35 @@ DABGPU_API int dabgpu_chan_get_fic(dabgpu_ctx* ctx, int stream, uint8_t* fibs_ho
 DABGPU_API int dabgpu_chan_get_msc(dabgpu_ctx* ctx, int stream, int sub_index, uint8_t* out_host, size_t out_cap,
                                    uint8_t* valid, int* bytes_per_cif);
 
-/* DAB+ superframe events of the last decoded frame, in the order AAC_Frame_Processor would have
- * fired its observers (OnFirecodeError/OnRSError/OnSuperFrameHeader/OnAccessUnitCRCError/OnAccessUnit). */
+/* Sub-channel event log (DAB+ or packet records) of the last decoded frame.  A DAB+ entry reports the superframe events in the
+ * order AAC_Frame_Processor would have fired its observers (OnFirecodeError/OnRSError/OnSuperFrameHeader/OnAccessUnitCRCError/
+ * OnAccessUnit).  A packet entry (DABGPU_PAYLOAD_PACKET / _PACKET_FEC) reports, in order:
+ *   DABGPU_EV_PACKET      one per packet the processor hands on (the adapter's callback): a = is_corrected, b = crc_ok (CRC16-CCITT
+ *                         of packet[:-2], init 0xFFFF, inverted, equals the last two bytes big-endian; EN 300 401 5.3.2),
+ *                         c = 10-bit packet address, d = 0; payload = the whole packet (24, 48, 72 or 96 bytes).  Without FEC
+ *                         every packet has is_corrected = 0.
+ *   DABGPU_EV_PACKET_FEC  each time an FEC set ends, just before the packets it releases (also when it releases none):
+ *                         a = 1 when the 12 rows were decoded, then b = rows decoded, c = rows uncorrectable, d = sum of the
+ *                         decoded rows' error counts; a = 0 when the set was abandoned (broken FEC counter or incomplete ring),
+ *                         then b = c = d = 0.  No payload. */
 enum { DABGPU_EV_FIRECODE_ERROR = 1, DABGPU_EV_RS_ERROR = 2, DABGPU_EV_SUPERFRAME_HEADER = 3,
-       DABGPU_EV_AU_CRC_ERROR = 4, DABGPU_EV_ACCESS_UNIT = 5 };
+       DABGPU_EV_AU_CRC_ERROR = 4, DABGPU_EV_ACCESS_UNIT = 5, DABGPU_EV_PACKET = 6, DABGPU_EV_PACKET_FEC = 7 };
 typedef struct { int32_t type, a, b, c, d, n_bytes; } dabgpu_event_header;  /* followed by n_bytes payload padded to 4 */
 DABGPU_API int dabgpu_chan_get_dabplus_events(dabgpu_ctx* ctx, int stream, int sub_index, uint8_t* log_host,
                                               size_t log_cap, size_t* log_bytes);
 
-/* DAB+ output of every sub-channel of streams [first, first+n) at once, packed on the GPU.
+/* Sub-channel event logs (DAB+ or packet records) of every sub-channel of streams [first, first+n) at once, packed on the GPU.
  * index_host: [n][max_subchannels][2] int32 = {byte offset into log_host, byte length}.  The log of (stream, sub) is
  * byte-identical to what dabgpu_chan_get_dabplus_events(stream, sub) returns after the same decode: dabgpu_event_header
- * records + payload padded to 4.  Length 0 = no events, not a DAB+ sub-channel, or an unused index.  Where the logs sit inside
+ * records + payload padded to 4.  Length 0 = no events, a STREAM sub-channel, or an unused index.  Where the logs sit inside
  * log_host is not part of the contract: read it through the index.
  *
+ * A packet entry with A = nb_cifs x bytes-per-CIF arriving per decode hands on at most 2472 + A bytes of packets (its FEC ring
+ * plus what arrived) and ends at most A / 24 FEC sets, so its log stays below 24 x (2472 + A) / 24 + (2472 + A) + 24 x (A / 24 + 1)
+ * bytes; dabgpu_dabplus_out_bound counts that for it.
+ *
  * dabgpu_dabplus_out_bound: the log_cap one decode of those streams can never exceed.  It follows from the sub-channel tables
- * (active DAB+ entries and their bytes per CIF): a decode runs one frame of at most 4 CIFs per stream and a superframe takes 5,
+ * (active DAB+ and packet entries and their bytes per CIF): a decode runs one frame of at most 4 CIFs per stream and a superframe takes 5,
  * so each (stream, sub) fires at most 7 events and 5 x bytes-per-CIF of AU payload.  It changes with dabgpu_msc_configure /
  * _add_subchannel / _remove_subchannel.  A log_cap below it gives DABGPU_ERR_OVERFLOW; NULL log_host or index_host gives
  * DABGPU_ERR_INVALID.  Both are refused before anything is queued and leave the context as it was.

@@ -19,6 +19,8 @@ OK, ERR_INVALID, ERR_CUDA, ERR_NOMEM, ERR_STATE, ERR_OVERFLOW = 0, -1, -2, -3, -
 IQ_U8, IQ_C32 = 0, 1
 MAX_SEGMENTS = 5
 EV_FIRECODE_ERROR, EV_RS_ERROR, EV_SUPERFRAME_HEADER, EV_AU_CRC_ERROR, EV_ACCESS_UNIT = 1, 2, 3, 4, 5
+EV_PACKET, EV_PACKET_FEC = 6, 7
+PAYLOAD_STREAM, PAYLOAD_DABPLUS, PAYLOAD_PACKET, PAYLOAD_PACKET_FEC = 0, 1, 2, 3
 WB_RAW_U8, WB_RAW_S8, WB_RAW_S16L, WB_RAW_F32L = 0, 1, 2, 3
 WB_FORMATS = {"raw_u8": WB_RAW_U8, "raw_s8": WB_RAW_S8, "raw_s16l": WB_RAW_S16L, "raw_f32l": WB_RAW_F32L}
 WB_BYTES_PER_SAMPLE = {WB_RAW_U8: 2, WB_RAW_S8: 2, WB_RAW_S16L: 4, WB_RAW_F32L: 8}
@@ -67,6 +69,10 @@ class ViterbiJob(C.Structure):
 
 class SubchannelC(C.Structure):
     _fields_ = [(n, C.c_int) for n in ("start_address", "length", "is_uep", "uep_prot_index", "eep_prot_level", "eep_type_b", "is_dabplus")]
+
+
+class SubchannelExC(C.Structure):
+    _fields_ = [("sc", SubchannelC), ("payload", C.c_int)]
 
 
 class ChanStatus(C.Structure):
@@ -121,7 +127,7 @@ EXPORTS = [
     "dabgpu_autocfg_create", "dabgpu_autocfg_destroy", "dabgpu_autocfg_push_fibs", "dabgpu_autocfg_dump", "dabgpu_autocfg_runnable",
     "dabgpu_host_alloc", "dabgpu_host_free", "dabgpu_ofdm_get_frame_data_vec", "dabgpu_ofdm_get_correlation_buffer", "dabgpu_autocfg_applied", "dabgpu_msc_add_subchannel", "dabgpu_msc_remove_subchannel", "dabgpu_chan_join",
     "dabgpu_autocfg_apply", "dabgpu_ofdm_get_response", "dabgpu_ofdm_get_frame_fft", "dabgpu_iq_convert", "dabgpu_softbits_to_bytes", "dabgpu_bytes_to_softbits",
-    "dabgpu_packet_fec_decode", "dabgpu_wideband_open", "dabgpu_wideband_process", "dabgpu_wideband_close",
+    "dabgpu_packet_fec_decode", "dabgpu_msc_configure_ex", "dabgpu_msc_add_subchannel_ex", "dabgpu_wideband_open", "dabgpu_wideband_process", "dabgpu_wideband_close",
     "dabgpu_wideband_plan", "dabgpu_wideband_open_any_rate", "dabgpu_wideband_reserve", "dabgpu_wideband_submit",
     "dabgpu_dabplus_out_bound", "dabgpu_chan_get_dabplus_all", "dabgpu_submit_ex", "dabgpu_wideband_submit_ex",
 ]
@@ -165,6 +171,8 @@ def load_library() -> C.CDLL:
     L.dabgpu_viterbi_decode.argtypes = [C.c_void_p, C.POINTER(ViterbiJob), C.c_int, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p]
     L.dabgpu_msc_configure.argtypes = [C.c_void_p, C.c_int, C.POINTER(SubchannelC), C.c_int]
     L.dabgpu_msc_add_subchannel.argtypes = [C.c_void_p, C.c_int, C.POINTER(SubchannelC), C.POINTER(C.c_int)]
+    L.dabgpu_msc_configure_ex.argtypes = [C.c_void_p, C.c_int, C.POINTER(SubchannelExC), C.c_int]
+    L.dabgpu_msc_add_subchannel_ex.argtypes = [C.c_void_p, C.c_int, C.POINTER(SubchannelExC), C.POINTER(C.c_int)]
     L.dabgpu_msc_remove_subchannel.argtypes = [C.c_void_p, C.c_int, C.c_int]
     L.dabgpu_chan_join.argtypes = [C.c_void_p]
     L.dabgpu_softbits_push.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int]
@@ -380,25 +388,32 @@ class DabGpu:
 
     # ---- channel decode ------------------------------------------------------------------
     @staticmethod
-    def _fill_sub(dst: SubchannelC, s) -> None:
-        dst.start_address, dst.length = s.start_address, s.length
-        dst.is_uep, dst.uep_prot_index = int(s.is_uep), s.uep_index
-        dst.eep_prot_level, dst.eep_type_b = s.eep_level, int(s.eep_type_b)
-        dst.is_dabplus = int(getattr(s, "dabplus", False))
+    def _fill_sub(dst: SubchannelExC, s) -> None:
+        """s.packet_fec (None when absent) selects packet mode: None = stream or DAB+ (s.dabplus), False = packets without FEC,
+        True = packets with FEC scheme 1."""
+        packet_fec = getattr(s, "packet_fec", None)
+        dabplus = bool(getattr(s, "dabplus", False)) and packet_fec is None
+        d = dst.sc
+        d.start_address, d.length = s.start_address, s.length
+        d.is_uep, d.uep_prot_index = int(s.is_uep), s.uep_index
+        d.eep_prot_level, d.eep_type_b = s.eep_level, int(s.eep_type_b)
+        d.is_dabplus = int(dabplus)
+        dst.payload = (PAYLOAD_PACKET_FEC if packet_fec else PAYLOAD_PACKET) if packet_fec is not None else \
+            (PAYLOAD_DABPLUS if dabplus else PAYLOAD_STREAM)
 
     def msc_configure(self, stream: int, subs: Sequence) -> None:
-        arr = (SubchannelC * max(len(subs), 1))()
+        arr = (SubchannelExC * max(len(subs), 1))()
         for i, s in enumerate(subs):
             self._fill_sub(arr[i], s)
-        _check(self.L.dabgpu_msc_configure(self.h, stream, arr, len(subs)))
+        _check(self.L.dabgpu_msc_configure_ex(self.h, stream, arr, len(subs)))
         self._subs[stream] = list(subs)
 
     def msc_add_subchannel(self, stream: int, sub) -> int:
         """Attach one more decoder without touching the running ones; returns its sub_index."""
-        d = SubchannelC()
+        d = SubchannelExC()
         self._fill_sub(d, sub)
         idx = C.c_int(-1)
-        _check(self.L.dabgpu_msc_add_subchannel(self.h, stream, C.byref(d), C.byref(idx)))
+        _check(self.L.dabgpu_msc_add_subchannel_ex(self.h, stream, C.byref(d), C.byref(idx)))
         self._subs.setdefault(stream, []).append(sub)
         return idx.value
 
@@ -439,7 +454,8 @@ class DabGpu:
         return out, valid
 
     def get_dabplus_events(self, stream: int, sub_index: int) -> bytes:
-        buf = np.zeros(1 << 16, dtype=np.uint8)
+        """The sub-channel event log (DAB+ or packet records) of the last decode."""
+        buf = np.zeros(1 << 17, dtype=np.uint8)
         n = C.c_size_t(0)
         _check(self.L.dabgpu_chan_get_dabplus_events(self.h, stream, sub_index, _ptr(buf), buf.size, C.byref(n)))
         return buf[:n.value].tobytes()

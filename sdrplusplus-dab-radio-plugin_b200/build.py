@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libdabgpu.so")
 SOURCES = ["dabgpu.cu"]
-HEADERS = ["common.cuh", "tables.cuh", "viterbi.cuh", "viterbi_lanes.cuh", "viterbi_lane_core.h", "chan.cuh", "dabplus.cuh", "ofdm.cuh", "ofdm_demod.cuh", "ofdm_host.cuh", "wideband.cuh", os.path.join("..", "..", "include", "dabgpu.h")]
+HEADERS = ["common.cuh", "tables.cuh", "viterbi.cuh", "viterbi_lanes.cuh", "viterbi_lane_core.h", "chan.cuh", "dabplus.cuh", "packet.cuh", "ofdm.cuh", "ofdm_demod.cuh", "ofdm_host.cuh", "wideband.cuh", os.path.join("..", "..", "include", "dabgpu.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

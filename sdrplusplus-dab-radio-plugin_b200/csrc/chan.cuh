@@ -18,7 +18,7 @@ struct SubCfgDev {
     uint32_t seg_in_base[DABGPU_MAX_SEGMENTS];
     uint8_t seg_pi[8];
     uint32_t n_seg, total_steps, n_out_bytes, out_offset;
-    uint32_t is_dabplus, pad0, pad1, pad2;
+    uint32_t is_dabplus, payload, pad1, pad2;   // payload: DABGPU_PAYLOAD_*
 };
 
 struct ChanDev {

@@ -5,6 +5,7 @@
 #include "viterbi_lanes.cuh"
 #include "chan.cuh"
 #include "dabplus.cuh"
+#include "packet.cuh"
 #include "ofdm_host.cuh"
 #include "wideband.cuh"
 #include "../host/fic_autoconfig.hpp"
@@ -16,9 +17,13 @@
 
 struct SubHost {
     dabgpu_subchannel sc;
+    int payload = DABGPU_PAYLOAD_STREAM;
     Schedule sched;
     uint32_t n_out_bytes, out_offset;
     bool active = true;   // false: removed by dabgpu_msc_remove_subchannel (the index stays reserved so that the others keep theirs)
+    int64_t pkt_region = -1;   // packet entries: offset of their region in the packet pool
+    uint64_t pkt_cap = 0;      // ... and its log capacity (pkt_item_bound)
+    bool is_packet() const { return payload == DABGPU_PAYLOAD_PACKET || payload == DABGPU_PAYLOAD_PACKET_FEC; }
 };
 
 struct dabgpu_ctx {
@@ -62,6 +67,8 @@ struct dabgpu_ctx {
 
     // DAB+ superframe stage
     DabPlusState dabplus;
+    // packet-mode sub-channels
+    PacketState packet;
     // channel stream: dabgpu_chan_decode runs on it (see there); join_dabplus() makes the main stream wait for it
     cudaStream_t s_dp = nullptr;
     cudaEvent_t ev_dp = nullptr, ev_dp_fork = nullptr;
@@ -351,6 +358,7 @@ void dabgpu_ctx_destroy(dabgpu_ctx* ctx) {
     if (ctx->s_d2h) { cudaStreamSynchronize(ctx->s_d2h); cudaStreamDestroy(ctx->s_d2h); }
     ofdm_destroy(ctx->ofdm);
     dabplus_destroy(ctx->dabplus);
+    packet_destroy(ctx->packet);
     DevBuf* bufs[] = {&ctx->d_vlplan, &ctx->d_vllist, &ctx->d_vlsym, &ctx->d_vlscratch, &ctx->d_prbs, &ctx->d_counter, &ctx->d_scratch, &ctx->d_jobs, &ctx->d_vsoft, &ctx->d_vout, &ctx->d_verr,
                       &ctx->d_frames, &ctx->d_frames_written, &ctx->d_frames_decoded, &ctx->d_frames_snapshot, &ctx->d_pushstage, &ctx->d_popstage, &ctx->d_frame_info, &ctx->d_subcfg, &ctx->d_nsubs,
                       &ctx->d_cifs_consumed, &ctx->d_fic_out, &ctx->d_fic_crc, &ctx->d_msc_out, &ctx->d_msc_valid, &ctx->d_deint, &ctx->d_status,
@@ -608,9 +616,16 @@ static int check_stream_range(dabgpu_ctx* ctx, int first, int n) {
 }
 
 // Validates one sub-channel description and builds its host / device records (out_offset is assigned by the caller).
-static int build_sub(dabgpu_ctx* ctx, const dabgpu_subchannel& sc, int index, SubHost* h, SubCfgDev* d) {
+static int build_sub(dabgpu_ctx* ctx, const dabgpu_subchannel_ex& ex, int index, SubHost* h, SubCfgDev* d) {
+    const dabgpu_subchannel& sc = ex.sc;
     h->sc = sc;
+    h->payload = ex.payload;
     h->active = true;
+    if (ex.payload < DABGPU_PAYLOAD_STREAM || ex.payload > DABGPU_PAYLOAD_PACKET_FEC)
+        return set_error(DABGPU_ERR_INVALID, "sub-channel %d: unknown payload kind %d", index, ex.payload);
+    if (h->is_packet() && sc.is_dabplus) return set_error(DABGPU_ERR_INVALID, "sub-channel %d: a packet-mode sub-channel cannot be DAB+", index);
+    if ((ex.payload == DABGPU_PAYLOAD_DABPLUS) != (sc.is_dabplus != 0))
+        return set_error(DABGPU_ERR_INVALID, "sub-channel %d: payload %d disagrees with is_dabplus %d", index, ex.payload, sc.is_dabplus);
     if (sc.start_address < 0 || sc.length <= 0 || (sc.start_address + sc.length) * 64 > ctx->P.nb_cif_bits)
         return set_error(DABGPU_ERR_INVALID, "Subchannel bits %d:%d overflows MSC channel with %d bits", sc.start_address * 64,
                          (sc.start_address + sc.length) * 64, ctx->P.nb_cif_bits);
@@ -644,10 +659,20 @@ static int build_sub(dabgpu_ctx* ctx, const dabgpu_subchannel& sc, int index, Su
     d->total_steps = uint32_t(steps);
     d->n_out_bytes = h->n_out_bytes;
     d->is_dabplus = sc.is_dabplus ? 1u : 0u;
+    d->payload = uint32_t(ex.payload);
     return DABGPU_OK;
 }
 
-static bool same_subchannel(const dabgpu_subchannel& a, const dabgpu_subchannel& b) {
+static dabgpu_subchannel_ex sub_ex(const dabgpu_subchannel& sc) {
+    dabgpu_subchannel_ex ex;
+    ex.sc = sc;
+    ex.payload = sc.is_dabplus ? DABGPU_PAYLOAD_DABPLUS : DABGPU_PAYLOAD_STREAM;
+    return ex;
+}
+
+static bool same_subchannel(const SubHost& x, const SubHost& y) {
+    const dabgpu_subchannel &a = x.sc, &b = y.sc;
+    if (x.payload != y.payload) return false;
     if (a.start_address != b.start_address || a.length != b.length || (a.is_uep != 0) != (b.is_uep != 0) || (a.is_dabplus != 0) != (b.is_dabplus != 0)) return false;
     return a.is_uep ? (a.uep_prot_index == b.uep_prot_index) : (a.eep_prot_level == b.eep_prot_level && (a.eep_type_b != 0) == (b.eep_type_b != 0));
 }
@@ -680,6 +705,32 @@ int dabgpu_msc_configure(dabgpu_ctx* ctx, int stream, const dabgpu_subchannel* s
     if (rc) return rc;
     if (n_subs < 0 || n_subs > ctx->max_subs) return set_error(DABGPU_ERR_INVALID, "n_subs %d exceeds max_subchannels %d", n_subs, ctx->max_subs);
     if (n_subs > 0 && !subs) return set_error(DABGPU_ERR_INVALID, "null sub-channel table");
+    std::vector<dabgpu_subchannel_ex> ex(static_cast<size_t>(n_subs));
+    for (int i = 0; i < n_subs; i++) ex[size_t(i)] = sub_ex(subs[i]);
+    return dabgpu_msc_configure_ex(ctx, stream, ex.data(), n_subs);
+}
+
+// A packet entry's region: kept from the old entry it continues, else a fresh one.  Call with the context synchronised.
+static int pkt_attach(dabgpu_ctx* ctx, SubHost& h, const SubHost* kept) {
+    if (!h.is_packet()) return DABGPU_OK;
+    if (kept) { h.pkt_region = kept->pkt_region; h.pkt_cap = kept->pkt_cap; return DABGPU_OK; }
+    h.pkt_cap = pkt_item_bound(uint32_t(ctx->P.nb_cifs), h.n_out_bytes);
+    uint64_t region = 0;
+    int rc = pkt_region_acquire(ctx->packet, h.pkt_cap, &region);
+    if (rc) return rc;
+    h.pkt_region = int64_t(region);
+    return DABGPU_OK;
+}
+static void pkt_detach(dabgpu_ctx* ctx, SubHost& h) {
+    if (h.pkt_region >= 0) pkt_region_release(ctx->packet, h.pkt_cap, uint64_t(h.pkt_region));
+    h.pkt_region = -1;
+}
+
+int dabgpu_msc_configure_ex(dabgpu_ctx* ctx, int stream, const dabgpu_subchannel_ex* subs, int n_subs) {
+    int rc = check_stream_range(ctx, stream, 1);
+    if (rc) return rc;
+    if (n_subs < 0 || n_subs > ctx->max_subs) return set_error(DABGPU_ERR_INVALID, "n_subs %d exceeds max_subchannels %d", n_subs, ctx->max_subs);
+    if (n_subs > 0 && !subs) return set_error(DABGPU_ERR_INVALID, "null sub-channel table");
     CUDA_TRY(cudaSetDevice(ctx->cfg.device));
     std::vector<SubHost> hs(static_cast<size_t>(n_subs));
     std::vector<SubCfgDev> dev(static_cast<size_t>(n_subs));
@@ -693,12 +744,23 @@ int dabgpu_msc_configure(dabgpu_ctx* ctx, int stream, const dabgpu_subchannel* s
     }
     if ((rc = ensure_scratch(ctx, max_steps))) return rc;
     CUDA_TRY(sync_ctx(ctx));
-    const std::vector<SubHost>& old = ctx->subs[size_t(stream)];
-    for (int i = 0; i < n_subs; i++) {
-        const bool keep = size_t(i) < old.size() && old[size_t(i)].active && old[size_t(i)].out_offset == hs[size_t(i)].out_offset &&
-                          same_subchannel(old[size_t(i)].sc, hs[size_t(i)].sc);
-        if ((rc = upload_sub(ctx, stream, i, dev[size_t(i)], !keep))) return rc;
-    }
+    std::vector<SubHost>& old = ctx->subs[size_t(stream)];
+    std::vector<bool> kept(std::max(old.size(), size_t(n_subs)), false);
+    for (int i = 0; i < n_subs; i++)
+        kept[size_t(i)] = size_t(i) < old.size() && old[size_t(i)].active && old[size_t(i)].out_offset == hs[size_t(i)].out_offset &&
+                          same_subchannel(old[size_t(i)], hs[size_t(i)]);
+    // packet regions of the new table first: when the pool cannot grow, the regions taken so far go back and the context keeps
+    // the old table, its regions and its item list untouched
+    for (int i = 0; i < n_subs; i++)
+        if ((rc = pkt_attach(ctx, hs[size_t(i)], kept[size_t(i)] ? &old[size_t(i)] : nullptr))) {
+            for (int j = 0; j < i; j++)
+                if (!kept[size_t(j)]) pkt_detach(ctx, hs[size_t(j)]);
+            return rc;
+        }
+    for (int i = 0; i < n_subs; i++)
+        if ((rc = upload_sub(ctx, stream, i, dev[size_t(i)], !kept[size_t(i)]))) return rc;
+    for (size_t i = 0; i < old.size(); i++)
+        if (!kept[i]) pkt_detach(ctx, old[i]);
     ctx->subs[size_t(stream)] = hs;
     return upload_nsubs(ctx, stream, hs.size());
 }
@@ -706,6 +768,12 @@ int dabgpu_msc_configure(dabgpu_ctx* ctx, int stream, const dabgpu_subchannel* s
 // Attaches a decoder to one more sub-channel of a stream without touching the running ones (BasicRadio::UpdateAfterProcessing,
 // basic_radio.cpp:98-131).  *sub_index_out = its index for dabgpu_chan_get_msc / _get_dabplus_events / dabgpu_msc_get_layout.
 int dabgpu_msc_add_subchannel(dabgpu_ctx* ctx, int stream, const dabgpu_subchannel* sub, int* sub_index_out) {
+    if (!sub) return set_error(DABGPU_ERR_INVALID, "null sub-channel");
+    const dabgpu_subchannel_ex ex = sub_ex(*sub);
+    return dabgpu_msc_add_subchannel_ex(ctx, stream, &ex, sub_index_out);
+}
+
+int dabgpu_msc_add_subchannel_ex(dabgpu_ctx* ctx, int stream, const dabgpu_subchannel_ex* sub, int* sub_index_out) {
     int rc = check_stream_range(ctx, stream, 1);
     if (rc) return rc;
     if (!sub) return set_error(DABGPU_ERR_INVALID, "null sub-channel");
@@ -721,7 +789,11 @@ int dabgpu_msc_add_subchannel(dabgpu_ctx* ctx, int stream, const dabgpu_subchann
     h.out_offset = d.out_offset = out_off;
     if ((rc = ensure_scratch(ctx, d.total_steps))) return rc;
     CUDA_TRY(sync_ctx(ctx));
-    if ((rc = upload_sub(ctx, stream, int(hs.size()), d, true))) return rc;
+    if ((rc = pkt_attach(ctx, h, nullptr))) return rc;
+    if ((rc = upload_sub(ctx, stream, int(hs.size()), d, true))) {
+        pkt_detach(ctx, h);
+        return rc;
+    }
     hs.push_back(h);
     if (sub_index_out) *sub_index_out = int(hs.size()) - 1;
     return upload_nsubs(ctx, stream, hs.size());
@@ -741,6 +813,7 @@ int dabgpu_msc_remove_subchannel(dabgpu_ctx* ctx, int stream, int sub_index) {
     d.out_offset = hs[size_t(sub_index)].out_offset;
     if ((rc = upload_sub(ctx, stream, sub_index, d, true))) return rc;
     hs[size_t(sub_index)].active = false;
+    pkt_detach(ctx, hs[size_t(sub_index)]);
     const size_t nb_cifs = size_t(ctx->P.nb_cifs);
     for (size_t c = 0; c < nb_cifs; c++)
         CUDA_TRY(cudaMemset(ctx->d_msc_valid.as<uint8_t>() + (size_t(stream) * nb_cifs + c) * ctx->max_subs + size_t(sub_index), 0, 1));
@@ -895,6 +968,27 @@ int dabgpu_autocfg_applied(dabgpu_autocfg* a, uint8_t* ids, int cap, int* n_out)
     return DABGPU_OK;
 }
 
+// The packet entries of every stream, by stream then index, on the host and (queued on ctx->stream) on the device.  Rebuilt when
+// the sub-channel tables change (cfg_epoch); every table change first synchronises the context, so nothing queued still reads
+// the old device copy then.
+static int pkt_items(dabgpu_ctx* ctx) {
+    PacketState& P = ctx->packet;
+    if (P.items_epoch == ctx->cfg_epoch) return DABGPU_OK;
+    P.items.clear();
+    for (size_t s = 0; s < ctx->subs.size(); s++)
+        for (size_t k = 0; k < ctx->subs[s].size(); k++) {
+            const SubHost& h = ctx->subs[s][k];
+            if (h.active && h.is_packet()) P.items.push_back(PktItemDev{uint32_t(s), uint32_t(k), uint64_t(h.pkt_region)});
+        }
+    if (!P.items.empty()) {
+        int rc;
+        if ((rc = P.d_items.alloc(P.items.size() * sizeof(PktItemDev)))) return rc;
+        CUDA_TRY(cudaMemcpyAsync(P.d_items.p, P.items.data(), P.items.size() * sizeof(PktItemDev), cudaMemcpyHostToDevice, ctx->stream));
+    }
+    P.items_epoch = ctx->cfg_epoch;
+    return DABGPU_OK;
+}
+
 // The kernels of one channel decode, all on ctx->stream (which dabgpu_chan_decode points at the channel stream meanwhile).
 static int chan_decode_body(dabgpu_ctx* ctx, int first, int n) {
     int rc;
@@ -929,6 +1023,8 @@ static int chan_decode_body(dabgpu_ctx* ctx, int first, int n) {
         if ((rc = launch_viterbi(ctx, ctx->d_jobs.as<VitJobDev>(), int(total), &vb, count_plan != nullptr))) return rc;
     }
     if ((rc = dabplus_run(ctx->dabplus, ctx->chan, first, n, ctx->vl_cache.max_subs_used, ctx->num_sms, ctx->stream, &ctx->launches, ctx->prof))) return rc;
+    if ((rc = pkt_items(ctx))) return rc;
+    if ((rc = packet_run(ctx->packet, ctx->chan, first, n, ctx->num_sms, ctx->stream, &ctx->launches, ctx->prof))) return rc;
     ctx->prof.begin(PROF_CHAN_MISC, ctx->stream);
     k_chan_finish<<<n, 32, 0, ctx->stream>>>(ctx->chan, first, n);
     ctx->prof.end(ctx->stream);
@@ -1036,11 +1132,13 @@ int dabgpu_chan_get_dabplus_events(dabgpu_ctx* ctx, int stream, int sub_index, u
         return set_error(DABGPU_ERR_INVALID, "sub-channel index %d not configured", sub_index);
     CUDA_TRY(cudaSetDevice(ctx->cfg.device));
     CUDA_TRY(sync_ctx(ctx));
+    const SubHost& h = ctx->subs[size_t(stream)][size_t(sub_index)];
+    if (h.is_packet()) return packet_get_events(ctx->packet, uint64_t(h.pkt_region), log_host, log_cap, log_bytes);
     return dabplus_get_events(ctx->dabplus, stream, sub_index, log_host, log_cap, log_bytes);
 }
 
-// The packed DAB+ output layout over every stream: dp_pack_item_bound for each active DAB+ sub-channel, 0 for every other
-// entry of the [max_streams][max_subs] table.  It depends only on the sub-channel tables and is rebuilt when they change
+// The packed output layout over every stream: dp_pack_item_bound for each active DAB+ sub-channel, pkt_item_bound for each
+// active packet entry, 0 for every other entry of the [max_streams][max_subs] table.  It depends only on the sub-channel tables and is rebuilt when they change
 // (cfg_epoch).  Every table change first synchronises the context, so no queued pack still reads the device copy then.
 static const std::vector<uint64_t>& dp_layout(dabgpu_ctx* ctx) {
     DabPlusState& D = ctx->dabplus;
@@ -1053,6 +1151,7 @@ static const std::vector<uint64_t>& dp_layout(dabgpu_ctx* ctx) {
                 D.layout[s * ms + k] = at;
                 const SubHost* h = k < ctx->subs[s].size() ? &ctx->subs[s][k] : nullptr;
                 if (h && h->active && h->sc.is_dabplus) at += dp_pack_item_bound(h->n_out_bytes);
+                if (h && h->active && h->is_packet()) at += h->pkt_cap;
             }
         D.layout.back() = at;
         D.layout_epoch = ctx->cfg_epoch;
@@ -1093,8 +1192,13 @@ static int dp_pack(dabgpu_ctx* ctx, int first, int n, size_t log_bytes, DevBuf& 
     if ((rc = d_buf.alloc(at + size_t(n) * ctx->max_subs * 8))) return rc;
     uint32_t subs_per_stream = 0;
     for (int s = first; s < first + n; s++) subs_per_stream = std::max(subs_per_stream, uint32_t(ctx->subs[size_t(s)].size()));
-    return dabplus_pack(D, first, n, subs_per_stream, d_buf.as<uint8_t>(), reinterpret_cast<int32_t*>(d_buf.as<uint8_t>() + at), ctx->stream,
-                        &ctx->launches, ctx->prof);
+    if ((rc = dabplus_pack(D, first, n, subs_per_stream, d_buf.as<uint8_t>(), reinterpret_cast<int32_t*>(d_buf.as<uint8_t>() + at), ctx->stream,
+                           &ctx->launches, ctx->prof)))
+        return rc;
+    // the packet entries' logs and index entries, over what k_dabplus_pack left empty for them
+    if ((rc = pkt_items(ctx))) return rc;
+    return packet_pack(ctx->packet, D.d_layout.as<uint64_t>(), first, n, ctx->max_subs, d_buf.as<uint8_t>(),
+                       reinterpret_cast<int32_t*>(d_buf.as<uint8_t>() + at), ctx->stream, &ctx->launches, ctx->prof);
 }
 
 static int dp_copy_out(dabgpu_ctx* ctx, int n, size_t log_bytes, const DevBuf& d_buf, const dabgpu_dabplus_out* out, cudaStream_t s) {

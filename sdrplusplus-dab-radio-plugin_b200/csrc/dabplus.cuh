@@ -123,9 +123,9 @@ struct DpShared : DpTables {
     __align__(16) uint8_t sfbuf[DP_WARPS][DP_SF_SMEM];
 };
 
-__device__ __forceinline__ void dp_load_shared(DpShared& sh) {
+__device__ __forceinline__ void dp_load_shared(DpTables& sh) {
     const uint4* src = reinterpret_cast<const uint4*>(&g_dp_tables);
-    uint4* dst = reinterpret_cast<uint4*>(static_cast<DpTables*>(&sh));
+    uint4* dst = reinterpret_cast<uint4*>(&sh);
     for (int i = threadIdx.x; i < int(sizeof(DpTables) / 16); i += blockDim.x) dst[i] = src[i];
     __syncthreads();
 }
@@ -539,14 +539,9 @@ __global__ void k_rs_batch(uint8_t* __restrict__ cw, const int n_cw, const int n
 #define PKT_FEC_ROWS 12
 #define PKT_FEC_DATA 188
 #define PKT_FEC_FRAME_BYTES 2448   // 204 * 12
-__global__ void k_packet_fec(uint8_t* __restrict__ frames, const int n_frames, int* __restrict__ counts) {
-    __shared__ DpShared sh;
-    dp_load_shared(sh);
-    const GfTables T{sh.gf_ex, sh.gf_lg};
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_frames * PKT_FEC_ROWS) return;
-    const int f = i / PKT_FEC_ROWS, y = i - f * PKT_FEC_ROWS;
-    uint8_t* row = frames + size_t(f) * PKT_FEC_FRAME_BYTES + y;
+// Row y of a frame (row = frame + y), corrected in place; returns the decoder's count (-1: uncorrectable, row untouched).
+// Shared with k_packet (packet.cuh), which decodes the sets of the packet-mode sub-channels inside the channel decode.
+__device__ int pkt_fec_row(const GfTables& T, uint8_t* row) {
     constexpr int nroots = 16, pad = 51, n = 204;
     uint8_t S[RS_MAX_ROOTS], loc[RS_MAX_ROOTS], xv[RS_MAX_ROOTS], ap[RS_MAX_ROOTS];
     int cnt = 0;
@@ -555,7 +550,17 @@ __global__ void k_packet_fec(uint8_t* __restrict__ frames, const int n_frames, i
         const int x = int(loc[j]) - pad;
         if (ap[j] && x < PKT_FEC_DATA) row[size_t(x) * PKT_FEC_ROWS] ^= xv[j];
     }
-    counts[i] = cnt;
+    return cnt;
+}
+
+__global__ void k_packet_fec(uint8_t* __restrict__ frames, const int n_frames, int* __restrict__ counts) {
+    __shared__ DpShared sh;
+    dp_load_shared(sh);
+    const GfTables T{sh.gf_ex, sh.gf_lg};
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_frames * PKT_FEC_ROWS) return;
+    const int f = i / PKT_FEC_ROWS, y = i - f * PKT_FEC_ROWS;
+    counts[i] = pkt_fec_row(T, frames + size_t(f) * PKT_FEC_FRAME_BYTES + y);
 }
 
 static int dabplus_init(DabPlusState& S, int max_streams, int max_subs, int nb_cifs) {

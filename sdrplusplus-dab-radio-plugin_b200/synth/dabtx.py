@@ -11,7 +11,7 @@ It is workload-generation code for tests and ``bench.py``; nothing here runs on 
 from __future__ import annotations
 
 from dataclasses import dataclass, field
-from typing import List, Optional, Sequence, Tuple
+from typing import Callable, List, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -245,6 +245,7 @@ class Subchannel:
     eep_level: int = 2      # 0-based: 2 => 3-A / 3-B
     eep_type_b: bool = False
     dabplus: bool = True    # payload carries DAB+ superframes (needs frame bytes % 24 == 0)
+    packet_fec: Optional[bool] = None   # not None: packet mode (EN 300 401 5.3.2), with FEC scheme 1 when True; dabplus is ignored
 
     def segments(self) -> List[Tuple[int, int]]:
         return uep_segments(self.uep_index) if self.is_uep else eep_segments(self.length, self.eep_level, self.eep_type_b)
@@ -363,18 +364,43 @@ def packet_fec_set(rng: np.random.Generator, lengths: Optional[Sequence[int]] = 
         p[0] = ((n // 24 - 1) << 6) | ((i & 3) << 4) | (int(rng.integers(0, 4)) << 2) | (address >> 8)
         p[1] = address & 0xFF
         packets.append(p)
-    table = np.concatenate(packets)
+    return packets + fec_packets(packets)
+
+
+def fec_packets(data_packets: Sequence[np.ndarray]) -> List[np.ndarray]:
+    """The nine FEC packets (address 1022, counters 0..8) carrying the RS(204,188) parity of the 12 rows of a 2256-byte
+    application data table (EN 300 401 5.3.5)."""
+    table = np.concatenate(data_packets)
+    assert table.size == 2256
     parity = np.zeros(192, dtype=np.uint8)
     for y in range(12):
         parity[y::12] = rs_encode([int(v) for v in table[y::12]], 16)
+    out = []
     for i in range(9):
         p = np.zeros(24, dtype=np.uint8)
         p[0] = (i << 2) | 0x03
         p[1] = 0xFE
         n = 22 if i < 8 else 16
         p[2:2 + n] = parity[22 * i:22 * i + n]
-        packets.append(p)
-    return packets
+        out.append(p)
+    return out
+
+
+def data_packet(rng: np.random.Generator, n: int, address: int, continuity: int, first: bool, last: bool,
+                useful: Optional[int] = None) -> np.ndarray:
+    """One packet (EN 300 401 5.3.2): length, continuity index, first/last flags, 10-bit address, command flag 0, useful data
+    length, useful data, zero padding, CRC16-CCITT over everything before it.  Address 0 is a padding packet (no useful data)."""
+    assert n in (24, 48, 72, 96) and 0 <= address < 1024
+    if useful is None:
+        useful = 0 if address == 0 else int(rng.integers(1, n - 4))
+    p = np.zeros(n, dtype=np.uint8)
+    p[0] = ((n // 24 - 1) << 6) | ((continuity & 3) << 4) | (int(first) << 3) | (int(last) << 2) | (address >> 8)
+    p[1] = address & 0xFF
+    p[2] = useful & 0x7F
+    p[3:3 + useful] = rng.integers(0, 256, size=useful, dtype=np.uint8)
+    crc = crc16_ccitt(p[:n - 2])
+    p[n - 2], p[n - 1] = crc >> 8, crc & 0xFF
+    return p
 
 
 def build_superframe(bitrate_kbps: int, rng: np.random.Generator, dac_rate: int = 1, sbr: int = 1,
@@ -429,9 +455,16 @@ class EnsembleTx:
     """Generates transmission-frame payload bits for a fixed sub-channel layout.
 
     ``logical_frames[sc.id]`` accumulates the decoded-domain payload bytes per CIF so tests can
-    compare decoder output (which lags 15 CIFs: cif_deinterleaver.cpp:36-71)."""
+    compare decoder output (which lags 15 CIFs: cif_deinterleaver.cpp:36-71).
 
-    def __init__(self, mode: int, subchannels: Sequence[Subchannel], seed: int = 1, fill_random: bool = True):
+    Packet-mode sub-channels (``packet_fec`` not None) carry whole packets per logical frame: data packets on a few addresses
+    (data groups of one to three packets with first/last flags and a continuity index per address) and padding packets; with
+    FEC, nine FEC packets follow every 2256 bytes of them.  ``packets[sc.id]`` records every packet as generated, FEC packets
+    included.  ``packet_hook(sc, packets) -> packets`` sees each batch (an FEC set, or one frame's worth without FEC) before the
+    stream is cut into logical frames, and may corrupt, drop or add packets."""
+
+    def __init__(self, mode: int, subchannels: Sequence[Subchannel], seed: int = 1, fill_random: bool = True,
+                 packet_hook: Optional[Callable] = None):
         self.p = MODES[mode]
         self.subchannels = list(subchannels)
         self.rng = np.random.default_rng(seed)
@@ -445,9 +478,53 @@ class EnsembleTx:
         self._enc_hist = {sc.id: [np.zeros(sc.nb_bits, dtype=np.uint8) for _ in range(16)] for sc in self.subchannels}
         self._figs = fig0_1(self.subchannels) + fig0_2(self.subchannels)
         self._fig_pos = 0
+        self.packet_hook = packet_hook
+        self.packets = {sc.id: [] for sc in self.subchannels if sc.packet_fec is not None}
+        self._pkt_buf = {k: np.zeros(0, dtype=np.uint8) for k in self.packets}
+        self._pkt_sent = {k: 0 for k in self.packets}
+        self._pkt_groups = {k: {} for k in self.packets}    # address -> [continuity index, packets left in the data group]
+
+    def _next_packet(self, sc: Subchannel, n: int) -> np.ndarray:
+        address = 0 if self.rng.random() < 0.1 else 1 + 3 * sc.id + int(self.rng.integers(0, 3))
+        if address == 0:
+            return data_packet(self.rng, n, 0, 0, True, True)
+        g = self._pkt_groups[sc.id].setdefault(address, [0, 0])
+        first = g[1] == 0
+        if first:
+            g[1] = int(self.rng.integers(1, 4))
+        g[1] -= 1
+        p = data_packet(self.rng, n, address, g[0], first, g[1] == 0)
+        g[0] = (g[0] + 1) & 3
+        return p
+
+    def _packet_batch(self, sc: Subchannel) -> np.ndarray:
+        nb = sc.frame_bytes
+        total = 2256 if sc.packet_fec else nb
+        pkts, used, pos = [], 0, self._pkt_sent[sc.id] % nb
+        while used < total:       # whole packets per logical frame
+            r = min(nb - pos, total - used, 96)
+            n = int(self.rng.choice([x for x in (24, 48, 72, 96) if x <= r]))
+            pkts.append(self._next_packet(sc, n))
+            used += n
+            pos = (pos + n) % nb
+        if sc.packet_fec:
+            pkts += fec_packets(pkts)
+        self.packets[sc.id] += [p.copy() for p in pkts]
+        if self.packet_hook is not None:
+            pkts = self.packet_hook(sc, pkts)
+        out = np.concatenate(pkts) if pkts else np.zeros(0, dtype=np.uint8)
+        self._pkt_sent[sc.id] += out.size
+        return out
 
     def _next_logical_frame(self, sc: Subchannel) -> np.ndarray:
         nb = sc.frame_bytes
+        if sc.packet_fec is not None:
+            assert nb % 24 == 0, "packet-mode sub-channels carry whole 24-byte units"
+            buf = self._pkt_buf[sc.id]
+            while buf.size < nb:
+                buf = np.concatenate([buf, self._packet_batch(sc)])
+            frame, self._pkt_buf[sc.id] = buf[:nb], buf[nb:]
+            return frame
         if sc.dabplus and nb % 24 == 0:
             buf = self._sf_buf[sc.id]
             if buf.size < nb:
